@@ -65,7 +65,14 @@ def parse_args():
     ap.add_argument("--keep-digest", action="store_true",
                     help="keep the per-forward weight digest of the plan cache inside the timed region "
                          "(default: weights frozen after warm-up, as a serving loop would)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write rank 0's outputs of the last timed headline step (mel, mel_postnet, codes) as "
+                         "DIR/<name>.npy in float32, at most 64 MB in all (beyond that a fixed seeded sample of the "
+                         "utterances); the inputs depend on the arguments only, so two builds compare output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "native" or args.workload != "batch"):
+        ap.error("--dump-outputs writes the headline batch of the native arm (--impl native --workload batch)")
+    return args
 
 
 def peaks():
@@ -280,6 +287,24 @@ def bench_inputs(B, T, rank):
     x = torch.rand(B, T, 80, generator=gen) * 6 - 5
     spk = lambda: torch.nn.functional.normalize(torch.randn(B, 256, generator=gen), dim=-1)
     return x, spk(), spk()
+
+
+DUMP_LIMIT = 64_000_000         # bytes --dump-outputs may write, .npy headers included
+
+
+def dump_outputs(dirname, outs):
+    """Write {name: CPU tensor with the utterances on dim 0} as dirname/<name>.npy in float32.  When the whole batch
+    exceeds DUMP_LIMIT, every array keeps the same utterances: a seeded sample that depends on the batch size only,
+    in batch order."""
+    import numpy as np
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    B = next(iter(outs.values())).shape[0]
+    per_utt = sum(t[0].numel() * 4 for t in outs.values())
+    keep = min(B, (DUMP_LIMIT - 4096 * len(outs)) // per_utt)        # 4 KB for every .npy header
+    rows = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    for name, t in outs.items():
+        np.save(os.path.join(dirname, name + ".npy"), t[rows].float().numpy())
 
 
 def time_cpu(run, frames, min_seconds, max_seconds, min_runs=3):
@@ -724,9 +749,10 @@ def run_native(args):
     x_h, c_org_h, c_trg_h = x_c.pin_memory(), co_c.pin_memory(), ct_c.pin_memory()
     x_d, c_org_d, c_trg_d = x_h.to(dev), c_org_h.to(dev), c_trg_h.to(dev)
     out_h = [None, None, None]
+    out_d = [None, None, None]
 
     def device_step():
-        return model(x_d, c_org_d, c_trg_d)
+        out_d[:] = model(x_d, c_org_d, c_trg_d)
 
     streamer = StreamingConverter(model, dev)      # public host-to-host API: copies overlap neighbouring batches
 
@@ -750,6 +776,8 @@ def run_native(args):
         model.freeze_weights()                     # serving loop: weights do not change between steps
     sampler = ClockSampler(ctx.local_rank) if rank == 0 else None
     ms_total, launches = timed_steps(ctx, device_step, args.steps, sampler)
+    # copied before the e2e and profiling passes run the model again; written to disk after the last measurement
+    dumped = dict(zip(("mel", "mel_postnet", "codes"), (t.cpu() for t in out_d))) if args.dump_outputs and rank == 0 else None
     frames_per_step = B * T * world
     value = frames_per_step * args.steps / (ms_total * 1e-3)
 
@@ -772,7 +800,9 @@ def run_native(args):
     dom_e = tensor_fams[dom]
     fused = lstm_fused_default()
     kernel_name = {"lstm_step": "lstm_fused_kernel" if fused else "lstm_step_kernel", "conv": "conv_gemm_kernel",
-                   "inproj": "conv_gemm_kernel", "linear": "conv_gemm_kernel"}[dom]
+                   "inproj": "conv_gemm_kernel", "linear": "conv_gemm_kernel",
+                   # weight-stationary LSTM kernels: the recurrence at small batches (ops.lstm_seq_ws / lstm_stack_ws)
+                   "lstm_ws": "lstm_ws_kernel", "lstm_stack": "lstm_stack_kernel"}[dom]
     # the timed region is sub-second and runs at the full SM clock (see `clocks`): the burst bf16 figure is the peak a
     # kernel timed like this can reach; the sustained (power-capped, seconds-long) figure is kept beside it
     short = ms_total < 1000.0
@@ -874,6 +904,8 @@ def run_native(args):
             "configs": configs,
             "ranks": [{"frames_per_step": r[0], "ms": r[1], "checksum": r[2]} for r in ranks],
         }
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -1,4 +1,5 @@
-import sys; sys.path.insert(0, "/root/repo/scripts"); sys.path.insert(0, "/root/repo")
+import os, sys
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import mixer_unit_timing as m
 m.run("fp16x2", 64, 1376, "none")
 m.run("fp16x2", 64, 1376, "gelu")
