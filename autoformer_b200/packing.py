@@ -64,7 +64,7 @@ def to_act(t: torch.Tensor, precision: str) -> torch.Tensor:
     if precision == "bf16":
         return t.to(torch.bfloat16)
     if precision in ("fp16x2", "f16"):
-        return t.to(torch.float16)
+        return sat_f16(t).to(torch.float16)       # saturating like the kernels' fp16 stores (cvt.rn.satfinite)
     hi, lo = split_f16(sat_f16(t)) if precision == "fp16s" else split_bf16(t)
     return torch.cat([hi, lo], dim=-1).contiguous()
 

@@ -18,7 +18,7 @@ GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 
 
 @pytest.mark.parametrize("C,d,B,L", [(64, 1, 2, 256), (64, 9, 1, 384), (32, 3, 3, 128), (32, 9, 2, 640), (64, 3, 150, 128),
-                                     (32, 1, 700, 128), (64, 9, 2, 128 * 37),
+                                     (32, 1, 700, 128), (64, 9, 2, 128 * 37), (32, 3, 2, 128 * 37),
                                      (128, 1, 2, 256), (128, 9, 1, 384), (128, 3, 3, 128), (128, 3, 301, 128),
                                      (128, 9, 2, 128 * 41)])
 def test_resblock2_matches_torch(C, d, B, L):
@@ -60,6 +60,50 @@ def test_resblock2_matches_torch(C, d, B, L):
     out2 = torch.zeros(B * L, C, device="cuda")
     blk(xd, B, L, out2=out2)
     assert rel_l2(out2.view(B, L, C), ya) < 2e-5
+    if C == 32:
+        _check_wav_epilogue(blk, xd, B, L, d, xa, xs, mid, ya, w3, b3, w1, wsc)
+
+
+def _check_wav_epilogue(blk, xd, B, L, d, xa, xs, mid, ya, w3, b3, w1, wsc):
+    """The generator's output layer fused into the block's epilogue (wav=, mono=): tanh(Conv1d(C -> 1, K)) over
+    ReflectionPad1d(K // 2) of LeakyReLU(y), run over 128-row tiles that overlap by K - 1.  Every sample is held to a
+    worst-case bound -- the first and last K // 2 of each utterance (mirrored rows) and both sides of every tile seam
+    included -- so an error confined to the seams or the ends shows, which the waveform's rel-L2 cannot see."""
+    U = 2.0 ** -23
+    C = ya.shape[2]
+    # per-element bound on the staged LeakyReLU(y): the k3 sums (one fp16 operand x two fp16 weight terms), the two-term
+    # rounding of the intermediate (which may round the other way), then block.4 + shortcut over the stored operands
+    s3 = F.conv1d(xa.abs().transpose(1, 2), w3.double().abs(), b3.double().abs(), dilation=d)
+    # LeakyReLU of a negative operand is 0.2f * x in fp32 on the device, 0.2 * x in fp64 here: the one-fp16 operand may
+    # round to the neighbouring value (one fp16 ulp, 2^-11 relative)
+    neg = F.conv1d((xa.abs() * (xs < 0)).transpose(1, 2), w3.double().abs(), dilation=d)
+    e_mid = (3 * 2 * C + 2) * U * s3 + 2.0 ** -11 * neg
+    e_mid = e_mid + 2 * (2.0 ** -22 * (mid.abs() + e_mid) + 2.0 ** -25)
+    s1 = F.conv1d(mid.abs(), w1.double().abs()) + F.conv1d(xs[:, d:d + L].abs().transpose(1, 2), wsc.double().abs())
+    s1 = s1 + blk.bias1.double().abs().cpu().view(1, C, 1)
+    e_y = (F.conv1d(e_mid, w1.double().abs()) + (4 * 2 * C + 2) * U * s1).transpose(1, 2)
+    e_a = e_y + 2 * U * ya.abs()
+    for K in (3, 5, 7):
+        g = torch.Generator().manual_seed(K)
+        w_out = torch.randn(K, C, generator=g) / (K * C) ** 0.5
+        b_out = 0.05 * K
+        wav = torch.full((B, L), float("nan"), device="cuda")
+        blk(xd, B, L, wav=wav, mono=(w_out.cuda(), b_out))
+        torch.cuda.synchronize()
+        pad = lambda t: F.pad(t.transpose(1, 2), (K // 2, K // 2), mode="reflect")
+        wk = w_out.double().t().unsqueeze(0)                                  # (1, C, K)
+        v = F.conv1d(pad(ya), wk).squeeze(1) + b_out
+        s = F.conv1d(pad(ya).abs(), wk.abs()).squeeze(1) + abs(b_out)
+        bound = F.conv1d(pad(e_a), wk.abs()).squeeze(1) + (K * C + 2) * U * s + 2e-6    # tanh_fast: ~1e-7 absolute
+        got = wav.cpu().double()
+        assert bool(torch.isfinite(got).all()), K
+        err = (got - torch.tanh(v)).abs()
+        stride = 128 - (K - 1)
+        edges = sorted({*range(K // 2), *range(L - K // 2, L)} | {t for j in range(1, L // stride + 1)
+                                                                  for t in (j * stride - 1, j * stride) if t < L})
+        assert bool((err[:, edges] <= bound[:, edges]).all()), (K, "utterance ends / tile seams", float(err[:, edges].max()))
+        bad = err > bound
+        assert not bool(bad.any()), (K, bad.nonzero()[:5].tolist(), float((err - bound).max()))
 
 
 @pytest.mark.parametrize("name", ["melgan_b1_t40", "melgan_b2_t17"])
