@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libavc_b200.so")
-SOURCES = ["avc_host.cu", "avc_gemm.cu", "avc_lstm.cu", "avc_lstm_ws.cu", "avc_lstm_stack.cu", "avc_misc.cu", "avc_meta.cu", "avc_resblock.cu", "avc_resblock_big.cu"]
+SOURCES = ["avc_host.cu", "avc_gemm.cu", "avc_lstm.cu", "avc_lstm_ws.cu", "avc_lstm_stack.cu", "avc_misc.cu", "avc_meta.cu", "avc_resblock.cu", "avc_resblock_big.cu", "avc_bn.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 

@@ -17,7 +17,7 @@ EXPORTS = ["avc_version", "avc_last_error", "avc_launch_count", "avc_conv_gemm",
            "avc_bilstm_small", "avc_concat_bcast", "avc_linear_l2norm", "avc_linear_rows", "avc_transpose_pad",
            "avc_conv_to_mono_tanh", "avc_gn_stats", "avc_gn_pool_residual", "avc_gn_apply", "avc_patchify",
            "avc_ln_transpose", "avc_meta_decoder_input", "avc_gather_codes", "avc_global_stats", "avc_adain", "avc_audio_frames",
-           "avc_complex_mag", "avc_resblock", "avc_resblock2", "avc_reflect_halo"]
+           "avc_complex_mag", "avc_resblock", "avc_resblock2", "avc_reflect_halo", "avc_bn_batch_stats", "avc_bn_apply"]
 
 
 MAX_SOURCES = 4
@@ -183,6 +183,33 @@ class Resblock2Desc(ctypes.Structure):
     ]
 
 
+BN_MAX_PARTS = 256      # AVC_BN_MAX_PARTS: avc_bn_batch_stats needs 2 + 2 * BN_MAX_PARTS * C doubles of scratch
+
+
+class BnApplyDesc(ctypes.Structure):
+    """struct avc_bn_apply_desc"""
+    _fields_ = [
+        ("v", ctypes.c_void_p),
+        ("v_ld", ctypes.c_longlong),
+        ("scale_shift", ctypes.c_void_p),
+        ("B", ctypes.c_int),
+        ("T", ctypes.c_int),
+        ("C", ctypes.c_int),
+        ("act", ctypes.c_int),
+        ("residual", ctypes.c_void_p),
+        ("res_ld", ctypes.c_longlong),
+        ("res_after_act", ctypes.c_int),
+        ("out", ctypes.c_void_p),
+        ("out_ld", ctypes.c_longlong),
+        ("out_rows_per_utt", ctypes.c_int),
+        ("out_row0", ctypes.c_int),
+        ("out_dtype", ctypes.c_int),
+        ("out_round_tf32", ctypes.c_int),
+        ("out2", ctypes.c_void_p),
+        ("out2_ld", ctypes.c_longlong),
+    ]
+
+
 _lib = None
 
 
@@ -248,6 +275,10 @@ def load():
     lib.avc_audio_frames.argtypes = [vp, vp, ci, ctypes.c_longlong, ci, ci, ci, ci, ci, vp]
     lib.avc_complex_mag.argtypes = [vp, vp, ctypes.c_longlong, ci, ci, ci, ci, vp]
     lib.avc_audio_frames.restype = lib.avc_complex_mag.restype = ctypes.c_int
+    lib.avc_bn_batch_stats.argtypes = [vp, ctypes.c_longlong, ci, ctypes.c_longlong, vp, vp, ctypes.c_float,
+                                       ctypes.c_float, ci, vp, vp, vp, vp, vp, vp]
+    lib.avc_bn_apply.argtypes = [ctypes.POINTER(BnApplyDesc), vp]
+    lib.avc_bn_batch_stats.restype = lib.avc_bn_apply.restype = ctypes.c_int
     for fn in (lib.avc_gn_stats, lib.avc_gn_pool_residual, lib.avc_gn_apply, lib.avc_patchify, lib.avc_ln_transpose,
                lib.avc_meta_decoder_input, lib.avc_gather_codes):
         fn.restype = ctypes.c_int

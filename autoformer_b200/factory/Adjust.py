@@ -3,7 +3,8 @@
 Re-estimates a speaker embedding from (mel, embedding): speaker-code concat, 3 x [Conv1d k5 + BatchNorm + ReLU],
 3 x LSTM(512 -> 768), last time step, Linear(768 -> 256), L2 normalisation.  Every piece re-uses a kernel of the
 conversion path: ``avc_concat_bcast``, ``avc_conv_gemm`` (BN folded, ReLU in the epilogue), ``avc_lstm_seq`` (only
-h_T of the top layer leaves the kernel) and ``avc_linear_l2norm``.  Eval-mode semantics, inference only.
+h_T of the top layer leaves the kernel) and ``avc_linear_l2norm``.  Eval-mode semantics by default; ``bn_stats =
+"batch"`` selects train-mode BatchNorm statistics (see autoformer_b200.AutoVC).  Inference only.
 """
 import torch
 import torch.nn as nn
@@ -15,10 +16,10 @@ from .Norm import ConvNorm, LinearNorm
 class AdjustPlan:
     """Packed weights of one ``Adjust`` block taken from a (possibly enclosing) state_dict under ``prefix``."""
 
-    def __init__(self, sd, prefix, precision, wavefront=None):
+    def __init__(self, sd, prefix, precision, wavefront=None, bn_owner=None):
         p = prefix + "." if prefix else ""
         self.precision = precision
-        self.convs = [layers.conv_bn_layer(sd, f"{p}convolutions.{i}", precision, "relu") for i in range(3)]
+        self.convs = [layers.conv_bn_layer(sd, f"{p}convolutions.{i}", precision, "relu", bn_owner) for i in range(3)]
         self.lstm = layers.LstmStack(layers.lstm_layers(sd, f"{p}lstm", 3, precision), precision, wavefront)
         self.w = sd[f"{p}embedding.linear_layer.weight"].float().contiguous()
         self.b = sd[f"{p}embedding.linear_layer.bias"].float().contiguous()
@@ -49,13 +50,16 @@ class Adjust(layers.PlanOwner, nn.Module):
         self.precision = "fp32"
         self.persistent_lstm = True
         self.wavefront = None           # None: the library default (layers.LstmStack)
+        self.bn_stats = "running"
         self._cache = layers.PlanCache()
 
     def _plan(self):
+        batch = layers.check_bn_stats(self.bn_stats) == "batch"
+
         def build():
             sd = layers.state_for_packing(self)
-            return AdjustPlan(sd, "", self.precision, self.wavefront)
-        return self._cache.get(self, (self.precision, self.wavefront), build)
+            return AdjustPlan(sd, "", self.precision, self.wavefront, self if batch else None)
+        return self._cache.get(self, (self.precision, self.wavefront, self.bn_stats), build, skip_bn_stats=batch)
 
     @ops.on_device_of_input
     @torch.no_grad()
@@ -63,4 +67,6 @@ class Adjust(layers.PlanOwner, nn.Module):
         if x.dim() == 4:
             x = x.squeeze(1)                                            # Adjust.py:30
         ops._require_cuda(x, emb)
+        if layers.check_bn_stats(self.bn_stats) == "batch" and x.shape[0] * x.shape[1] == 1:
+            raise ValueError(f"Expected more than 1 value per channel when training, got input size {(1, 512, 1)}")
         return self._plan()(x.contiguous().float(), emb.contiguous().float(), self.persistent_lstm)

@@ -2,8 +2,9 @@
 
 Same constructor ``AutoVC(dim_neck, dim_emb, dim_pre, freq)``, same ``forward(x, c_org, c_trg)`` contract and the
 same ``state_dict`` key names as the reference (factory/AutoVC.py:182-211), so reference checkpoints load
-unchanged.  Semantics are the reference's *eval-mode* forward (BatchNorm uses running statistics, SURVEY.md 0.1);
-inference only (outputs carry no autograd graph).  There is no CPU / eager fallback.
+unchanged.  By default the semantics are the reference's *eval-mode* forward (BatchNorm uses running statistics,
+SURVEY.md 0.1); ``bn_stats = "batch"`` selects its train-mode BatchNorm instead (batch statistics, running buffers
+updated).  Inference only (outputs carry no autograd graph).  There is no CPU / eager fallback.
 """
 import warnings
 
@@ -72,18 +73,20 @@ def check_hyper_parameters(dim_neck, dim_emb, dim_pre, freq):
 
 
 class _Plan:
-    def __init__(self, model, precision):
+    def __init__(self, model, precision, bn_owner=None):
         sd = layers.state_for_packing(model)
         self.precision = precision
-        self.enc_convs = [layers.conv_bn_layer(sd, f"encoder.convolutions.{i}", precision, "relu") for i in range(3)]
+        self.enc_convs = [layers.conv_bn_layer(sd, f"encoder.convolutions.{i}", precision, "relu", bn_owner)
+                          for i in range(3)]
         self.enc_lstm = layers.BiLstmSmall(sd, "encoder.lstm", 2, precision)
         self.lstm1 = layers.lstm_layers(sd, "decoder.lstm1", 1, precision)
-        self.dec_convs = [layers.conv_bn_layer(sd, f"decoder.convolutions.{i}", precision, "relu") for i in range(3)]
+        self.dec_convs = [layers.conv_bn_layer(sd, f"decoder.convolutions.{i}", precision, "relu", bn_owner)
+                          for i in range(3)]
         self.lstm2 = layers.lstm_layers(sd, "decoder.lstm2", 2, precision)
         self.linear = ops.ConvGemm(*packing.pack_linear(sd["decoder.linear_projection.linear_layer.weight"],
                                                         sd["decoder.linear_projection.linear_layer.bias"], precision),
                                    tag="linear")
-        self.postnet = layers.Postnet(sd, "postnet", precision)
+        self.postnet = layers.Postnet(sd, "postnet", precision, bn_owner)
 
 
 class AutoVC(layers.PlanOwner, nn.Module):
@@ -93,7 +96,10 @@ class AutoVC(layers.PlanOwner, nn.Module):
     three-product tensor-core arithmetic, ~3e-5 from the fp32 reference | "fp16x2": fp16 activations x two-term
     fp16 weights, two products, ~4e-4, 1.45x faster | "tf32": one TF32 pass, ~1e-3 | "bf16": one bf16 pass, ~1e-2),
     ``persistent_lstm`` (one cooperative launch per LSTM layer instead of one launch per frame),
-    ``collect_taps`` (keep fp32 copies of every stage in ``self.taps`` for parity tests)."""
+    ``collect_taps`` (keep fp32 copies of every stage in ``self.taps`` for parity tests),
+    ``bn_stats`` ("running" default: every BatchNorm folded with its running statistics, eval semantics | "batch":
+    every BatchNorm normalises with the statistics of the call's B x T frames and updates running_mean, running_var
+    and num_batches_tracked on the device, as nn.BatchNorm1d in train mode -- how the reference's notebooks convert)."""
 
     def __init__(self, dim_neck, dim_emb, dim_pre, freq):
         super().__init__()
@@ -106,11 +112,14 @@ class AutoVC(layers.PlanOwner, nn.Module):
         self.persistent_lstm = True
         self.collect_taps = False
         self.taps = {}
+        self.bn_stats = "running"
         self._cache = layers.PlanCache()
         self._warned_train = False
 
     def _plan(self):
-        return self._cache.get(self, (self.precision,), lambda: _Plan(self, self.precision))
+        batch = layers.check_bn_stats(self.bn_stats) == "batch"
+        return self._cache.get(self, (self.precision, self.bn_stats),
+                               lambda: _Plan(self, self.precision, self if batch else None), skip_bn_stats=batch)
 
     # hooks of the AdaIN "2" variants (factory/_adain.py); the plain model uses the mel as is and the plain postnet
     def _encoder_features(self, x, plan, B, T):
@@ -122,9 +131,10 @@ class AutoVC(layers.PlanOwner, nn.Module):
     @ops.on_device_of_input
     @torch.no_grad()
     def forward(self, x, c_org, c_trg):
-        if self.training and not self._warned_train:
+        if self.training and not self._warned_train and self.bn_stats != "batch":
             warnings.warn("autoformer_b200.AutoVC runs the eval-mode forward (BatchNorm running statistics) "
-                          "even in train() mode; it is an inference path")
+                          "even in train() mode; it is an inference path (bn_stats='batch' selects train-mode "
+                          "BatchNorm statistics)")
             self._warned_train = True
         if x.dim() == 4:
             x = x.squeeze(1)                                    # AutoVC.py:46
@@ -135,6 +145,8 @@ class AutoVC(layers.PlanOwner, nn.Module):
         F, H = self.freq, self.dim_neck
         if T % F != 0:
             raise IndexError(f"T={T} is not a multiple of freq={F} (reference indexes i+freq-1, AutoVC.py:60-66)")
+        if layers.check_bn_stats(self.bn_stats) == "batch" and B * T == 1:
+            raise ValueError(f"Expected more than 1 value per channel when training, got input size {(B, 512, T)}")
         plan = self._plan()
         prec = plan.precision
         dev = x.device

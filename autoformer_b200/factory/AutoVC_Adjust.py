@@ -17,6 +17,7 @@ class AutoVC_Adjust(AutoVC):
 
     def _adjust(self, x, emb):
         self.adjust.precision = self.precision
+        self.adjust.bn_stats = self.bn_stats                                    # governs the Adjust BatchNorms too
         self.adjust.persistent_lstm = self.persistent_lstm
         return self.adjust(x, emb)
 

@@ -17,6 +17,7 @@ class MetaConv_Adjust(MetaBase):
 
     def _adjust(self, x, emb):
         self.adjust.precision = self.precision
+        self.adjust.bn_stats = self.bn_stats                                    # governs the Adjust BatchNorms too
         return self.adjust(x, emb)
 
     @ops.on_device_of_input

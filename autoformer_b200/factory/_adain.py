@@ -26,8 +26,9 @@ class AdaIN(nn.Module):
 
 
 class AdaINPlan:
-    def __init__(self, sd, precision):
-        self.pre = [layers.conv_bn_layer(sd, f"encoder.feature_pre_extract.{i}", precision, "none") for i in range(3)]
+    def __init__(self, sd, precision, bn_owner=None):
+        self.pre = [layers.conv_bn_layer(sd, f"encoder.feature_pre_extract.{i}", precision, "none", bn_owner)
+                    for i in range(3)]
         self.combine = [ops.ConvGemm(*packing.pack_conv(sd[f"postnet.feature_last_combine.{i}.0.conv.weight"],
                                                         sd[f"postnet.feature_last_combine.{i}.0.conv.bias"], precision),
                                      act="none", tag="conv") for i in range(3)]
@@ -49,10 +50,12 @@ class AdaINMixin:
         self._target_stats = None
 
     def _adain_plan(self):
+        batch = layers.check_bn_stats(self.bn_stats) == "batch"
+
         def build():
             sd = layers.state_for_packing(self)
-            return AdaINPlan(sd, self.precision)
-        return self._adain_cache.get(self, (self.precision,), build)
+            return AdaINPlan(sd, self.precision, self if batch else None)
+        return self._adain_cache.get(self, (self.precision, self.bn_stats), build, skip_bn_stats=batch)
 
     # ---- hooks called by the base forward
     def _encoder_features(self, x, plan, B, T):

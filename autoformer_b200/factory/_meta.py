@@ -159,16 +159,16 @@ class MixerPlan:
 
 
 class BlockPlan:
-    def __init__(self, sd, prefix, kind, crop, precision):
+    def __init__(self, sd, prefix, kind, crop, precision, bn_owner=None):
         f = lambda k: sd[f"{prefix}.{k}"].float().contiguous()
         self.kind, self.crop, self.precision = kind, crop, precision
         self.gn1 = (f("norm1.weight"), f("norm1.bias"))
         self.gn2 = (f("norm2.weight"), f("norm2.bias"))
         if kind == "conv":
-            self.token_mixer = layers.conv_bn_layer(sd, f"{prefix}.token_mixer", precision, "relu")
-        self.conv_1 = layers.conv_bn_layer(sd, f"{prefix}.conv_1", precision, "relu")
+            self.token_mixer = layers.conv_bn_layer(sd, f"{prefix}.token_mixer", precision, "relu", bn_owner)
+        self.conv_1 = layers.conv_bn_layer(sd, f"{prefix}.conv_1", precision, "relu", bn_owner)
         self.mlp = MixerPlan(sd, f"{prefix}.mlp", crop, 8, 88, precision)
-        self.conv_2 = layers.conv_bn_layer(sd, f"{prefix}.conv_2", precision, "relu")
+        self.conv_2 = layers.conv_bn_layer(sd, f"{prefix}.conv_2", precision, "relu", bn_owner)
 
     def __call__(self, x, B, L, want_op):
         """x fp32 [B][L][512] -> (x' fp32, x' operand format or None)   (MetaBlock.forward, MetaPool.py:66-77)."""
@@ -193,24 +193,24 @@ class BlockPlan:
 
 
 class _Plan:
-    def __init__(self, model, kind, precision):
+    def __init__(self, model, kind, precision, bn_owner=None):
         sd = layers.state_for_packing(model)
         self.precision = precision
         emb = lambda p: ops.ConvGemm(*packing.pack_conv(sd[p + ".weight"].float(), sd[p + ".bias"].float(), precision),
                                      tag="conv")
         self.enc_embed = emb("encoder.embding.proj")
-        self.enc_blocks = [BlockPlan(sd, f"encoder.metablock.{i}", kind, 176, precision) for i in range(3)]
-        self.enc_out_conv = layers.conv_bn_layer(sd, "encoder.output_conv", precision, "relu")
+        self.enc_blocks = [BlockPlan(sd, f"encoder.metablock.{i}", kind, 176, precision, bn_owner) for i in range(3)]
+        self.enc_out_conv = layers.conv_bn_layer(sd, "encoder.output_conv", precision, "relu", bn_owner)
         self.enc_mlp = MixerPlan(sd, "encoder.mlp", 176, 16, 2 * model.dim_neck, precision)
         self.dec_embed = emb("decoder.embding.proj")
-        self.dec_block = BlockPlan(sd, "decoder.metablock.0", kind, 344, precision)
-        self.dec_out_conv_1 = layers.conv_bn_layer(sd, "decoder.output_conv_1", precision, "relu")
+        self.dec_block = BlockPlan(sd, "decoder.metablock.0", kind, 344, precision, bn_owner)
+        self.dec_out_conv_1 = layers.conv_bn_layer(sd, "decoder.output_conv_1", precision, "relu", bn_owner)
         self.dec_mlp = MixerPlan(sd, "decoder.mlp", 344, 8, 88, precision)
-        self.dec_out_conv_2 = layers.conv_bn_layer(sd, "decoder.output_conv_2", precision, "relu")
+        self.dec_out_conv_2 = layers.conv_bn_layer(sd, "decoder.output_conv_2", precision, "relu", bn_owner)
         self.linear = ops.ConvGemm(*packing.pack_linear(sd["decoder.linear_projection.linear_layer.weight"],
                                                         sd["decoder.linear_projection.linear_layer.bias"], precision),
                                    tag="linear")
-        self.postnet = layers.Postnet(sd, "postnet", precision)
+        self.postnet = layers.Postnet(sd, "postnet", precision, bn_owner)
 
 
 class MetaBase(layers.PlanOwner, nn.Module):
@@ -225,11 +225,15 @@ class MetaBase(layers.PlanOwner, nn.Module):
         self.precision = "fp32"
         self.collect_taps = False
         self.taps = {}
+        self.bn_stats = "running"       # "batch": train-mode BatchNorm statistics (see autoformer_b200.AutoVC)
         self._cache = layers.PlanCache()
         self._warned_train = False
 
     def _plan(self):
-        return self._cache.get(self, (self.precision,), lambda: _Plan(self, self.KIND, self.precision))
+        batch = layers.check_bn_stats(self.bn_stats) == "batch"
+        return self._cache.get(self, (self.precision, self.bn_stats),
+                               lambda: _Plan(self, self.KIND, self.precision, self if batch else None),
+                               skip_bn_stats=batch)
 
     # hooks of the AdaIN "2" variants (factory/_adain.py)
     def _encoder_features(self, x, plan, B, T):
@@ -241,8 +245,9 @@ class MetaBase(layers.PlanOwner, nn.Module):
     @ops.on_device_of_input
     @torch.no_grad()
     def forward(self, x, c_org, c_trg):
-        if self.training and not self._warned_train:
-            warnings.warn("autoformer_b200 Meta models run the eval-mode forward (BatchNorm running statistics)")
+        if self.training and not self._warned_train and self.bn_stats != "batch":
+            warnings.warn("autoformer_b200 Meta models run the eval-mode forward (BatchNorm running statistics); "
+                          "bn_stats='batch' selects train-mode BatchNorm statistics")
             self._warned_train = True
         if x.dim() == 4:
             x = x.squeeze(1)
@@ -258,6 +263,7 @@ class MetaBase(layers.PlanOwner, nn.Module):
                                "channel mismatch in PatchEmbed, as in the reference")
         if T % F != 0:
             raise IndexError(f"T={T} is not a multiple of freq={F}")
+        layers.check_bn_stats(self.bn_stats)
         plan = self._plan()
         prec, dev = plan.precision, x.device
         taps = self.taps if self.collect_taps else None

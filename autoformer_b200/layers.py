@@ -2,6 +2,7 @@
 import os
 
 import torch
+import torch.nn as nn
 
 from . import ops, packing
 from .packing import TORCH_DTYPE
@@ -41,6 +42,25 @@ def plan_to(obj, device, _seen=None):
     return obj
 
 
+def bn_stat_buffer_ids(module):
+    """ids of the running_mean / running_var / num_batches_tracked buffers of every BatchNorm under `module`."""
+    ids = set()
+    for m in module.modules():
+        if isinstance(m, nn.modules.batchnorm._BatchNorm):
+            ids.update(id(t) for t in (m.running_mean, m.running_var, m.num_batches_tracked) if t is not None)
+    return ids
+
+
+BN_STATS = ("running", "batch")
+
+
+def check_bn_stats(mode):
+    if mode not in BN_STATS:
+        raise ValueError(f"bn_stats={mode!r}: 'running' (BatchNorm folded with its running statistics) or 'batch' "
+                         "(statistics of each call's batch, updating the running buffers: nn.BatchNorm1d in train mode)")
+    return mode
+
+
 class PlanCache:
     """Re-pack weights only when a parameter/buffer was replaced, moved or modified.
 
@@ -58,10 +78,13 @@ class PlanCache:
         self.frozen = False
 
     @staticmethod
-    def fingerprint(module, extra=(), contents=True):
+    def fingerprint(module, extra=(), contents=True, skip_bn_stats=False):
         items = []
         by_dev = {}
+        skip = bn_stat_buffer_ids(module) if skip_bn_stats else ()
         for t in list(module.parameters()) + list(module.buffers()):
+            if id(t) in skip:
+                continue
             items.append((t.data_ptr(), t._version, str(t.device), tuple(t.shape), str(t.dtype)))
             if contents and t.numel() and t.is_floating_point():
                 by_dev.setdefault(t.device, []).append(t.detach())
@@ -77,10 +100,13 @@ class PlanCache:
         self.key = None
         self.plan = None
 
-    def get(self, module, extra, builder):
+    def get(self, module, extra, builder, skip_bn_stats=False):
+        """``skip_bn_stats``: leave the BatchNorm running buffers out of the key -- a batch-statistics plan does not
+        read them at packing time, and every one of its forwards updates them, which would otherwise re-pack the plan
+        on the next call."""
         if self.frozen and self.plan is not None and self.key is not None and self.key[1] == tuple(extra):
             return self.plan
-        key = self.fingerprint(module, extra, True)
+        key = self.fingerprint(module, extra, True, skip_bn_stats)
         if key != self.key:
             plan = builder()
             if PACK_ON_CPU:
@@ -117,8 +143,50 @@ class PlanOwner:
         return self
 
 
-def conv_bn_layer(sd, prefix, precision, act):
-    """nn.Sequential(ConvNorm(k5,p2), BatchNorm1d) (+act) -> one packed conv (factory/AutoVC.py:26-39)."""
+class BatchStatsConvBn:
+    """nn.Sequential(ConvNorm(k5,p2), BatchNorm1d) (+act) with the BatchNorm in training mode: each call normalises with
+    the statistics of its own B x T rows and updates the module's running buffers, as the reference's notebooks run
+    every such layer (they never call .eval(), SURVEY.md fact 1).
+
+    Three launches after the conv's own: the conv (its bias, nothing folded) writes v as exact fp32; avc_bn_batch_stats
+    reduces v per channel and updates running_mean / running_var / num_batches_tracked on the device;
+    avc_bn_apply writes act(scale v + shift) (+ residual) where the folded layer's epilogue would have.  The buffers
+    are read from the live nn.BatchNorm1d at every call (not from the packing-time state_dict), so ``state_dict()``
+    shows the updates and momentum / eps are the module's own."""
+
+    def __init__(self, sd, prefix, precision, act, bn):
+        self.conv = ops.ConvGemm(*packing.pack_conv(sd[f"{prefix}.0.conv.weight"], sd[f"{prefix}.0.conv.bias"],
+                                                    precision), act="none", tag="conv")
+        self.gamma = sd[f"{prefix}.1.weight"].detach().float().contiguous()
+        self.beta = sd[f"{prefix}.1.bias"].detach().float().contiguous()
+        self.bn = bn
+        self.act = act
+        self.precision = precision
+        self.C = self.gamma.numel()
+        if bn.running_mean is None:
+            raise ValueError(f"{prefix}.1: batch statistics need the running buffers (track_running_stats=True)")
+
+    def __call__(self, srcs, B, T, out=None, out2=None, residual=None, res_after=False):
+        """Same outputs as ConvGemm.__call__ with the BatchNorm folded: out (operand format) and / or out2 (fp32),
+        residual fp32 added before the activation, or after it with res_after."""
+        if B * T <= 1:
+            raise ValueError(f"Expected more than 1 value per channel when training, got input size {(B, self.C, T)}")
+        bn = self.bn
+        v = torch.empty(B * T, self.C, dtype=torch.float32, device=self.gamma.device)
+        self.conv(srcs, B, T, out2=v)
+        ss = ops.bn_batch_stats(v, self.gamma, self.beta, bn.eps, bn.momentum, bn.running_mean, bn.running_var,
+                                bn.num_batches_tracked)
+        return ops.bn_apply(v, ss, B, T, self.act, out=out, out2=out2, residual=residual, res_after=res_after,
+                            out_fmt=self.precision)
+
+
+def conv_bn_layer(sd, prefix, precision, act, bn_owner=None):
+    """nn.Sequential(ConvNorm(k5,p2), BatchNorm1d) (+act) -> one packed conv (factory/AutoVC.py:26-39).
+
+    bn_owner None: the BatchNorm folded into the conv with its running statistics (eval semantics).  bn_owner = the
+    module `prefix` is relative to: batch statistics (``BatchStatsConvBn``) on that module's live BatchNorm."""
+    if bn_owner is not None:
+        return BatchStatsConvBn(sd, prefix, precision, act, bn_owner.get_submodule(f"{prefix}.1"))
     w, b = packing.fold_bn(sd[f"{prefix}.0.conv.weight"], sd[f"{prefix}.0.conv.bias"], sd[f"{prefix}.1.weight"],
                            sd[f"{prefix}.1.bias"], sd[f"{prefix}.1.running_mean"], sd[f"{prefix}.1.running_var"])
     return ops.ConvGemm(*packing.pack_conv(w, b, precision), act=act, tag="conv")
@@ -317,9 +385,9 @@ class BiLstmSmall:
 class Postnet:
     """Five conv+BN layers, tanh on the first four, residual add fused into the last (factory/AutoVC.py:117-179,206-209)."""
 
-    def __init__(self, sd, prefix, precision):
+    def __init__(self, sd, prefix, precision, bn_owner=None):
         self.precision = precision
-        self.convs = [conv_bn_layer(sd, f"{prefix}.convolutions.{i}", precision, "tanh" if i < 4 else "none")
+        self.convs = [conv_bn_layer(sd, f"{prefix}.convolutions.{i}", precision, "tanh" if i < 4 else "none", bn_owner)
                       for i in range(5)]
 
     def hidden(self, mel_op, B, T, taps=None):

@@ -819,6 +819,78 @@ def adain(x, x_stats, t_stats, precision, want_f32=False):
     return out_op, out_f32
 
 
+# ------------------------------------------------------------------------------------------------ batch-statistics BatchNorm
+def bn_batch_stats(v, gamma, beta, eps=1e-5, momentum=0.1, running_mean=None, running_var=None,
+                   num_batches_tracked=None, scale_shift=None):
+    """v [rows][C] fp32 (row stride >= C) -> scale_shift [2][C] fp32 = (gamma / sqrt(var + eps), beta - mean * scale)
+    with the statistics of all rows, as nn.BatchNorm1d in training mode; updates the running buffers in place on the
+    device (momentum None: cumulative average).  Raises ValueError, as torch does, for a single row."""
+    lib = _lib.load()
+    _require_cuda(v, gamma, beta, running_mean, running_var, num_batches_tracked)
+    assert v.dtype == torch.float32 and v.dim() == 2 and v.stride(1) == 1
+    rows, C = v.shape
+    if rows <= 1:
+        raise ValueError(f"Expected more than 1 value per channel when training, got input size {(rows, C)}")
+    for t in (gamma, beta, running_mean, running_var):
+        assert t is None or (t.dtype == torch.float32 and t.is_contiguous() and t.numel() == C)
+    assert (running_mean is None) == (running_var is None)
+    if num_batches_tracked is not None:
+        assert num_batches_tracked.dtype == torch.int64 and num_batches_tracked.numel() == 1
+    if momentum is None and (num_batches_tracked is None or running_mean is None):
+        raise ValueError("momentum=None (cumulative average) needs the running buffers and num_batches_tracked")
+    if scale_shift is None:
+        scale_shift = torch.empty(2, C, dtype=torch.float32, device=v.device)
+    assert scale_shift.dtype == torch.float32 and scale_shift.is_contiguous() and scale_shift.shape == (2, C)
+    # from the stream-ordered caching allocator, so layers run on two streams never share it
+    scratch = torch.empty(2 + 2 * _lib.BN_MAX_PARTS * C, dtype=torch.float64, device=v.device)
+    with PROFILER.span("bn_stats", bytes=4.0 * rows * C, launches=2):
+        _lib.check(lib.avc_bn_batch_stats(v.data_ptr(), rows, C, v.stride(0), gamma.data_ptr(), beta.data_ptr(),
+                                          float(eps), 0.0 if momentum is None else float(momentum),
+                                          1 if momentum is None else 0, _ptr(running_mean), _ptr(running_var),
+                                          _ptr(num_batches_tracked), scale_shift.data_ptr(), scratch.data_ptr(),
+                                          _stream()), "avc_bn_batch_stats")
+    return scale_shift
+
+
+def bn_apply(v, scale_shift, B, T, act="none", out=None, out2=None, residual=None, res_after=False, out_fmt=None,
+             round_tf32=True):
+    """act(scale * v + shift) (+ residual before or after the activation) for v [B*T][C] fp32 -> out [B][rows][C']
+    (operand format `out_fmt`, written at rows 0..T-1) and / or out2 [B*T][C] exact fp32."""
+    lib = _lib.load()
+    _require_cuda(v, scale_shift, out, out2, residual)
+    assert v.dtype == torch.float32 and v.dim() == 2 and v.stride(1) == 1 and v.shape[0] == B * T
+    C = v.shape[1]
+    assert scale_shift.dtype == torch.float32 and scale_shift.is_contiguous() and scale_shift.shape == (2, C)
+    assert out is not None or out2 is not None
+    d = _lib.BnApplyDesc()
+    d.v, d.v_ld, d.scale_shift = v.data_ptr(), v.stride(0), scale_shift.data_ptr()
+    d.B, d.T, d.C = B, T, C
+    d.act = _lib.ACTS[act]
+    nbytes = 4.0 * B * T * C
+    if residual is not None:
+        assert residual.dtype == torch.float32 and residual.stride(-1) == 1 and residual.shape[-1] >= C
+        d.residual, d.res_ld, d.res_after_act = residual.data_ptr(), residual.stride(-2), 1 if res_after else 0
+        nbytes += 4.0 * B * T * C
+    if out is not None:
+        fmt = out_fmt
+        assert fmt is not None, "bn_apply: out needs its operand format (a precision name)"
+        assert out.dim() == 3 and out.shape[0] == B and out.shape[1] >= T and out.stride(2) == 1
+        assert out.dtype == TORCH_DTYPE[fmt] and out.shape[2] >= packing.act_channels(C, fmt)
+        assert out.stride(0) == out.shape[1] * out.stride(1)
+        d.out, d.out_ld, d.out_rows_per_utt, d.out_row0 = out.data_ptr(), out.stride(1), out.shape[1], 0
+        d.out_dtype = _dt(fmt)
+        d.out_round_tf32 = 1 if (round_tf32 and out.dtype == torch.float32) else 0
+        nbytes += B * T * packing.act_channels(C, fmt) * out.element_size()
+    if out2 is not None:
+        assert out2.dtype == torch.float32 and out2.dim() == 2 and out2.stride(1) == 1 and out2.shape[0] == B * T
+        assert out2.shape[1] >= C
+        d.out2, d.out2_ld = out2.data_ptr(), out2.stride(0)
+        nbytes += 4.0 * B * T * C
+    with PROFILER.span("bn_apply", bytes=nbytes):
+        _lib.check(lib.avc_bn_apply(ctypes.byref(d), _stream()), "avc_bn_apply")
+    return out if out is not None else out2
+
+
 # ------------------------------------------------------------------------------------------------ Audio2Mel front end
 def audio_frames(audio, pad, hop, rows, precision):
     """audio [B][L] fp32 -> reflect-padded signal as rows of `hop` samples [B][rows][hop] in operand format."""

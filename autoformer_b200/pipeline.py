@@ -91,6 +91,8 @@ class StreamingConverter:
     the result of the PREVIOUS submission (or None): while batch i computes, batch i+1 uploads and batch i-1
     downloads.  ``flush()`` returns the last result.  Results are pinned host tensors owned by the converter and are
     overwritten two submissions later (double buffering) -- copy them if they must live longer.
+    The model runs in submission order on the one compute stream, so a model with ``bn_stats = "batch"`` updates its
+    BatchNorm running buffers in that order too.
     """
 
     def __init__(self, model, device=None):
@@ -175,9 +177,14 @@ def convert_batches(model, batches, reduce=None, pair_below=PAIR_BELOW):
     every length bucket) therefore run TWO AT A TIME on two streams, with each persistent LSTM grid capped at half of the
     device (``ops.LSTM_CTA_BUDGET``) so that both cooperative launches are resident together -- measured
     (scripts/two_stream_probe.py): 212 x 1024 + 180 x 992 frames 71.6 -> 52.3 ms, outputs bit-equal to the one-stream
-    run.  Utterances stay independent and every batch keeps its exact length; only the schedule changes."""
+    run.  Utterances stay independent and every batch keeps its exact length; only the schedule changes.
+
+    A model with ``bn_stats = "batch"`` updates its BatchNorm running buffers on every call, so the order of the calls
+    matters: its batches run in the order given on the current stream, exactly as a plain loop of ``model(*b)``."""
     from . import ops
     reduce = reduce or (lambda out: out)
+    if getattr(model, "bn_stats", "running") == "batch":
+        return [reduce(model(*b)) for b in batches]
     results = [None] * len(batches)
     small = [i for i, b in enumerate(batches) if 64 < b[0].shape[0] <= pair_below]
     # (batches of <= 64 utterances take the weight-stationary kernels, whose grids fill the device: no pairing)

@@ -419,6 +419,54 @@ int avc_adain(const float* x, const float* x_stats, const float* t_stats, float*
               int out_round_tf32, long long rows, int C, void* stream);
 
 /*
+ * Batch-statistics BatchNorm: nn.BatchNorm1d in training mode (torch.nn.functional.batch_norm, training=True), which is
+ * how the reference's notebooks run every conv + BN layer -- they never call .eval() (conversion.ipynb cells 3 and 8,
+ * util/evaluate.py; layers factory/AutoVC.py:26-39,117-171, factory/MetaPool.py:37-43,92-99, factory/Adjust.py:17-20,
+ * factory/AutoVC2.py:54-60).  The conv runs unfolded through avc_conv_gemm (its own bias, AVC_ACT_NONE) into
+ * v [rows][v_ld] fp32 (out2); these two calls then normalise it.
+ *
+ * avc_bn_batch_stats: per channel c of v (C channels, C % 4 == 0, rows > 1), over ALL rows:
+ *   mean_c, var_c (biased);  scale_shift[0][c] = gamma_c / sqrt(var_c + eps),  scale_shift[1][c] = beta_c - mean_c * scale_c
+ *   running_mean_c <- (1 - m) running_mean_c + m mean_c
+ *   running_var_c  <- (1 - m) running_var_c  + m var_c * rows / (rows - 1)        (unbiased, as torch)
+ *   *num_batches_tracked += 1
+ *   m = momentum, or 1 / num_batches_tracked (after the increment) when `cumulative` (nn.BatchNorm1d(momentum=None)).
+ *   running_mean / running_var / num_batches_tracked may be NULL (no update; the cumulative average needs all three).
+ *   Two launches: fp64 partial sums of v and v^2 per (row chunk, channel) into `scratch`, then one merge per channel in a
+ *   fixed order -- the result is bitwise reproducible on a given device.  Every input stays on the device: nothing is
+ *   read back to the host.  scratch: 2 + 2 * AVC_BN_MAX_PARTS * C doubles.
+ *
+ * avc_bn_apply: y = act(scale_c * v + shift_c) with an optional fp32 residual added before the activation or after it
+ *   (res_after_act: x + relu(BN(conv)), factory/MetaPool.py:68,75; the postnet's mel + BN(conv), factory/AutoVC.py:206-209).
+ *   act: AVC_ACT_NONE / RELU / TANH.  Row r = b * T + t of v, residual and out2; `out` (operand format, the stores of the
+ *   GEMM epilogue: out_dtype codes as avc_gemm_desc) at row b * out_rows_per_utt + out_row0 + t.  Any of out / out2.
+ */
+#define AVC_BN_MAX_PARTS 256
+int avc_bn_batch_stats(const float* v, long long rows, int C, long long v_ld, const float* gamma, const float* beta,
+                       float eps, float momentum, int cumulative, float* running_mean, float* running_var,
+                       long long* num_batches_tracked, float* scale_shift, double* scratch, void* stream);
+
+typedef struct avc_bn_apply_desc {
+  const float* v;            /* [B*T][v_ld] fp32 */
+  long long v_ld;
+  const float* scale_shift;  /* [2][C] fp32 from avc_bn_batch_stats */
+  int B, T, C;
+  int act;                   /* AVC_ACT_NONE / AVC_ACT_RELU / AVC_ACT_TANH */
+  const float* residual;     /* optional fp32 [B*T][res_ld] */
+  long long res_ld;
+  int res_after_act;         /* add the residual after the activation instead of before it */
+  void* out;                 /* optional operand-format output [B][out_rows_per_utt][out_ld] */
+  long long out_ld;
+  int out_rows_per_utt, out_row0;
+  int out_dtype;             /* 0 fp32, 1 bf16, 2 split bf16, 3 fp16, 4 split fp16 */
+  int out_round_tf32;
+  float* out2;               /* optional exact fp32 [B*T][out2_ld] */
+  long long out2_ld;
+} avc_bn_apply_desc;
+
+int avc_bn_apply(const avc_bn_apply_desc* d, void* stream);
+
+/*
  * Audio2Mel front end (melgan/modules.py:26-69): reflect-pad by (n_fft - hop)/2, STFT(n_fft, hop, hann, center=False),
  * magnitude, mel filter bank, log10(clamp(., 1e-5)).  The STFT runs as an implicit-GEMM convolution on the tensor cores:
  * the padded signal is viewed as rows of `hop` samples (hop = 256 "channels"), a frame is n_fft / hop = 4 consecutive
