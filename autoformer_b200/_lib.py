@@ -17,7 +17,8 @@ EXPORTS = ["avc_version", "avc_last_error", "avc_launch_count", "avc_conv_gemm",
            "avc_bilstm_small", "avc_concat_bcast", "avc_linear_l2norm", "avc_linear_rows", "avc_transpose_pad",
            "avc_conv_to_mono_tanh", "avc_gn_stats", "avc_gn_pool_residual", "avc_gn_apply", "avc_patchify",
            "avc_ln_transpose", "avc_meta_decoder_input", "avc_gather_codes", "avc_global_stats", "avc_adain", "avc_audio_frames",
-           "avc_complex_mag", "avc_resblock", "avc_resblock2", "avc_reflect_halo", "avc_bn_batch_stats", "avc_bn_apply"]
+           "avc_complex_mag", "avc_resblock", "avc_resblock2", "avc_reflect_halo", "avc_bn_batch_stats", "avc_bn_apply",
+           "avc_zero_tail"]
 
 
 MAX_SOURCES = 4
@@ -88,6 +89,7 @@ class LstmDesc(ctypes.Structure):
         ("xin_ld", ctypes.c_longlong),
         ("w_ih", ctypes.c_void_p),
         ("bias", ctypes.c_void_p),
+        ("lengths", ctypes.c_void_p),
     ]
 
 
@@ -105,6 +107,7 @@ class LstmWsDesc(ctypes.Structure):
         ("H", ctypes.c_int),
         ("debug_clk", ctypes.c_void_p),
         ("dtype", ctypes.c_int),
+        ("lengths", ctypes.c_void_p),
     ]
 
 
@@ -126,6 +129,7 @@ class LstmStackDesc(ctypes.Structure):
         ("H", ctypes.c_int),
         ("L", ctypes.c_int),
         ("debug_clk", ctypes.c_void_p),
+        ("lengths", ctypes.c_void_p),
     ]
 
 
@@ -239,11 +243,14 @@ def load():
     lib.avc_reflect_halo.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_longlong, ctypes.c_int,
                                      ctypes.c_int, ctypes.c_int, ctypes.c_void_p]
     lib.avc_reflect_halo.restype = ctypes.c_int
+    lib.avc_zero_tail.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_longlong, ctypes.c_int,
+                                  ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]
+    lib.avc_zero_tail.restype = ctypes.c_int
     lib.avc_resblock2.argtypes = [ctypes.POINTER(Resblock2Desc), ctypes.c_void_p]
     lib.avc_resblock2.restype = ctypes.c_int
     lib.avc_bilstm_small.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
                                      ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
-                                     ctypes.c_void_p]
+                                     ctypes.c_void_p, ctypes.c_void_p]
     lib.avc_bilstm_small.restype = ctypes.c_int
     lib.avc_concat_bcast.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
                                      ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,

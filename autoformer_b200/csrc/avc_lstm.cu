@@ -751,12 +751,35 @@ static int lstm_cta_group() {
   return v;
 }
 
+// h_last[b] = hseq_f32[b][lengths[b] - 1] (a padded batch).  The recurrence kernels keep their T - 1 store: a
+// per-utterance comparison in their cell epilogue costs 4-9 registers in every instantiation (-Xptxas -v), so the
+// variable-length form reads the exact fp32 copy of the sequence instead -- the same bits the in-kernel store writes.
+__global__ void __launch_bounds__(256) gather_last_kernel(const float* __restrict__ hseq_f32, const int* __restrict__ lengths,
+                                                          float* __restrict__ h_last, int T, int H) {
+  const int b = blockIdx.x;
+  const float4* src = reinterpret_cast<const float4*>(hseq_f32 + ((long long)b * T + __ldg(lengths + b) - 1) * H);
+  float4* dst = reinterpret_cast<float4*>(h_last + (long long)b * H);
+  for (int i = threadIdx.x; i < H / 4; i += blockDim.x) dst[i] = src[i];
+}
+
 }  // namespace avc
 
 extern "C" int avc_lstm_seq(const avc_lstm_desc* d, void* stream_v) {
   using namespace avc;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
   AVC_REQUIRE(d != nullptr, "avc_lstm_seq: null descriptor");
+  if (d->lengths && d->h_last) {
+    AVC_REQUIRE(d->hseq_f32 != nullptr, "avc_lstm_seq: lengths with h_last need hseq_f32 (h_last is read from it)");
+    avc_lstm_desc full = *d;
+    full.h_last = nullptr;
+    full.lengths = nullptr;
+    const int rc = avc_lstm_seq(&full, stream_v);
+    if (rc != 0) return rc;
+    gather_last_kernel<<<d->B, 256, 0, stream>>>(d->hseq_f32, d->lengths, d->h_last, d->T, d->H);
+    AVC_CHECK_CUDA(cudaGetLastError());
+    count_launch();
+    return 0;
+  }
   AVC_REQUIRE(d->dtype >= AVC_DTYPE_TF32 && d->dtype <= AVC_DTYPE_F16, "avc_lstm_seq: bad dtype %d", d->dtype);
   AVC_REQUIRE(d->gate_group == 16 || d->gate_group == 28 || d->gate_group == 32, "avc_lstm_seq: gate_group %d (16, 28 or 32)",
               d->gate_group);

@@ -60,6 +60,7 @@ struct alignas(64) StackParams {
   unsigned int* grid_barrier;
   long long* debug_clk;               // optional: 16 clock64 stamps per (tick, CTA)
   int B, T, H, L;
+  const int* lengths;                 // optional [B]: h_last[n] is the top layer's h at frame lengths[n] - 1 (NULL: T - 1)
 };
 
 __device__ __forceinline__ uint32_t st_map_to_cta(uint32_t smem_addr, uint32_t rank) {
@@ -95,7 +96,9 @@ struct StackCfg {
   static int smem_bytes(int H) { return h_tiles(H) * kHTile + kRedBytes + kStageBytes + 128 + 1024 /* alignment slack */; }
 };
 
-template <int AR>
+// RAGGED: h_last[n] at frame lengths[n] - 1.  A separate instantiation, because the per-utterance comparison changes
+// the register allocation of the kernel; the fixed-length instantiation is the kernel as it is without lengths.
+template <int AR, bool RAGGED>
 __global__ void __launch_bounds__(StackCfg<AR>::kThreads, 1) lstm_stack_kernel(const __grid_constant__ StackParams p) {
   using Cfg = StackCfg<AR>;
   constexpr int NQ = Cfg::NQ, IT = Cfg::IT;
@@ -370,7 +373,7 @@ __global__ void __launch_bounds__(StackCfg<AR>::kThreads, 1) lstm_stack_kernel(c
           uint4* o = reinterpret_cast<uint4*>(hs_l + ((long long)(t + 1) * p.B + n) * p.H + ug);
           o[0] = make_uint4(pack_f16(h0.x, h0.y), pack_f16(h0.z, h0.w), pack_f16(h1.x, h1.y), pack_f16(h1.z, h1.w));
           o[1] = make_uint4(pack_f16(h2.x, h2.y), pack_f16(h2.z, h2.w), pack_f16(h3.x, h3.y), pack_f16(h3.z, h3.w));
-          if (top && t == p.T - 1 && p.h_last) {
+          if (top && (RAGGED ? is_last_frame(p.lengths, n, t, p.T) : t == p.T - 1) && p.h_last) {
             float4* hl = reinterpret_cast<float4*>(p.h_last + (long long)n * p.H + ug);
             hl[0] = h0; hl[1] = h1; hl[2] = h2; hl[3] = h3;
           }
@@ -394,10 +397,10 @@ __global__ void __launch_bounds__(StackCfg<AR>::kThreads, 1) lstm_stack_kernel(c
   }
 }
 
-template <int AR>
+template <int AR, bool RAGGED>
 static int launch_stack(const StackParams& p, const avc_lstm_stack_desc* d, cudaStream_t stream) {
   using Cfg = StackCfg<AR>;
-  auto kern = lstm_stack_kernel<AR>;
+  auto kern = lstm_stack_kernel<AR, RAGGED>;
   const int smem = Cfg::smem_bytes(d->H);
   AVC_REQUIRE(smem <= 227 * 1024, "avc_lstm_stack_ws: H=%d B=%d needs %d bytes of shared memory", d->H, d->B, smem);
   static int configured[PerDeviceOnce::kMaxDevices] = {};   // largest size set so far, per device
@@ -482,11 +485,16 @@ extern "C" int avc_lstm_stack_ws(const avc_lstm_stack_desc* d, void* stream_v) {
   p.xproj0 = d->xproj0;
   p.hs = static_cast<__half*>(d->hs);
   p.h_last = d->h_last;
+  p.lengths = d->lengths;
   p.grid_barrier = d->grid_barrier;
   p.debug_clk = d->debug_clk;
   p.B = d->B;
   p.T = d->T;
   p.H = d->H;
   p.L = d->L;
-  return ar == 16 ? launch_stack<16>(p, d, stream) : ar == 32 ? launch_stack<32>(p, d, stream) : launch_stack<64>(p, d, stream);
+  if (p.lengths)
+    return ar == 16 ? launch_stack<16, true>(p, d, stream) : ar == 32 ? launch_stack<32, true>(p, d, stream)
+                                                          : launch_stack<64, true>(p, d, stream);
+  return ar == 16 ? launch_stack<16, false>(p, d, stream) : ar == 32 ? launch_stack<32, false>(p, d, stream)
+                                                         : launch_stack<64, false>(p, d, stream);
 }

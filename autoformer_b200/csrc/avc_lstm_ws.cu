@@ -50,6 +50,7 @@ struct alignas(64) WsParams {
   long long* debug_clk;   // optional: 8 clock64 stamps per (frame, CTA)
   int B, T, H;
   int chunks;             // 64-channel chunks of this CTA's K-slice
+  const int* lengths;     // optional [B]: h_last[n] is h at frame lengths[n] - 1 (NULL: T - 1)
 };
 
 template <int AR, int S>
@@ -328,7 +329,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) lstm_ws_kernel(const __grid_con
               *reinterpret_cast<uint2*>(o + p.H) = make_uint2(pack_bf16(lx, ly), pack_bf16(lz, lw));
             }
             if (p.hseq_f32) *reinterpret_cast<float4*>(p.hseq_f32 + orow * p.H + ug + i * 4) = h;
-            if (p.h_last && t == p.T - 1) *reinterpret_cast<float4*>(p.h_last + (long long)n * p.H + ug + i * 4) = h;
+            if (p.h_last && is_last_frame(p.lengths, n, t, p.T)) *reinterpret_cast<float4*>(p.h_last + (long long)n * p.H + ug + i * 4) = h;
           }
           fence_proxy_async_global();   // order the h stores before later async-proxy (TMA) reads
         }
@@ -426,6 +427,7 @@ extern "C" int avc_lstm_seq_ws(const avc_lstm_ws_desc* d, void* stream_v) {
   p.hseq = static_cast<__nv_bfloat16*>(d->hseq);
   p.hseq_f32 = d->hseq_f32;
   p.h_last = d->h_last;
+  p.lengths = d->lengths;
   p.grid_barrier = d->grid_barrier;
   p.debug_clk = d->debug_clk;
   p.B = d->B;

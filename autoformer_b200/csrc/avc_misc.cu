@@ -60,13 +60,34 @@ __global__ void __launch_bounds__(256) concat_bcast_kernel(const float* __restri
 // ---------------------------------------------------------------------------------------------
 constexpr int kSmallWarps = 8;   // 4 utterances x 2 directions per CTA
 
+// Padded utterance (Tb < T valid frames): direction `dir`'s half of out rows Tb..T-1 and of codes Tb/freq..T/freq-1 is
+// written as 0, by `nthreads` threads of index `tid`.  Zero is all-zero bits in every out_mode.
+__device__ __noinline__ void zero_bilstm_tail(void* out, int out_mode, float* codes, int b, int T, int H, int freq, int Tb,
+                                              int dir, int tid, int nthreads) {
+  if (out) {
+    const int es = out_mode == 0 ? 4 : 2;
+    const int parts = out_mode == 2 ? 2 : 1;               // split bf16: [hi(2H) | lo(2H)]
+    char* base = static_cast<char*>(out);
+    for (int i = tid; i < (T - Tb) * parts * H; i += nthreads) {
+      const int u = i % H, part = (i / H) % parts, t = Tb + i / (H * parts);
+      const long long e = ((long long)b * T + t) * (2LL * parts * H) + part * 2 * H + dir * H + u;
+      if (es == 4) reinterpret_cast<float*>(base)[e] = 0.0f; else reinterpret_cast<unsigned short*>(base)[e] = 0;
+    }
+  }
+  if (codes) {
+    const int n_codes = T / freq;
+    for (int i = tid; i < (n_codes - Tb / freq) * H; i += nthreads)
+      codes[((long long)b * n_codes + Tb / freq + i / H) * (2LL * H) + dir * H + i % H] = 0.0f;
+  }
+}
+
 // REGW (H == 32 only): every lane keeps the 4 x 32 recurrent weights of its hidden unit in registers and h_{t-1} is
 // exchanged with warp shuffles, so a step issues 32 SHFL + 128 FMA instead of 64 shared-memory loads (the shared-memory
 // variant is bound by those loads: 2.2 K cycles per step against ~0.6 K here).
 template <int UPL, bool REGW>   // hidden units per lane: 1 (H <= 32) or 2 (H <= 64)
 __global__ void __launch_bounds__(kSmallWarps * 32) bilstm_small_kernel(
     const float* __restrict__ xproj, const float* __restrict__ w_hh, void* __restrict__ out, int out_mode, int round,
-    float* __restrict__ codes, int B, int T, int H, int freq) {
+    float* __restrict__ codes, int B, int T, int H, int freq, const int* __restrict__ lengths) {
   extern __shared__ float4 smem4[];
   constexpr int HP = UPL * 32;
   float4* Wt = smem4;                                              // [2][H][HP]
@@ -92,9 +113,10 @@ __global__ void __launch_bounds__(kSmallWarps * 32) bilstm_small_kernel(
 
   const int b = blockIdx.x * (kSmallWarps / 2) + (warp >> 1);
   const int dir = warp & 1;
-  if (b >= B) return;
+  if (b >= B) return;          // no CTA barrier past this point: the 4 utterances of a CTA may differ in length
   const float4* W = Wt + dir * H * HP;
   const int n_codes = T / freq;
+  const int Tb = lengths ? __ldg(lengths + b) : T;   // valid frames of this utterance
   float c[UPL];
   float zx[UPL][4];
   for (int e = 0; e < UPL; ++e) c[e] = 0.0f;
@@ -108,21 +130,21 @@ __global__ void __launch_bounds__(kSmallWarps * 32) bilstm_small_kernel(
       for (int g = 0; g < 4; ++g) dst[e][g] = (u < H) ? __ldg(xp + g * H + u) : 0.0f;
     }
   };
-  load_x(dir ? T - 1 : 0, zx);
+  load_x(dir ? Tb - 1 : 0, zx);
   float4 wreg[REGW ? 32 : 1];
   float hprev = 0.0f;
   if (REGW) {
 #pragma unroll
     for (int k = 0; k < 32; ++k) wreg[k] = W[k * HP + lane];
   }
-  for (int s = 0; s < T; ++s) {
-    const int t = dir ? T - 1 - s : s;
+  for (int s = 0; s < Tb; ++s) {
+    const int t = dir ? Tb - 1 - s : s;
     float z[UPL][4];
 #pragma unroll
     for (int e = 0; e < UPL; ++e)
 #pragma unroll
       for (int g = 0; g < 4; ++g) z[e][g] = zx[e][g];
-    if (s + 1 < T) load_x(dir ? t - 1 : t + 1, zx);   // prefetch the next frame's projection
+    if (s + 1 < Tb) load_x(dir ? t - 1 : t + 1, zx);   // prefetch the next frame's projection
     if (REGW) {
 #pragma unroll
       for (int k = 0; k < 32; ++k) {
@@ -186,6 +208,7 @@ __global__ void __launch_bounds__(kSmallWarps * 32) bilstm_small_kernel(
       }
     }
   }
+  if (Tb < T) zero_bilstm_tail(out, out_mode, codes, b, T, H, freq, Tb, dir, lane, 32);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -199,7 +222,8 @@ __global__ void __launch_bounds__(kSmallWarps * 32) bilstm_small_kernel(
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(128) bilstm32_kernel(const float* __restrict__ xproj, const float* __restrict__ w_hh,
                                                        void* __restrict__ out, int out_mode, int round,
-                                                       float* __restrict__ codes, int T, int freq) {
+                                                       float* __restrict__ codes, int T, int freq,
+                                                       const int* __restrict__ lengths) {
   constexpr int H = 32;
   __shared__ __align__(16) float hb[2][H];
   const int tid = threadIdx.x;
@@ -220,22 +244,23 @@ __global__ void __launch_bounds__(128) bilstm32_kernel(const float* __restrict__
   if (tid < 2 * H) (&hb[0][0])[tid] = 0.0f;
   __syncthreads();
   const int n_codes = T / freq;
+  const int Tb = lengths ? __ldg(lengths + b) : T;   // valid frames of this utterance (uniform over the CTA)
   // this lane adds the input projection of gate `part` of its unit to its partial sum (the butterfly spreads it)
   const float* xp = xproj + (long long)b * T * (8LL * H) + dir * 4 * H + part * H + u;
-  auto frame = [&](int s) { return dir ? T - 1 - s : s; };
+  auto frame = [&](int s) { return dir ? Tb - 1 - s : s; };
   constexpr int kPre = 4;                      // projections in flight
   float xq[kPre];
 #pragma unroll
-  for (int i = 0; i < kPre; ++i) xq[i] = i < T ? __ldg(xp + (long long)frame(i) * (8LL * H)) : 0.0f;
+  for (int i = 0; i < kPre; ++i) xq[i] = i < Tb ? __ldg(xp + (long long)frame(i) * (8LL * H)) : 0.0f;
   float c = 0.0f;
-  for (int s0 = 0; s0 < T; s0 += kPre) {
+  for (int s0 = 0; s0 < Tb; s0 += kPre) {
 #pragma unroll
     for (int i = 0; i < kPre; ++i) {
       const int s = s0 + i;
-      if (s >= T) break;
+      if (s >= Tb) break;
       const int t = frame(s);
       const float xv = xq[i];
-      if (s + kPre < T) xq[i] = __ldg(xp + (long long)frame(s + kPre) * (8LL * H));
+      if (s + kPre < Tb) xq[i] = __ldg(xp + (long long)frame(s + kPre) * (8LL * H));
       const float4 h0 = *reinterpret_cast<const float4*>(&hb[s & 1][8 * part]);
       const float4 h1 = *reinterpret_cast<const float4*>(&hb[s & 1][8 * part + 4]);
       const float hk[8] = {h0.x, h0.y, h0.z, h0.w, h1.x, h1.y, h1.z, h1.w};
@@ -281,6 +306,7 @@ __global__ void __launch_bounds__(128) bilstm32_kernel(const float* __restrict__
       __syncthreads();      // h_t complete (and every lane done with h_{t-1}) before the next step
     }
   }
+  if (Tb < T) zero_bilstm_tail(out, out_mode, codes, b, T, H, freq, Tb, dir, tid, 128);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -448,7 +474,7 @@ extern "C" int avc_concat_bcast(const float* seq, const float* vec, void* out, i
 }
 
 extern "C" int avc_bilstm_small(const float* xproj, const float* w_hh, void* out, int out_dtype, int out_round_tf32,
-                                float* codes, int B, int T, int H, int freq, void* stream_v) {
+                                float* codes, int B, int T, int H, int freq, void* stream_v, const int* lengths) {
   using namespace avc;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
   AVC_REQUIRE(xproj && w_hh && (out || codes), "avc_bilstm_small: null buffer");
@@ -463,19 +489,19 @@ extern "C" int avc_bilstm_small(const float* xproj, const float* w_hh, void* out
   // layers): B = 1 1.15 -> 0.78 ms, B = 32 1.47 -> 0.79 ms, but B = 512 0.21 -> 0.24 ms (issue-bound there): small batches only
   static const bool lanes4 = getenv("AVC_BILSTM_WARP") == nullptr;   // AVC_BILSTM_WARP=1: the warp-per-direction kernel (A/B timing)
   if (H == 32 && lanes4 && B <= 128) {
-    bilstm32_kernel<<<2 * B, 128, 0, stream>>>(xproj, w_hh, out, out_dtype, out_round_tf32, codes, T, freq);
+    bilstm32_kernel<<<2 * B, 128, 0, stream>>>(xproj, w_hh, out, out_dtype, out_round_tf32, codes, T, freq, lengths);
   } else if (H == 32) {   // AutoVC "A" (dim_neck = 32): recurrent weights in registers
     auto kern = bilstm_small_kernel<1, true>;
     AVC_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, kSmallWarps * 32, smem, stream>>>(xproj, w_hh, out, out_dtype, out_round_tf32, codes, B, T, H, freq);
+    kern<<<grid, kSmallWarps * 32, smem, stream>>>(xproj, w_hh, out, out_dtype, out_round_tf32, codes, B, T, H, freq, lengths);
   } else if (upl == 1) {
     auto kern = bilstm_small_kernel<1, false>;
     AVC_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, kSmallWarps * 32, smem, stream>>>(xproj, w_hh, out, out_dtype, out_round_tf32, codes, B, T, H, freq);
+    kern<<<grid, kSmallWarps * 32, smem, stream>>>(xproj, w_hh, out, out_dtype, out_round_tf32, codes, B, T, H, freq, lengths);
   } else {
     auto kern = bilstm_small_kernel<2, false>;
     AVC_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, kSmallWarps * 32, smem, stream>>>(xproj, w_hh, out, out_dtype, out_round_tf32, codes, B, T, H, freq);
+    kern<<<grid, kSmallWarps * 32, smem, stream>>>(xproj, w_hh, out, out_dtype, out_round_tf32, codes, B, T, H, freq, lengths);
   }
   AVC_CHECK_CUDA(cudaGetLastError());
   count_launch();
@@ -561,6 +587,38 @@ extern "C" int avc_reflect_halo(void* buf, int B, int rows_per_utt, long long ro
   const long long blocks = (total + 255) / 256;
   reflect_halo_kernel<<<(unsigned)(blocks < 4096 ? blocks : 4096), 256, 0, stream>>>(
       static_cast<uint4*>(buf), rows_per_utt, vec, row0, L, reflect, total);
+  AVC_CHECK_CUDA(cudaGetLastError());
+  count_launch();
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Padded tails of a variable-length batch: rows row0 + lengths[b] .. row0 + T - 1 of utterance b set to zero
+// ---------------------------------------------------------------------------------------------
+namespace avc {
+__global__ void __launch_bounds__(256) zero_tail_kernel(uint4* __restrict__ buf, long long rows_per_utt, int vec_per_row,
+                                                        int row0, int T, const int* __restrict__ lengths) {
+  const int b = blockIdx.y;
+  const int len = __ldg(lengths + b);
+  const long long total = (long long)(T - len) * vec_per_row;
+  uint4* base = buf + (b * rows_per_utt + row0 + len) * vec_per_row;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x)
+    base[i] = make_uint4(0u, 0u, 0u, 0u);
+}
+}  // namespace avc
+
+extern "C" int avc_zero_tail(void* buf, int B, int rows_per_utt, long long row_bytes, int row0, int T, const int* lengths,
+                             void* stream_v) {
+  using namespace avc;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
+  AVC_REQUIRE(buf != nullptr && lengths != nullptr, "avc_zero_tail: null buffer");
+  AVC_REQUIRE(B > 0 && B <= 65535 && T > 0 && row0 >= 0 && rows_per_utt >= row0 + T && row_bytes > 0 && row_bytes % 16 == 0,
+              "avc_zero_tail: bad geometry B=%d rows=%d row_bytes=%lld row0=%d T=%d", B, rows_per_utt, row_bytes, row0, T);
+  const int vec = static_cast<int>(row_bytes / 16);
+  // enough CTAs per utterance for its longest possible tail; an utterance's CTAs past its own tail exit at once
+  const long long per_utt = ((long long)T * vec + 255) / 256;
+  const dim3 grid((unsigned)(per_utt < 64 ? per_utt : 64), (unsigned)B);
+  zero_tail_kernel<<<grid, 256, 0, stream>>>(static_cast<uint4*>(buf), rows_per_utt, vec, row0, T, lengths);
   AVC_CHECK_CUDA(cudaGetLastError());
   count_launch();
   return 0;

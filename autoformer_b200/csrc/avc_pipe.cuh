@@ -203,6 +203,16 @@ __device__ __forceinline__ void grid_arrive_wait(unsigned int* bar, unsigned int
   } while (seen < target);
 }
 
+// Frame of utterance b whose h goes to h_last: lengths[b] - 1 of a padded batch, else T - 1.  The length is read where it
+// is compared, with a volatile load the compiler can neither hoist into a register held across the frame loop nor
+// speculate (the weight-stationary kernel keeps its register allocation with it, -Xptxas -v).
+__device__ __forceinline__ bool is_last_frame(const int* lengths, int b, int t, int T) {
+  if (!lengths) return t == T - 1;
+  int len;
+  asm volatile("ld.global.nc.s32 %0, [%1];" : "=r"(len) : "l"(lengths + b));
+  return t == len - 1;
+}
+
 __device__ __forceinline__ float sigmoid_fast(float x) { return __fdividef(1.0f, 1.0f + __expf(-x)); }
 // tanh with ~1e-7 absolute error (tanh.approx is only good to 2^-11, too coarse for a 1e-3 end-to-end gate).
 __device__ __forceinline__ float tanh_fast(float x) {

@@ -99,7 +99,12 @@ class AutoVC(layers.PlanOwner, nn.Module):
     ``collect_taps`` (keep fp32 copies of every stage in ``self.taps`` for parity tests),
     ``bn_stats`` ("running" default: every BatchNorm folded with its running statistics, eval semantics | "batch":
     every BatchNorm normalises with the statistics of the call's B x T frames and updates running_mean, running_var
-    and num_batches_tracked on the device, as nn.BatchNorm1d in train mode -- how the reference's notebooks convert)."""
+    and num_batches_tracked on the device, as nn.BatchNorm1d in train mode -- how the reference's notebooks convert).
+
+    ``forward(x, c_org, c_trg, lengths=...)`` converts a padded batch of utterances of different lengths
+    (nn.utils.rnn.pack_padded_sequence semantics): utterance b has ``lengths[b]`` valid frames (a multiple of freq) and
+    gets exactly the mel, mel_postnet and codes of converting ``x[b:b+1, :lengths[b]]`` alone; frames and codes past its
+    end are 0, and what the input holds there is ignored."""
 
     def __init__(self, dim_neck, dim_emb, dim_pre, freq):
         super().__init__()
@@ -130,7 +135,7 @@ class AutoVC(layers.PlanOwner, nn.Module):
 
     @ops.on_device_of_input
     @torch.no_grad()
-    def forward(self, x, c_org, c_trg):
+    def forward(self, x, c_org, c_trg, *, lengths=None):
         if self.training and not self._warned_train and self.bn_stats != "batch":
             warnings.warn("autoformer_b200.AutoVC runs the eval-mode forward (BatchNorm running statistics) "
                           "even in train() mode; it is an inference path (bn_stats='batch' selects train-mode "
@@ -147,6 +152,11 @@ class AutoVC(layers.PlanOwner, nn.Module):
             raise IndexError(f"T={T} is not a multiple of freq={F} (reference indexes i+freq-1, AutoVC.py:60-66)")
         if layers.check_bn_stats(self.bn_stats) == "batch" and B * T == 1:
             raise ValueError(f"Expected more than 1 value per channel when training, got input size {(B, 512, T)}")
+        if lengths is not None:
+            if self.bn_stats == "batch":
+                raise ValueError("lengths with bn_stats='batch': batch statistics over padded frames match no "
+                                 "per-utterance conversion; convert each length separately")
+            lengths = layers.upload_lengths(lengths, B, T, x.device, F)
         plan = self._plan()
         prec = plan.precision
         dev = x.device
@@ -157,13 +167,19 @@ class AutoVC(layers.PlanOwner, nn.Module):
         # ---- encoder: concat speaker code, 3x conv+BN+ReLU, BiLSTM, code down-sampling (AutoVC.py:45-68)
         x = self._encoder_features(x, plan, B, T)
         h = ops.concat_bcast(x, c_org, T, 1, prec)
+        # a padded batch: every buffer a k = 5 convolution reads gets its rows past each utterance's end zeroed (the
+        # zero padding of converting it alone); conv 2's output feeds a 1x1 projection and the length-aware BiLSTM
+        if lengths is not None:
+            ops.zero_tail(h, 0, T, lengths)
         for i, conv in enumerate(plan.enc_convs):
             o = ops.alloc_act(B, T, 512, prec, dev)
             conv(h, B, T, out=o)
             h = o
+            if lengths is not None and i < 2:
+                ops.zero_tail(h, 0, T, lengths)
             if taps is not None:
                 taps[f"enc_conv{i}"] = packing.act_to_float(h, prec)
-        enc_out, codes = plan.enc_lstm(h, B, T, freq=F, want_out=taps is not None)
+        enc_out, codes = plan.enc_lstm(h, B, T, freq=F, want_out=taps is not None, **layers._lengths_kw(lengths))
         if taps is not None:
             taps["enc_lstm"] = enc_out
         flat_codes = codes.reshape(B, -1)                        # cat(codes, dim=-1), AutoVC.py:195,211
@@ -179,10 +195,14 @@ class AutoVC(layers.PlanOwner, nn.Module):
         h = plan.lstm1[0](h, B, T, hseq_f32=f32, persistent=self.persistent_lstm)
         if taps is not None:
             taps["dec_lstm1"] = f32
+        if lengths is not None:
+            ops.zero_tail(h, 0, T, lengths)
         for i, conv in enumerate(plan.dec_convs):
             o = ops.alloc_act(B, T, self.dim_pre, prec, dev)
             conv(h, B, T, out=o)
             h = o
+            if lengths is not None and i < 2:        # conv 2 feeds the causal lstm2
+                ops.zero_tail(h, 0, T, lengths)
             if taps is not None:
                 taps[f"dec_conv{i}"] = packing.act_to_float(h, prec)
         h = plan.lstm2[0](h, B, T, persistent=self.persistent_lstm)
@@ -195,7 +215,13 @@ class AutoVC(layers.PlanOwner, nn.Module):
         plan.linear(h, B, T, out=mel_op, out2=mel.view(B * T, 80))
 
         # ---- postnet + residual (AutoVC.py:173-179, 206-209)
-        post = self._run_postnet(plan, mel_op, mel, B, T, taps)
+        if lengths is None:
+            post = self._run_postnet(plan, mel_op, mel, B, T, taps)
+        else:
+            ops.zero_tail(mel_op, 0, T, lengths)
+            post = plan.postnet(mel_op, mel, B, T, taps, lengths=lengths)
+            ops.zero_tail(mel, 0, T, lengths)
+            ops.zero_tail(post, 0, T, lengths)
         if taps is not None:
             taps["mel"] = mel
             taps["mel_postnet"] = post

@@ -37,17 +37,23 @@ class LstmDV(layers.PlanOwner, nn.Module):
     def _plan(self):
         return self._cache.get(self, (self.precision, self.wavefront), self._build_plan)
 
-    def _last_hidden(self, plan, x):
-        """h_T of the top LSTM layer, fp32 (B, dim_cell)   (LstmDV.py:20-21: ``lstm_out[:, -1, :]``)."""
+    def _last_hidden(self, plan, x, lengths=None):
+        """h_T of the top LSTM layer, fp32 (B, dim_cell)   (LstmDV.py:20-21: ``lstm_out[:, -1, :]``); with lengths, h at
+        frame lengths[b] - 1 of utterance b."""
         ops._require_cuda(x)
         x = x.contiguous().float()
         B, T, _ = x.shape
         h = ops.to_act(x, self.precision)
         h_last = torch.empty(B, self.dim_cell, dtype=torch.float32, device=x.device)
-        return plan["lstm"].last_hidden(h, B, T, h_last, persistent=self.persistent_lstm)
+        if lengths is None:
+            return plan["lstm"].last_hidden(h, B, T, h_last, persistent=self.persistent_lstm)
+        return plan["lstm"].last_hidden(h, B, T, h_last, persistent=self.persistent_lstm,
+                                        lengths=layers.upload_lengths(lengths, B, T, x.device))
 
     @ops.on_device_of_input
     @torch.no_grad()
-    def forward(self, x):
+    def forward(self, x, *, lengths=None):
+        """lengths: optional per-utterance valid frames of a padded batch (list or tensor); the d-vector of utterance b
+        is then that of ``x[b:b+1, :lengths[b]]`` alone."""
         plan = self._plan()
-        return ops.linear_l2norm(self._last_hidden(plan, x), plan["w"], plan["b"])        # LstmDV.py:21-24
+        return ops.linear_l2norm(self._last_hidden(plan, x, lengths), plan["w"], plan["b"])        # LstmDV.py:21-24

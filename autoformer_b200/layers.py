@@ -192,6 +192,31 @@ def conv_bn_layer(sd, prefix, precision, act, bn_owner=None):
     return ops.ConvGemm(*packing.pack_conv(w, b, precision), act=act, tag="conv")
 
 
+def upload_lengths(lengths, B, T, device, multiple=1):
+    """Per-utterance lengths of a padded batch (a list, a CPU tensor or a CUDA tensor, read back once), validated on the
+    host -- B entries, 1 <= lengths[b] <= T, multiples of `multiple` -- and uploaded once as a device int32 [B] tensor.
+    The kernels trust these values, so nothing unchecked reaches them."""
+    if torch.is_tensor(lengths):
+        lengths = lengths.detach().cpu().reshape(-1).tolist()
+    vals = [int(v) for v in lengths]
+    if len(vals) != B:
+        raise ValueError(f"lengths has {len(vals)} entries for a batch of {B} utterances")
+    bad = [v for v in vals if not 1 <= v <= T]
+    if bad:
+        raise ValueError(f"lengths must lie in [1, T={T}]; got {bad[:4]}")
+    bad = [v for v in vals if v % multiple]
+    if bad:
+        raise ValueError(f"lengths must be multiples of freq={multiple} (pad each utterance as pipeline.convert does); "
+                         f"got {bad[:4]}")
+    return torch.tensor(vals, dtype=torch.int32).to(device)
+
+
+def _lengths_kw(lengths):
+    """``lengths=`` for an ops call of a variable-length batch; nothing at all for a fixed-length one, so the ops of a
+    fixed-length forward are called exactly as they were before variable-length batches existed."""
+    return {} if lengths is None else {"lengths": lengths}
+
+
 def lstm_ws_default():
     """AVC_LSTM_WS=0 keeps small batches on the batched recurrence kernel (A/B timing)."""
     return os.environ.get("AVC_LSTM_WS", "1") != "0"
@@ -255,7 +280,9 @@ class LstmLayer:
         kx = (self.C_in + packing.KC[self.precision] - 1) // packing.KC[self.precision]
         return self.fused and (kx <= 6 or B >= 192)
 
-    def __call__(self, x, B, T, hseq_f32=None, h_last=None, persistent=False, hseq=None):
+    def __call__(self, x, B, T, hseq_f32=None, h_last=None, persistent=False, hseq=None, lengths=None):
+        """lengths: optional device int32 [B] of a padded batch; h_last[b] is then h at frame lengths[b] - 1 (hseq
+        keeps all T frames: the recurrence is causal, so the frames past a length never reach a valid one)."""
         cap = ops.persistent_batch_cap(self.H) if persistent else 0
         if persistent and B > cap > 0:
             # utterances are independent: a batch too large for one wave of the persistent grid runs as sub-batches
@@ -264,7 +291,8 @@ class LstmLayer:
             for b0 in range(0, B, cap):
                 b1 = min(B, b0 + cap)
                 self(x[b0:b1], b1 - b0, T, hseq_f32=hseq_f32[b0:b1] if hseq_f32 is not None else None,
-                     h_last=h_last[b0:b1] if h_last is not None else None, persistent=True, hseq=out[b0:b1])
+                     h_last=h_last[b0:b1] if h_last is not None else None, persistent=True, hseq=out[b0:b1],
+                     **_lengths_kw(lengths[b0:b1] if lengths is not None else None))
             return out
         if persistent and self.ws and ops.ws_supported(B, self.H, self.precision):
             # small batch: dense input projection, then the recurrence with W_hh resident in shared memory
@@ -272,7 +300,7 @@ class LstmLayer:
             xp = torch.empty(B * T, 4 * self.H, dtype=torch.float32, device=x.device)
             ih(x, B, T, out2=xp)
             out = ops.lstm_seq_ws(xp, hh, B, T, self.H, hseq=hseq, hseq_f32=hseq_f32, h_last=h_last,
-                                  precision=self.precision)
+                                  precision=self.precision, **_lengths_kw(lengths))
             if out is not None:
                 return out
             self.ws = False             # the device cannot hold the grid: batched kernel from now on
@@ -281,12 +309,13 @@ class LstmLayer:
         if fused:
             wih, bias, hh = self.fused_packs(group)
             return ops.lstm_seq(None, hh, B, T, self.H, self.precision, group, hseq=hseq, hseq_f32=hseq_f32,
-                                h_last=h_last, persistent=persistent, xin=x, w_ih=wih, bias=bias, c_in=self.C_in)
+                                h_last=h_last, persistent=persistent, xin=x, w_ih=wih, bias=bias, c_in=self.C_in,
+                                **_lengths_kw(lengths))
         ih, hh = self.packs(group)
         xp = torch.empty(B * T, 4 * self.H, dtype=torch.float32, device=x.device)
         ih(x, B, T, out2=xp)
         return ops.lstm_seq(xp, hh, B, T, self.H, self.precision, group, hseq=hseq, hseq_f32=hseq_f32, h_last=h_last,
-                            persistent=persistent)
+                            persistent=persistent, **_lengths_kw(lengths))
 
 
 def lstm_layers(sd, prefix, num_layers, precision):
@@ -330,19 +359,22 @@ class LstmStack:
                 all(l.H == self.H and l.C_in == self.H for l in self.layers[1:]) and
                 ops.stack_supported(B, self.H, len(self.layers), self.precision))
 
-    def last_hidden(self, x, B, T, h_last, persistent=False):
-        """x: the first layer's input in the operand format; fills h_last [B][H] fp32 with h_{T-1} of the top layer."""
+    def last_hidden(self, x, B, T, h_last, persistent=False, lengths=None):
+        """x: the first layer's input in the operand format; fills h_last [B][H] fp32 with h_{T-1} of the top layer
+        (with lengths, a device int32 [B]: h at frame lengths[b] - 1 of utterance b)."""
         if self.eligible(B, persistent):
             first = self.layers[0]
             ih, _ = first.packs(packing.WS_GROUP)
             xp = torch.empty(B * T, 4 * self.H, dtype=torch.float32, device=x.device)
             ih(x, B, T, out2=xp)
-            if ops.lstm_stack_ws(xp, self.packs(), B, T, self.H, h_last=h_last) is not None:
+            if ops.lstm_stack_ws(xp, self.packs(), B, T, self.H, h_last=h_last, **_lengths_kw(lengths)) is not None:
                 return h_last
             self.wavefront = False      # the device cannot hold the grid: layer by layer from now on
         h = x
         for i, layer in enumerate(self.layers):
-            h = layer(h, B, T, h_last=h_last if i == len(self.layers) - 1 else None, persistent=persistent)
+            top = i == len(self.layers) - 1
+            h = layer(h, B, T, h_last=h_last if top else None, persistent=persistent,
+                      **_lengths_kw(lengths if top else None))
         return h_last
 
 
@@ -361,8 +393,9 @@ class BiLstmSmall:
             self.layers.append((ih, hh))
         self.H = self.layers[0][1].shape[2]
 
-    def __call__(self, x, B, T, freq=None, want_out=False):
-        """Returns (out [B][T][2H] of the last layer or None, codes [B][T/freq][2H] fp32 or None)."""
+    def __call__(self, x, B, T, freq=None, want_out=False, lengths=None):
+        """Returns (out [B][T][2H] of the last layer or None, codes [B][T/freq][2H] fp32 or None).  lengths: optional
+        device int32 [B] of a padded batch (multiples of freq): out rows / codes past an utterance's end are 0."""
         H = self.H
         out = None
         codes = None
@@ -372,13 +405,14 @@ class BiLstmSmall:
             ih(x, B, T, out2=xp)
             if not last:
                 out = ops.alloc_act(B, T, 2 * H, self.precision, x.device)
-                ops.bilstm_small(xp, hh, B, T, H, out=out, split=self.precision == "fp32")
+                ops.bilstm_small(xp, hh, B, T, H, out=out, split=self.precision == "fp32", **_lengths_kw(lengths))
                 x = out
             else:
                 out = torch.empty(B, T, 2 * H, dtype=torch.float32, device=x.device) if (want_out or freq is None) else None
                 if freq is not None:
                     codes = torch.empty(B, T // freq, 2 * H, dtype=torch.float32, device=x.device)
-                ops.bilstm_small(xp, hh, B, T, H, out=out, codes=codes, freq=freq or 1, round_tf32=False)
+                ops.bilstm_small(xp, hh, B, T, H, out=out, codes=codes, freq=freq or 1, round_tf32=False,
+                                 **_lengths_kw(lengths))
         return out, codes
 
 
@@ -390,20 +424,23 @@ class Postnet:
         self.convs = [conv_bn_layer(sd, f"{prefix}.convolutions.{i}", precision, "tanh" if i < 4 else "none", bn_owner)
                       for i in range(5)]
 
-    def hidden(self, mel_op, B, T, taps=None):
-        """The four conv+BN+tanh layers: [B][T][80] -> [B][T][512], operand format."""
+    def hidden(self, mel_op, B, T, taps=None, lengths=None):
+        """The four conv+BN+tanh layers: [B][T][80] -> [B][T][512], operand format.  lengths (device int32 [B]): the
+        rows past each utterance's end are zeroed after every layer, as the next k = 5 convolution's zero padding."""
         h = mel_op
         for i in range(4):
             o = ops.alloc_act(B, T, 512, self.precision, h.device)
             self.convs[i](h, B, T, out=o)
+            if lengths is not None:
+                ops.zero_tail(o, 0, T, lengths)
             h = o
             if taps is not None:
                 taps[f"post_conv{i}"] = packing.act_to_float(h, self.precision)
         return h
 
-    def __call__(self, mel_op, mel_f32, B, T, taps=None):
+    def __call__(self, mel_op, mel_f32, B, T, taps=None, lengths=None):
         """mel_op: [B][T][80] operand dtype; mel_f32: exact fp32 [B][T][80].  Returns mel + postnet(mel), fp32."""
-        h = self.hidden(mel_op, B, T, taps)
+        h = self.hidden(mel_op, B, T, taps) if lengths is None else self.hidden(mel_op, B, T, taps, lengths=lengths)
         out = torch.empty(B, T, 80, dtype=torch.float32, device=h.device)
         self.convs[4](h, B, T, out2=out.view(B * T, 80), residual=mel_f32.view(B * T, 80))
         return out

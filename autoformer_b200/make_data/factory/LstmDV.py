@@ -33,9 +33,10 @@ class LstmDV(_Embedder):
 
     @ops.on_device_of_input
     @torch.no_grad()
-    def forward(self, x):
+    def forward(self, x, *, lengths=None):
+        """lengths: as the embedder's (factory/LstmDV.py): per-utterance valid frames of a padded batch."""
         plan = self._plan()
-        h_last = self._last_hidden(plan, x)
+        h_last = self._last_hidden(plan, x, lengths)
         embeds, d_vec = ops.linear_rows(h_last, plan["w"], plan["b"], want_raw=True, want_normed=True)   # :21-23
         predictions, _ = ops.linear_rows(embeds, plan["w_out"], plan["b_out"], want_raw=True)            # :24
         return predictions, d_vec                                                                         # :25

@@ -256,6 +256,28 @@ def reflect_halo(buf, row0, L, reflect):
     return buf
 
 
+def _check_lengths(lengths, B):
+    """Per-utterance lengths of a padded batch: a device int32 [B] tensor (values are validated by the caller, on the
+    host, before the upload -- the kernels trust them)."""
+    assert lengths.dtype == torch.int32 and lengths.is_contiguous() and lengths.shape == (B,), (lengths.shape, B)
+    _require_cuda(lengths)
+    return lengths.data_ptr()
+
+
+def zero_tail(buf, row0, T, lengths):
+    """Zero rows row0 + lengths[b] .. row0 + T - 1 of utterance b of a channels-last buffer [B][rows][C'] (any operand
+    format): the padded frames of a variable-length batch then read as the zero padding of the next convolution."""
+    lib = _lib.load()
+    _require_cuda(buf)
+    assert buf.dim() == 3 and buf.is_contiguous()
+    B, rows, _ = buf.shape
+    row_bytes = buf.shape[2] * buf.element_size()
+    with PROFILER.span("zero_tail", bytes=float(B * T * row_bytes)):
+        _lib.check(lib.avc_zero_tail(buf.data_ptr(), B, rows, row_bytes, row0, T, _check_lengths(lengths, B), _stream()),
+                   "avc_zero_tail")
+    return buf
+
+
 # Cap on the CTAs one persistent LSTM launch may take (None: the whole device).  pipeline.convert_pairs sets it to half
 # the SMs while it runs two under-filled batches on two streams, so that both cooperative grids are resident together.
 LSTM_CTA_BUDGET = None
@@ -307,10 +329,12 @@ def choose_gate_group(B, H, persistent=False, n_sm=148, fused=False, precision=N
 
 
 def lstm_seq(xproj, w_hh, B, T, H, precision, group, hseq=None, hseq_f32=None, h_last=None, persistent=False,
-             debug_clk=None, xin=None, w_ih=None, bias=None, c_in=None):
+             debug_clk=None, xin=None, w_ih=None, bias=None, c_in=None, lengths=None):
     """Run the recurrence of one uni-directional layer.  Either xproj [B*T][4H] fp32 (packed gate order, bias
     included), or -- fused input projection -- the layer input xin [B][T][C'] in the operand format of `precision`
-    with w_ih / bias from packing.pack_lstm_ih_fused and c_in logical input channels."""
+    with w_ih / bias from packing.pack_lstm_ih_fused and c_in logical input channels.
+    lengths: optional device int32 [B] of a padded batch -- h_last[b] is then h at frame lengths[b] - 1 (taken from the
+    exact fp32 sequence, allocated here when hseq_f32 is not given)."""
     lib = _lib.load()
     fused = xin is not None
     _require_cuda(xin if fused else xproj, w_hh)
@@ -344,6 +368,10 @@ def lstm_seq(xproj, w_hh, B, T, H, precision, group, hseq=None, hseq_f32=None, h
         d.xproj = xproj.data_ptr()
     d.w_hh = w_hh.data_ptr()
     d.hseq = hseq.data_ptr()
+    if lengths is not None:
+        d.lengths = _check_lengths(lengths, B)
+        if h_last is not None and hseq_f32 is None:
+            hseq_f32 = torch.empty(B, T, H, dtype=torch.float32, device=dev)
     if hseq_f32 is not None:
         assert hseq_f32.is_contiguous() and hseq_f32.shape == (B, T, H) and hseq_f32.dtype == torch.float32
         d.hseq_f32 = hseq_f32.data_ptr()
@@ -395,10 +423,12 @@ def ws_supported(B, H, precision, n_sm=148):
     return chunks * 2 * ar * 128 + red + stage + 1152 <= 227 * 1024 and 2 * ar + 64 * chunks <= 512
 
 
-def lstm_seq_ws(xproj, w_hh, B, T, H, hseq=None, hseq_f32=None, h_last=None, debug_clk=None, precision="fp32"):
+def lstm_seq_ws(xproj, w_hh, B, T, H, hseq=None, hseq_f32=None, h_last=None, debug_clk=None, precision="fp32",
+                lengths=None):
     """Small-batch recurrence with W_hh resident in shared memory (split precision).  xproj [B*T][4H] fp32 and w_hh
     [4H][2H] bf16 in the packing.WS_GROUP gate order.  Returns hseq, or None when the device cannot hold the grid
-    (nothing was launched; the caller uses lstm_seq)."""
+    (nothing was launched; the caller uses lstm_seq).  lengths: optional device int32 [B], h_last[b] = h at frame
+    lengths[b] - 1."""
     lib = _lib.load()
     _require_cuda(xproj, w_hh)
     dev = w_hh.device
@@ -418,6 +448,8 @@ def lstm_seq_ws(xproj, w_hh, B, T, H, hseq=None, hseq_f32=None, h_last=None, deb
     if h_last is not None:
         assert h_last.is_contiguous() and h_last.shape == (B, H) and h_last.dtype == torch.float32
         d.h_last = h_last.data_ptr()
+    if lengths is not None:
+        d.lengths = _check_lengths(lengths, B)
     bar = torch.empty(256, dtype=torch.int32, device=dev)             # zeroed by the library
     d.grid_barrier = bar.data_ptr()
     d.B, d.T, d.H = B, T, H
@@ -445,11 +477,12 @@ def stack_supported(B, H, L, precision, n_sm=148):
     return tiles * ar * 128 + 2 * ar * 64 * 4 + 4096 + 1152 <= 227 * 1024
 
 
-def lstm_stack_ws(xproj0, packs, B, T, H, h_last=None, hs=None, debug_clk=None):
+def lstm_stack_ws(xproj0, packs, B, T, H, h_last=None, hs=None, debug_clk=None, lengths=None):
     """All layers of a small-batch LSTM stack as one wavefront launch.  xproj0 [B*T][4H] fp32 (layer 0's dense input
     projection, biases included), `packs` = [(w_ih, w_hh, bias)] per layer (packing.pack_lstm_stack; w_ih and bias are
     None for layer 0); all in the packing.WS_GROUP gate order.  Returns the scratch sequences hs [L][T+1][B][H] fp16
-    (frame t+1 of layer l = h^l_t), or None when the device cannot hold the grid (nothing was launched)."""
+    (frame t+1 of layer l = h^l_t), or None when the device cannot hold the grid (nothing was launched).
+    lengths: optional device int32 [B], h_last[b] = the top layer's h at frame lengths[b] - 1."""
     lib = _lib.load()
     _require_cuda(xproj0, packs[0][1])
     dev = packs[0][1].device
@@ -470,6 +503,8 @@ def lstm_stack_ws(xproj0, packs, B, T, H, h_last=None, hs=None, debug_clk=None):
     if h_last is not None:
         assert h_last.is_contiguous() and h_last.shape == (B, H) and h_last.dtype == torch.float32
         d.h_last = h_last.data_ptr()
+    if lengths is not None:
+        d.lengths = _check_lengths(lengths, B)
     bar = torch.empty(256, dtype=torch.int32, device=dev)             # zeroed by the library
     d.grid_barrier = bar.data_ptr()
     d.B, d.T, d.H, d.L = B, T, H, L
@@ -484,9 +519,10 @@ def lstm_stack_ws(xproj0, packs, B, T, H, h_last=None, hs=None, debug_clk=None):
     return hs
 
 
-def bilstm_small(xproj, w_hh, B, T, H, out=None, codes=None, freq=1, round_tf32=True, split=False):
+def bilstm_small(xproj, w_hh, B, T, H, out=None, codes=None, freq=1, round_tf32=True, split=False, lengths=None):
     """xproj [B*T][8H] fp32; w_hh [2][4H][H] fp32; out [B][T][2H] (fp32/bf16; split: [B][T][4H] bf16) and/or
-    codes [B][T/freq][2H] fp32."""
+    codes [B][T/freq][2H] fp32.  lengths: optional device int32 [B] of a padded batch (each a multiple of freq, checked
+    by the caller): utterance b runs over its first lengths[b] frames only, later out rows and codes are 0."""
     lib = _lib.load()
     _require_cuda(xproj, w_hh)
     assert xproj.dtype == torch.float32 and xproj.is_contiguous() and xproj.numel() == B * T * 8 * H
@@ -499,9 +535,10 @@ def bilstm_small(xproj, w_hh, B, T, H, out=None, codes=None, freq=1, round_tf32=
     if codes is not None:
         assert codes.is_contiguous() and codes.dtype == torch.float32 and codes.shape == (B, T // freq, 2 * H)
         codes_ptr = codes.data_ptr()
+    len_ptr = _check_lengths(lengths, B) if lengths is not None else None
     with PROFILER.span("bilstm_small", flops=2.0 * 2 * 4 * H * H * B * T, bytes=4.0 * B * T * 8 * H):
         _lib.check(lib.avc_bilstm_small(xproj.data_ptr(), w_hh.data_ptr(), out_ptr, out_dtype, 1 if round_tf32 else 0,
-                                        codes_ptr, B, T, H, freq, _stream()), "avc_bilstm_small")
+                                        codes_ptr, B, T, H, freq, _stream(), len_ptr), "avc_bilstm_small")
     return out, codes
 
 

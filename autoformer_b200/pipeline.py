@@ -3,8 +3,9 @@
 Follows the reference's own recipe for utterances whose length is not a multiple of ``freq``: zero-pad the mel at
 the end, convert, trim the padding off again (util/evaluate.py:36-43 ``crop_mel`` pads with constant 0;
 :85-92 trims ``mel_trans`` back), then vocode ``mel_trans.transpose(2, 1)`` (conversion.ipynb cell 14,
-util/evaluate.py:96-98).  Utterances of one call share the same T (callers bucket by exact length: zero padding
-changes the result, SURVEY.md 5)."""
+util/evaluate.py:96-98).  ``convert`` and ``convert_batches`` take batches whose utterances share one T (plain zero
+padding changes the result, SURVEY.md 5); ``convert_utterances`` and ``embed_utterances`` take utterances of any length
+and batch them with per-utterance lengths, which gives each one exactly its result converted alone."""
 import os
 
 import numpy as np
@@ -153,6 +154,48 @@ class StreamingConverter:
         self.pending = None
         ev.synchronize()
         return tuple(self.host_out[s])
+
+
+def _ragged_batches(mels, max_batch, multiple):
+    """(T_batch, ids, padded input [n][T_batch][80], lengths) per variable-length batch (sharding.make_ragged_batches);
+    utterance i padded with zeros to a multiple of `multiple` frames (util/evaluate.py:36-43), then to T_batch."""
+    from . import sharding
+    for T_batch, ids in sharding.make_ragged_batches([m.shape[0] for m in mels], max_batch, multiple):
+        lens = [(mels[i].shape[0] + multiple - 1) // multiple * multiple for i in ids]
+        x = mels[ids[0]].new_zeros(len(ids), T_batch, mels[ids[0]].shape[1])
+        for k, i in enumerate(ids):
+            x[k, :mels[i].shape[0]] = mels[i]
+        yield T_batch, ids, x, lens
+
+
+@torch.no_grad()
+def convert_utterances(model, mels, c_org, c_trg, max_batch=512):
+    """Convert utterances of any lengths: mels is a list of (T_i, 80) device tensors, c_org / c_trg (N, dim_emb).
+    Each is zero-padded to a multiple of ``model.freq`` (the reference's recipe, as ``convert``), the utterances are
+    batched by ``sharding.make_ragged_batches`` and every batch runs once with per-utterance lengths.  Returns the
+    list of converted mels (mel_postnet, (T_i, 80)) in input order, each trimmed to T_i."""
+    out = [None] * len(mels)
+    for _, ids, x, lens in _ragged_batches(mels, max_batch, model.freq):
+        idx = torch.as_tensor(ids, device=c_org.device)
+        _, post, _ = model(x, c_org[idx], c_trg[idx], lengths=lens)
+        post = post.squeeze(1)
+        for k, i in enumerate(ids):
+            out[i] = post[k, :mels[i].shape[0]]
+    return out
+
+
+@torch.no_grad()
+def embed_utterances(embedder, mels, max_batch=64):
+    """LstmDV d-vectors of utterances of any lengths (list of (T_i, 80) device tensors) with variable-length batches:
+    row i of the (N, dim_emb) result is the embedder's output for mels[i] alone.  The default batch of 64 keeps the
+    small-batch recurrence kernels (their cost per frame does not grow up to 64 utterances)."""
+    out = [None] * len(mels)
+    for _, ids, x, lens in _ragged_batches(mels, max_batch, 1):
+        e = embedder(x, lengths=lens)
+        e = e[1] if isinstance(e, tuple) else e                  # the classifier twin returns (predictions, d_vec)
+        for k, i in enumerate(ids):
+            out[i] = e[k]
+    return torch.stack(out)
 
 
 # ------------------------------------------------------------------------------------------------ side-by-side batches

@@ -3,8 +3,14 @@
 In eval mode every utterance is independent, so the path shards by utterance with NO data-path collective:
 weights are replicated, each rank converts its own batches, and ``torch.distributed`` (NCCL over NVLink on the GPU
 box, gloo in the CPU tests) is used only to gather fixed-size per-rank records (frames, time, checksum) and, on
-request, the outputs.  Utterances are bucketed by EXACT length: zero padding changes the result because the
-backward LSTM and LstmDV's last step see the padding (SURVEY.md 5), so batches never mix lengths.
+request, the outputs.  Two ways to batch utterances of different lengths:
+
+- ``plan``: bucketed by EXACT length, one launch sequence per distinct length (plain zero padding would change the
+  result: the backward LSTM and LstmDV's last step would see the padding, SURVEY.md 5);
+- ``plan_ragged``: sorted by length and cut into full batches, each padded to its longest utterance and run with
+  per-utterance ``lengths`` (AutoVC / LstmDV ``forward(..., lengths=...)``), which gives every utterance exactly the
+  result of converting it alone.  The recurrences cost per frame whatever the batch size, so a few full batches are
+  cheaper than one under-filled batch per length.
 """
 from collections import defaultdict
 
@@ -77,6 +83,19 @@ def assign_batches(batches, world_size, cost=frames_cost):
 
 def plan(lengths, world_size, max_batch=512, cost=frames_cost):
     return assign_batches(make_batches(bucket_by_length(lengths), max_batch), world_size, cost)
+
+
+def make_ragged_batches(lengths, max_batch=512, multiple=1):
+    """Variable-length batches: each length is padded up to `multiple` (AutoVC's freq), utterances are sorted by padded
+    length (descending, ties by id) and consecutive runs of ``max_batch`` form the batches.  Returns [(T_batch, ids)]
+    with T_batch the longest padded length of the run."""
+    padded = [(int(t) + multiple - 1) // multiple * multiple for t in lengths]
+    order = sorted(range(len(padded)), key=lambda i: (-padded[i], i))
+    return [(padded[order[s]], order[s:s + max_batch]) for s in range(0, len(order), max_batch)]
+
+
+def plan_ragged(lengths, world_size, max_batch=512, multiple=1, cost=frames_cost):
+    return assign_batches(make_ragged_batches(lengths, max_batch, multiple), world_size, cost)
 
 
 def gather_records(record, device=None):

@@ -240,6 +240,10 @@ typedef struct avc_lstm_desc {
   long long xin_ld;          /* elements per input row */
   const void* w_ih;          /* [4H][Kp] packed row order, Kp = C_in rounded up to the k-block; dtype 2: [4H][2Kp] */
   const float* bias;         /* [4H] fp32 b_ih + b_hh, packed order */
+  const int* lengths;        /* optional [B] int32, 1 <= lengths[b] <= T (may be NULL = all T): h_last[b] is h at frame
+                                lengths[b] - 1 (a padded batch, pack_padded_sequence semantics), read from hseq_f32, which
+                                is then required.  hseq is still written for all T frames; the recurrence is causal, so
+                                frames past a length never reach a valid one */
 } avc_lstm_desc;
 
 /* Returned by avc_lstm_seq in persistent mode when the grid cannot be co-resident (one wave); nothing was launched. */
@@ -266,6 +270,7 @@ typedef struct avc_lstm_ws_desc {
   long long* debug_clk;       /* optional device buffer, 8 x int64 per (frame, CTA): clock64 stamps (profiling aid) */
   int dtype;                  /* 0 or AVC_DTYPE_BF16X3: as above; AVC_DTYPE_F16 ("fp16x2"): w_hh = [w_hi | w_lo] fp16,
                                  hseq [B][T][H] fp16 */
+  const int* lengths;         /* optional [B] int32 (may be NULL): h_last[b] = h at frame lengths[b] - 1, as avc_lstm_desc */
 } avc_lstm_ws_desc;
 
 int avc_lstm_seq_ws(const avc_lstm_ws_desc* d, void* stream);
@@ -296,6 +301,8 @@ typedef struct avc_lstm_stack_desc {
   unsigned int* grid_barrier;                 /* one counter; zeroed by the library */
   int B, T, H, L;
   long long* debug_clk;                       /* optional device buffer, 16 x int64 per (tick, CTA), T + 2 (L - 1) ticks */
+  const int* lengths;                         /* optional [B] int32 (may be NULL): h_last[b] = top-layer h at frame
+                                                 lengths[b] - 1, as avc_lstm_desc; hs is still written for all T frames */
 } avc_lstm_stack_desc;
 
 int avc_lstm_stack_ws(const avc_lstm_stack_desc* d, void* stream);
@@ -308,9 +315,14 @@ int avc_lstm_stack_ws(const avc_lstm_stack_desc* d, void* stream);
  *   w_hh   [2][4H][H] fp32 (PyTorch row order i,f,g,o)
  *   out    [B][T][2H] (fwd | bwd) in out_dtype (2: [B][T][4H] split bf16), or NULL
  *   codes  [B][T/freq][2H] fp32, or NULL
+ *   lengths optional [B] int32 (NULL = every utterance has T frames): utterance b of a padded batch has lengths[b]
+ *          valid frames, 1 <= lengths[b] <= T, a multiple of freq when codes are written (the caller checks).  Its
+ *          forward direction stops at frame lengths[b] - 1 and its backward direction starts there from the zero state
+ *          (nn.utils.rnn.pack_padded_sequence semantics); out rows t >= lengths[b] and codes j >= lengths[b] / freq are
+ *          written as 0.  xproj rows past a length are never read.
  */
 int avc_bilstm_small(const float* xproj, const float* w_hh, void* out, int out_dtype, int out_round_tf32,
-                     float* codes, int B, int T, int H, int freq, void* stream);
+                     float* codes, int B, int T, int H, int freq, void* stream, const int* lengths);
 
 /*
  * out[b,t,:] = [ seq[b, t / div, 0:C1] || vec[b, 0:C2] ]   (channels-last concat with broadcast)
@@ -346,6 +358,17 @@ int avc_linear_rows(const float* h, const float* w, const float* bias, float* ou
  * utterance with this launch (a few KB).  row_bytes multiple of 16.
  */
 int avc_reflect_halo(void* buf, int B, int rows_per_utt, long long row_bytes, int row0, int L, int reflect, void* stream);
+
+/*
+ * Zero the padded tail of every utterance of a channels-last buffer [B][rows_per_utt][row_bytes]: rows
+ * row0 + lengths[b] .. row0 + T - 1 of utterance b (lengths: device int32 [B], 1 <= lengths[b] <= T).  A zero is
+ * all-zero bits in every operand format (fp32, bf16, fp16, split hi | lo), so after this launch the rows past an
+ * utterance's end read as the zero padding the next convolution expects (avc_conv_gemm reads rows outside the buffer
+ * as zero, and a padded batch must give each utterance the result of converting it alone).  16-byte stores, nothing
+ * else is touched; row_bytes multiple of 16.
+ */
+int avc_zero_tail(void* buf, int B, int rows_per_utt, long long row_bytes, int row0, int T, const int* lengths,
+                  void* stream);
 
 /*
  * in [B][C][L] fp32 (channels-first, the reference's (B, 80, T) mel layout) -> out [B][L + 2*pad][C'] channels-last in
