@@ -184,6 +184,9 @@ class Resblock2Desc(ctypes.Structure):
         ("mono_w", ctypes.c_void_p),
         ("mono_bias", ctypes.c_float),
         ("mono_taps", ctypes.c_int),
+        ("lengths", ctypes.c_void_p),
+        ("tile_start", ctypes.c_void_p),
+        ("n_tiles", ctypes.c_int),
     ]
 
 
@@ -241,7 +244,7 @@ def load():
     lib.avc_resblock.argtypes = [ctypes.POINTER(ResblockDesc), ctypes.c_void_p]
     lib.avc_resblock.restype = ctypes.c_int
     lib.avc_reflect_halo.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_longlong, ctypes.c_int,
-                                     ctypes.c_int, ctypes.c_int, ctypes.c_void_p]
+                                     ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]
     lib.avc_reflect_halo.restype = ctypes.c_int
     lib.avc_zero_tail.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_longlong, ctypes.c_int,
                                   ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p]
@@ -266,7 +269,8 @@ def load():
                                       ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]
     lib.avc_transpose_pad.restype = ctypes.c_int
     lib.avc_conv_to_mono_tanh.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_float, ctypes.c_void_p,
-                                          ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]
+                                          ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_void_p,
+                                          ctypes.c_void_p]
     lib.avc_conv_to_mono_tanh.restype = ctypes.c_int
     vp, ci = ctypes.c_void_p, ctypes.c_int
     lib.avc_gn_stats.argtypes = [vp, vp, ci, ctypes.c_longlong, ctypes.c_float, vp]

@@ -402,32 +402,42 @@ __global__ void __launch_bounds__(256) transpose_pad_kernel(const float* __restr
 constexpr int kMonoTile = 256;
 __global__ void __launch_bounds__(kMonoTile) conv_to_mono_tanh_kernel(const float* __restrict__ x,
                                                                       const float* __restrict__ w, float bias,
-                                                                      float* __restrict__ out, int L, int C, int K) {
+                                                                      float* __restrict__ out, int L, int C, int K,
+                                                                      const int* __restrict__ lengths) {
   extern __shared__ float sm[];
   const int half = K / 2;
   const int rows = kMonoTile + K - 1;
+  const int b = blockIdx.y;
+  const int t0 = blockIdx.x * kMonoTile;
+  const int len = lengths ? __ldg(lengths + b) : L;     // a padded batch: reflect at the utterance's end, 0 past it
+  if (t0 >= len) {
+    if (t0 + (int)threadIdx.x < L) out[(long long)b * L + t0 + threadIdx.x] = 0.f;
+    return;
+  }
   // rows of C + 4 floats: 16-byte aligned, and consecutive rows start 4 banks apart, so the float4 reads of a quarter
   // warp (8 threads, one row each, same column) cover all 32 banks once -- the kernel is HBM-bound only when it issues
   // 16-byte shared-memory loads (scalar loads made it LDS-bound at 29 % of the HBM peak, ncu r02)
   const int ldx = C + 4;
   float* xs = sm;                       // [rows][C + 4]
   float* ws = sm + rows * ldx;          // [K][C]
-  const int b = blockIdx.y;
-  const int t0 = blockIdx.x * kMonoTile;
   for (int i = threadIdx.x; i < K * C; i += blockDim.x) ws[i] = w[i];
   const int c4 = C / 4;
   for (int i = threadIdx.x; i < rows * c4; i += blockDim.x) {
     const int r = i / c4, c = (i - r * c4) * 4;
     int src = t0 + r - half;
     if (src < 0) src = -src;                         // ReflectionPad1d: edge sample not repeated
-    if (src >= L) src = 2 * (L - 1) - src;
+    if (src >= len) src = 2 * (len - 1) - src;
     float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (src >= 0 && src < L) v = __ldg(reinterpret_cast<const float4*>(x + ((long long)b * L + src) * C + c));
+    if (src >= 0 && src < len) v = __ldg(reinterpret_cast<const float4*>(x + ((long long)b * L + src) * C + c));
     *reinterpret_cast<float4*>(xs + r * ldx + c) = v;
   }
   __syncthreads();
   const int t = t0 + threadIdx.x;
   if (t >= L) return;
+  if (t >= len) {
+    out[(long long)b * L + t] = 0.f;
+    return;
+  }
   float acc0 = bias, acc1 = 0.f, acc2 = 0.f, acc3 = 0.f;
   for (int k = 0; k < K; ++k) {
     const float4* xr = reinterpret_cast<const float4*>(xs + (threadIdx.x + k) * ldx);
@@ -552,7 +562,8 @@ extern "C" int avc_transpose_pad(const float* in, void* out, int B, int C, int L
 // ---------------------------------------------------------------------------------------------
 namespace avc {
 __global__ void __launch_bounds__(256) reflect_halo_kernel(uint4* __restrict__ buf, long long rows_per_utt, int vec_per_row,
-                                                           long long row0, long long L, int reflect, long long total) {
+                                                           long long row0, long long L, int reflect, long long total,
+                                                           const int* __restrict__ lengths) {
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const int v = static_cast<int>(i % vec_per_row);
     long long r = i / vec_per_row;
@@ -564,8 +575,9 @@ __global__ void __launch_bounds__(256) reflect_halo_kernel(uint4* __restrict__ b
       src = row0 + (k + 1);
     } else {
       const int j = k - reflect + 1;
-      dst = row0 + L - 1 + j;
-      src = row0 + L - 1 - j;
+      const long long end = lengths ? (long long)__ldg(lengths + b) : L;    // the utterance's own last row
+      dst = row0 + end - 1 + j;
+      src = row0 + end - 1 - j;
     }
     uint4* base = buf + b * rows_per_utt * vec_per_row;
     base[dst * vec_per_row + v] = base[src * vec_per_row + v];
@@ -574,7 +586,7 @@ __global__ void __launch_bounds__(256) reflect_halo_kernel(uint4* __restrict__ b
 }  // namespace avc
 
 extern "C" int avc_reflect_halo(void* buf, int B, int rows_per_utt, long long row_bytes, int row0, int L, int reflect,
-                                void* stream_v) {
+                                void* stream_v, const int* lengths) {
   using namespace avc;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
   AVC_REQUIRE(buf != nullptr, "avc_reflect_halo: null buffer");
@@ -586,7 +598,7 @@ extern "C" int avc_reflect_halo(void* buf, int B, int rows_per_utt, long long ro
   const long long total = (long long)B * 2 * reflect * vec;
   const long long blocks = (total + 255) / 256;
   reflect_halo_kernel<<<(unsigned)(blocks < 4096 ? blocks : 4096), 256, 0, stream>>>(
-      static_cast<uint4*>(buf), rows_per_utt, vec, row0, L, reflect, total);
+      static_cast<uint4*>(buf), rows_per_utt, vec, row0, L, reflect, total, lengths);
   AVC_CHECK_CUDA(cudaGetLastError());
   count_launch();
   return 0;
@@ -712,7 +724,7 @@ extern "C" int avc_complex_mag(const float* spec, void* mag, long long rows, int
 }
 
 extern "C" int avc_conv_to_mono_tanh(const float* x, const float* w, float bias, float* out, int B, int L, int C, int K,
-                                     void* stream_v) {
+                                     void* stream_v, const int* lengths) {
   using namespace avc;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
   AVC_REQUIRE(x && w && out, "avc_conv_to_mono_tanh: null buffer");
@@ -721,7 +733,7 @@ extern "C" int avc_conv_to_mono_tanh(const float* x, const float* w, float bias,
   const size_t smem = ((size_t)(kMonoTile + K - 1) * (C + 4) + (size_t)K * C) * sizeof(float);
   AVC_CHECK_CUDA(cudaFuncSetAttribute(conv_to_mono_tanh_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   dim3 grid((L + kMonoTile - 1) / kMonoTile, B);
-  conv_to_mono_tanh_kernel<<<grid, kMonoTile, smem, stream>>>(x, w, bias, out, L, C, K);
+  conv_to_mono_tanh_kernel<<<grid, kMonoTile, smem, stream>>>(x, w, bias, out, L, C, K, lengths);
   AVC_CHECK_CUDA(cudaGetLastError());
   count_launch();
   return 0;

@@ -213,6 +213,18 @@ __device__ __forceinline__ bool is_last_frame(const int* lengths, int b, int t, 
   return t == len - 1;
 }
 
+// Utterance of `tile` in the compacted tile space of a padded batch: the b with tile_start[b] <= tile < tile_start[b + 1]
+// (tile_start [B + 1] is a strictly increasing prefix table, every utterance has at least one tile).
+__device__ __forceinline__ int ragged_tile_utt(const int* __restrict__ tile_start, int B, int tile) {
+  int lo = 0, hi = B;
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (__ldg(tile_start + mid) <= tile) lo = mid;
+    else hi = mid;
+  }
+  return lo;
+}
+
 __device__ __forceinline__ float sigmoid_fast(float x) { return __fdividef(1.0f, 1.0f + __expf(-x)); }
 // tanh with ~1e-7 absolute error (tanh.approx is only good to 2^-11, too coarse for a 1e-3 end-to-end gate).
 __device__ __forceinline__ float tanh_fast(float x) {

@@ -426,7 +426,23 @@ struct alignas(64) Rb2Params {
   float mono_bias;
   int mono_taps;
   float* wav;                 // [B][L] fp32
+  // padded batch (RAGGED instantiation): valid rows per utterance and the prefix table of its tiles
+  const int* lengths;
+  const int* tile_start;
 };
+
+// Utterance and first window row of `tile`: fixed tiles_per_utt, or the compacted tile space of a padded batch.  Every
+// role goes through here, so they all agree on the tile sequence and the ring / phase counting is unchanged.
+template <bool RAGGED>
+__device__ __forceinline__ void rb2_tile(const Rb2Params& p, int tile, int& b, int& t0) {
+  if constexpr (RAGGED) {
+    b = ragged_tile_utt(p.tile_start, p.B, tile);
+    t0 = (tile - __ldg(p.tile_start + b)) * p.tile_stride - p.tile_lead;
+  } else {
+    b = tile / p.tiles_per_utt;
+    t0 = (tile % p.tiles_per_utt) * p.tile_stride - p.tile_lead;
+  }
+}
 
 // NCH channels starting at c0 of row `row` as two fp16 terms into operand tile(s) at `tiles`, 128-byte swizzle.
 template <int C, int NCH>
@@ -513,7 +529,9 @@ __device__ __forceinline__ void issue_src_f16(uint32_t a0, uint32_t a1, uint32_t
   }
 }
 
-template <int C>
+// RAGGED: a padded batch, only the tiles that hold a valid row (see avc_resblock2_desc.lengths).  A separate
+// instantiation: the fixed-length one is compiled exactly as it is without lengths.
+template <int C, bool RAGGED>
 __global__ void __launch_bounds__(Rb2Cfg<C>::kThreads, Rb2Cfg<C>::kCtasPerSm) resblock2_kernel(const __grid_constant__ Rb2Params p) {
   using Cfg = Rb2Cfg<C>;
   constexpr int P = Cfg::kParts;
@@ -576,7 +594,8 @@ __global__ void __launch_bounds__(Rb2Cfg<C>::kThreads, Rb2Cfg<C>::kCtasPerSm) re
     if (lane == 0) {
       int it = 0;
       for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x, ++it) {
-        const int b = tile / p.tiles_per_utt, t0 = (tile % p.tiles_per_utt) * p.tile_stride - p.tile_lead;
+        int b, t0;
+        rb2_tile<RAGGED>(p, tile, b, t0);
         const int buf = it & 1, use = it >> 1;
         if (use > 0) mbar_wait(&win_free[buf], (use - 1) & 1);
         mbar_arrive_expect_tx(&win_full[buf], P * win_rows * kRowBytes);
@@ -632,7 +651,8 @@ __global__ void __launch_bounds__(Rb2Cfg<C>::kThreads, Rb2Cfg<C>::kCtasPerSm) re
     float* const s_part = reinterpret_cast<float*>(s_mid);      // [2 channel halves][8][128] partial sums (8 KB of 16)
     int it = 0;
     for (int tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x, ++it) {
-      const int b = tile / p.tiles_per_utt, t0 = (tile % p.tiles_per_utt) * p.tile_stride - p.tile_lead;
+      int b, t0;
+      rb2_tile<RAGGED>(p, tile, b, t0);
       float v[NCH];
       uint4 hi[NCH / 8], lo[NCH / 8];
       // ---- epilogue 1: intermediate = LeakyReLU(conv3 + b3) as two fp16 terms in shared memory
@@ -721,16 +741,21 @@ __global__ void __launch_bounds__(Rb2Cfg<C>::kThreads, Rb2Cfg<C>::kCtasPerSm) re
           // output r of this tile is sample t0 + K/2 + r: the sum over the taps k of the per-row partial dot products of
           // tile rows r + k (mirrored at the two ends of the utterance), both channel halves
           const int K = p.mono_taps, t = t0 + p.tile_lead + row;
+          const int len = RAGGED ? __ldg(p.lengths + b) : p.L;     // mirrored at the utterance's own last sample
           if (h == 0 && row < p.tile_stride && t < p.L) {
-            float acc = p.mono_bias;
-            for (int k = 0; k < K; ++k) {
-              int tau = t + k - p.tile_lead;
-              if (tau < 0) tau = -tau;
-              if (tau >= p.L) tau = 2 * (p.L - 1) - tau;
-              const int rr = tau - t0;
-              acc += s_part[k * kBlockM + rr] + s_part[(8 + k) * kBlockM + rr];
+            if (RAGGED && t >= len) {
+              p.wav[(long long)b * p.L + t] = 0.f;
+            } else {
+              float acc = p.mono_bias;
+              for (int k = 0; k < K; ++k) {
+                int tau = t + k - p.tile_lead;
+                if (tau < 0) tau = -tau;
+                if (tau >= len) tau = 2 * (len - 1) - tau;
+                const int rr = tau - t0;
+                acc += s_part[k * kBlockM + rr] + s_part[(8 + k) * kBlockM + rr];
+              }
+              p.wav[(long long)b * p.L + t] = tanh_fast(acc);
             }
-            p.wav[(long long)b * p.L + t] = tanh_fast(acc);
           }
           continue;          // nothing is stored by TMA; the next tile's barrier orders these reads before its writes
         }
@@ -755,10 +780,10 @@ __global__ void __launch_bounds__(Rb2Cfg<C>::kThreads, Rb2Cfg<C>::kCtasPerSm) re
   }
 }
 
-template <int C>
+template <int C, bool RAGGED>
 static int launch2(const Rb2Params& p, cudaStream_t stream) {
   using Cfg = Rb2Cfg<C>;
-  auto kern = resblock2_kernel<C>;
+  auto kern = resblock2_kernel<C, RAGGED>;
   static PerDeviceOnce configured;
   if (configured.first_use()) {
     AVC_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
@@ -792,6 +817,12 @@ extern "C" int avc_resblock2(const avc_resblock2_desc* d, void* stream_v) {
               "avc_resblock2: the fused output convolution takes C = 32 and 3, 5 or 7 taps (C=%d, %d taps)", d->C,
               d->mono_taps);
   AVC_REQUIRE((long long)d->B * d->L < (1LL << 31), "avc_resblock2: B*L too large");
+  if (d->lengths) {
+    const int stride = d->wav ? kBlockM - (d->mono_taps - 1) : kBlockM;
+    AVC_REQUIRE(d->tile_start && d->n_tiles >= d->B && d->n_tiles <= (long long)d->B * ((d->L + stride - 1) / stride),
+                "avc_resblock2: lengths need tile_start and n_tiles in [B, B * ceil(L / %d)] (n_tiles %d)", stride,
+                d->n_tiles);
+  }
   if (d->C == 128) return launch_resblock2_big(d, stream);
   const int C = d->C, P = C == 64 ? 2 : 1;
   const uint64_t B = (uint64_t)d->B, L = (uint64_t)d->L;
@@ -845,7 +876,13 @@ extern "C" int avc_resblock2(const avc_resblock2_desc* d, void* stream_v) {
     p.tiles_per_utt = (d->L + p.tile_stride - 1) / p.tile_stride;
   }
   p.n_tiles = d->B * p.tiles_per_utt;
-  return C == 64 ? launch2<64>(p, stream) : launch2<32>(p, stream);
+  if (d->lengths) {
+    p.lengths = d->lengths;
+    p.tile_start = d->tile_start;
+    p.n_tiles = d->n_tiles;
+    return C == 64 ? launch2<64, true>(p, stream) : launch2<32, true>(p, stream);
+  }
+  return C == 64 ? launch2<64, false>(p, stream) : launch2<32, false>(p, stream);
 }
 
 extern "C" int avc_resblock(const avc_resblock_desc* d, void* stream_v) {

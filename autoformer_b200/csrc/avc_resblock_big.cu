@@ -68,6 +68,7 @@ struct alignas(64) Params {
   int B, L, dilation;
   int n_tiles, tiles_per_utt, n_pairs;
   long long* debug_clk;    // optional: 16 clock64 stamps per tile of CTA 0 (first 64 tiles)
+  const int* tile_start;   // RAGGED: [B + 1] prefix table of the tiles that hold a valid row (avc_resblock2_desc)
 };
 
 __device__ __forceinline__ void tma_store_3d(const void* tmap, const void* smem_src, int c0, int c1, int c2) {
@@ -111,6 +112,9 @@ __device__ __forceinline__ void write_split32(uint8_t* tiles, int row, int c0, c
 
 using namespace big;      // (the kernel itself lives in avc:: so that profilers list it beside the library's other kernels)
 
+// RAGGED: a padded batch, only the tiles that hold a valid row; a separate instantiation, the fixed-length one is compiled
+// exactly as it is without lengths.
+template <bool RAGGED>
 __global__ void __launch_bounds__(big::kThreads, 1) resblock2_big_kernel(const __grid_constant__ big::Params p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* base = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -170,12 +174,22 @@ __global__ void __launch_bounds__(big::kThreads, 1) resblock2_big_kernel(const _
     if (p.debug_clk && blockIdx.x == 0 && it < 64) p.debug_clk[it * 16 + k] = clock64();
   };
 
-  // tile of this CTA in pair-iteration `u`: 2u + rank (a phantom tile past the end loads zeros and stores nothing)
+  // tile of this CTA in pair-iteration `u`: 2u + rank (a phantom tile past the end loads zeros and stores nothing).  In a
+  // padded batch the tiles are those that hold a valid row, and the two tiles of a pair may belong to two utterances.
   auto tile_coords = [&](int u, int& b, int& t0, bool& real) {
     const int tile = 2 * u + rank;
     real = tile < p.n_tiles;
-    b = tile / p.tiles_per_utt;
-    t0 = (tile - b * p.tiles_per_utt) * kBlockM;
+    if constexpr (RAGGED) {
+      b = p.B;                 // phantom: the utterance past the last one, all of it out of bounds
+      t0 = 0;
+      if (real) {
+        b = ragged_tile_utt(p.tile_start, p.B, tile);
+        t0 = (tile - __ldg(p.tile_start + b)) * kBlockM;
+      }
+    } else {
+      b = tile / p.tiles_per_utt;
+      t0 = (tile - b * p.tiles_per_utt) * kBlockM;
+    }
   };
 
   if (warp == 0) {
@@ -456,11 +470,15 @@ int launch_resblock2_big(const avc_resblock2_desc* d, cudaStream_t stream) {
   p.dilation = d->dilation;
   p.tiles_per_utt = d->L / kBlockM;
   p.n_tiles = d->B * p.tiles_per_utt;
+  if (d->lengths) {
+    p.tile_start = d->tile_start;
+    p.n_tiles = d->n_tiles;
+  }
   p.n_pairs = (p.n_tiles + 1) / 2;
   p.debug_clk = d->debug_clk;
-  auto kern = resblock2_big_kernel;
-  static PerDeviceOnce configured;
-  if (configured.first_use()) {
+  auto kern = d->lengths ? resblock2_big_kernel<true> : resblock2_big_kernel<false>;
+  static PerDeviceOnce configured[2];
+  if (configured[d->lengths ? 1 : 0].first_use()) {
     AVC_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
   }
   const int resident_pairs = num_sms() / 2;

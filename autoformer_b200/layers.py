@@ -192,10 +192,9 @@ def conv_bn_layer(sd, prefix, precision, act, bn_owner=None):
     return ops.ConvGemm(*packing.pack_conv(w, b, precision), act=act, tag="conv")
 
 
-def upload_lengths(lengths, B, T, device, multiple=1):
+def check_lengths(lengths, B, T, multiple=1):
     """Per-utterance lengths of a padded batch (a list, a CPU tensor or a CUDA tensor, read back once), validated on the
-    host -- B entries, 1 <= lengths[b] <= T, multiples of `multiple` -- and uploaded once as a device int32 [B] tensor.
-    The kernels trust these values, so nothing unchecked reaches them."""
+    host -- B entries, 1 <= lengths[b] <= T, multiples of `multiple` -- as a list of ints."""
     if torch.is_tensor(lengths):
         lengths = lengths.detach().cpu().reshape(-1).tolist()
     vals = [int(v) for v in lengths]
@@ -208,7 +207,13 @@ def upload_lengths(lengths, B, T, device, multiple=1):
     if bad:
         raise ValueError(f"lengths must be multiples of freq={multiple} (pad each utterance as pipeline.convert does); "
                          f"got {bad[:4]}")
-    return torch.tensor(vals, dtype=torch.int32).to(device)
+    return vals
+
+
+def upload_lengths(lengths, B, T, device, multiple=1):
+    """``check_lengths``, then uploaded once as a device int32 [B] tensor.  The kernels trust these values, so nothing
+    unchecked reaches them."""
+    return torch.tensor(check_lengths(lengths, B, T, multiple), dtype=torch.int32).to(device)
 
 
 def _lengths_kw(lengths):

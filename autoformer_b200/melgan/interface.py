@@ -30,7 +30,10 @@ class MelVocoder:
         """audio (B, L) -> log-mel (B, 80, L // 256)   (interface.py:33-41)."""
         return self.fft(audio.unsqueeze(1).to(self.device))
 
-    def inverse(self, mel):
-        """mel (B, 80, T) -> waveform (B, 256 T)."""
+    def inverse(self, mel, lengths=None):
+        """mel (B, 80, T) -> waveform (B, 256 T).  lengths: a zero-padded batch of utterances of lengths[b] frames
+        (Generator.forward); samples past 256 lengths[b] are 0."""
         with torch.no_grad():
-            return self.mel2wav(mel.to(self.device)).squeeze(1)
+            if lengths is None:
+                return self.mel2wav(mel.to(self.device)).squeeze(1)
+            return self.mel2wav(mel.to(self.device), lengths=lengths).squeeze(1)

@@ -245,13 +245,29 @@ class Generator(layers.PlanOwner, nn.Module):
         build = (lambda: _PlanF16s(self)) if self.precision == "fp16s" else (lambda: _Plan(self, self.precision))
         return self._cache.get(self, (self.precision,), build)
 
-    def _forward_f16s(self, plan, x):
-        """The "fp16s" data flow (see _PlanF16s): raw residual stream as two fp16 terms, one tensor between kernels."""
+    def _ragged_rows(self, plan, lengths, B, T, device):
+        """Validated lengths of a padded batch -> RaggedRows of the stem (index 0) and of every stage (index si + 1),
+        one upload.  The reference's own ReflectionPad1d(3) needs at least 4 frames."""
+        vals = layers.check_lengths(lengths, B, T)
+        if min(vals) < 4:
+            raise ValueError(f"lengths must be at least 4 frames (ReflectionPad1d(3) of the first layer); got {min(vals)}")
+        if self.collect_taps:
+            raise NotImplementedError("stage taps (collect_taps) of a variable-length batch")
+        scales = [1]
+        for r in self.ratios:
+            scales.append(scales[-1] * r)
+        return ops.ragged_rows(vals, scales, (128, 128 - (plan.w_out.shape[0] - 1)), device)
+
+    def _forward_f16s(self, plan, x, rows=None):
+        """The "fp16s" data flow (see _PlanF16s): raw residual stream as two fp16 terms, one tensor between kernels.
+        rows: RaggedRows per level of a padded batch (see forward)."""
         B, _, T = x.shape
         dev = x.device
         P = "fp16s"
         taps = self.taps if self.collect_taps else None
         m0 = ops.transpose_pad(x, 3, P)                                   # model.0 + layout change
+        if rows is not None:
+            ops.reflect_halo(m0, 3, T, 3, lengths=rows[0].rows)           # ReflectionPad1d(3) at each utterance's end
         cur = ops.alloc_act(B, T, plan.stem.meta["N"], P, dev)
         plan.stem(m0, B, T, out=cur)                                      # model.1 (+ model.2's LeakyReLU)
         L = T
@@ -261,32 +277,42 @@ class Generator(layers.PlanOwner, nn.Module):
             Lr = r * L
             last_stage = si + 1 == n_stage
             d0 = blocks[0][0]
+            rs = rows[si + 1] if rows is not None else None
+            halo_kw = layers._lengths_kw(rs.rows if rs is not None else None)
+            block_kw = layers._lengths_kw(rs)
+            if rows is not None:
+                ops.zero_tail(cur, 0, L, rows[si].rows)    # the ConvTranspose reads frame m + 1 = lengths[b] as zero
             if self.fuse_resblocks and ops.Resblock2.eligible(C, Lr):
                 xs = ops.alloc_act(B, Lr + 2 * d0, C, P, dev)
                 for up, p0 in up_raw:                                                   # ConvTranspose1d: raw stream
                     up(cur, B, L, out=xs, out_row0=d0, phases=r, phase0=p0, phase_count=r // len(up_raw))
-                ops.reflect_halo(xs, d0, Lr, d0)                                        # + the first block's halo rows
+                ops.reflect_halo(xs, d0, Lr, d0, **halo_kw)                             # + the first block's halo rows
                 if taps is not None:
                     taps[f"up{si}"] = packing.act_to_float(xs[:, d0:d0 + Lr], P)
                 for j, (d, _, _, fused) in enumerate(blocks):
                     if j + 1 < len(blocks):
                         dn = blocks[j + 1][0]
                         ys = ops.alloc_act(B, Lr + 2 * dn, C, P, dev)
-                        fused(xs, B, Lr, y=ys, y_row0=dn, y_reflect=dn)
+                        fused(xs, B, Lr, y=ys, y_row0=dn, y_reflect=dn, **block_kw)
+                        if rs is not None:
+                            # the right halo at each utterance's end: its rows lie inside the last tile, which the
+                            # block TMA-stores whole, so they are written after the block, not by it
+                            ops.reflect_halo(ys, dn, Lr, dn, lengths=rs.rows)
                         xs = ys
                     elif not last_stage:
                         cur = ops.alloc_act(B, Lr, C, P, dev)
-                        fused(xs, B, Lr, y=cur, y_act=True)                              # + the next model.{i} LeakyReLU
+                        fused(xs, B, Lr, y=cur, y_act=True, **block_kw)                  # + the next model.{i} LeakyReLU
                         if taps is not None:
                             taps[f"stage{si}"] = _inv_lrelu(packing.act_to_float(cur, P))
                     elif taps is None and self.fuse_output_conv and C == 32:
                         # model.22-25 (LeakyReLU, ReflectionPad1d(3), Conv1d(32 -> 1, k7), tanh) in the block's epilogue:
-                        # the block's output (1 GB at B = 32) is neither written nor re-read
-                        wav = torch.empty(B, Lr, dtype=torch.float32, device=dev)
-                        fused(xs, B, Lr, wav=wav, mono=(plan.w_out, plan.b_out))
+                        # the block's output (1 GB at B = 32) is neither written nor re-read.  A padded batch skips the
+                        # tiles past each utterance's end, so their samples come from the zero fill.
+                        wav = (torch.zeros if rs is not None else torch.empty)(B, Lr, dtype=torch.float32, device=dev)
+                        fused(xs, B, Lr, wav=wav, mono=(plan.w_out, plan.b_out), **block_kw)
                     else:
                         final = torch.empty(B * Lr, C, dtype=torch.float32, device=dev)
-                        fused(xs, B, Lr, out2=final)
+                        fused(xs, B, Lr, out2=final, **block_kw)
                         if taps is not None:
                             taps[f"stage{si}"] = _inv_lrelu(final.view(B, Lr, C))
             else:
@@ -295,7 +321,7 @@ class Generator(layers.PlanOwner, nn.Module):
                 for up, p0 in up_act:
                     up(cur, B, L, out=xa, out_row0=d0, out_raw=x_raw, phases=r, out_fmt="f16", raw_fmt=P, phase0=p0,
                        phase_count=r // len(up_act))
-                ops.reflect_halo(xa, d0, Lr, d0)
+                ops.reflect_halo(xa, d0, Lr, d0, **halo_kw)
                 if taps is not None:
                     taps[f"up{si}"] = packing.act_to_float(x_raw, P)
                 for j, (d, c3, k1, _) in enumerate(blocks):
@@ -305,8 +331,10 @@ class Generator(layers.PlanOwner, nn.Module):
                         dn = blocks[j + 1][0]
                         y_raw = ops.alloc_act(B, Lr, C, P, dev)
                         ya = ops.alloc_act(B, Lr + 2 * dn, C, "f16", dev)
-                        k1([h1, x_raw], B, Lr, out=ya, out_row0=dn, reflect=dn, out_raw=y_raw, out_fmt="f16", raw_fmt=P,
-                           halo_after=True)
+                        k1([h1, x_raw], B, Lr, out=ya, out_row0=dn, reflect=dn if rs is None else 0, out_raw=y_raw,
+                           out_fmt="f16", raw_fmt=P, halo_after=True)
+                        if rs is not None:
+                            ops.reflect_halo(ya, dn, Lr, dn, lengths=rs.rows)
                         x_raw, xa = y_raw, ya
                     elif not last_stage:
                         cur = ops.alloc_act(B, Lr, C, P, dev)
@@ -320,20 +348,28 @@ class Generator(layers.PlanOwner, nn.Module):
                             taps[f"stage{si}"] = _inv_lrelu(final.view(B, Lr, C))
             L = Lr
         if wav is None:
-            wav = ops.conv_to_mono_tanh(final.view(B, L, -1), plan.w_out, plan.b_out)  # model.22-25
+            last_kw = layers._lengths_kw(rows[-1].rows if rows is not None else None)
+            wav = ops.conv_to_mono_tanh(final.view(B, L, -1), plan.w_out, plan.b_out, **last_kw)  # model.22-25
         return wav.unsqueeze(1)
 
     @ops.on_device_of_input
     @torch.no_grad()
-    def forward(self, x):
-        """x (B, input_size, T) log-mel -> waveform (B, 1, hop_length * T)   (melgan/modules.py:129-130)."""
+    def forward(self, x, lengths=None):
+        """x (B, input_size, T) log-mel -> waveform (B, 1, hop_length * T)   (melgan/modules.py:129-130).
+
+        lengths (list, CPU or CUDA tensor of B ints, 4 <= lengths[b] <= T): a zero-padded batch of utterances of
+        different lengths.  Samples < hop_length * lengths[b] of utterance b are what the generator gives for
+        x[b:b+1, :, :lengths[b]] alone, the samples past them are 0, and whatever x holds past lengths[b] is ignored."""
         ops._require_cuda(x)
         plan = self._plan()
         prec = plan.precision
+        rows = None
+        if lengths is not None:
+            rows = self._ragged_rows(plan, lengths, x.shape[0], x.shape[2], x.device)
         if prec == "fp16s":
             if self.collect_taps:
                 self.taps.clear()
-            return self._forward_f16s(plan, x.contiguous().float())
+            return self._forward_f16s(plan, x.contiguous().float(), rows)
         x = x.contiguous().float()
         B, _, T = x.shape
         dev = x.device
@@ -341,6 +377,8 @@ class Generator(layers.PlanOwner, nn.Module):
         if taps is not None:
             taps.clear()
         m0 = ops.transpose_pad(x, 3, prec)                                # model.0 + layout change
+        if rows is not None:
+            ops.reflect_halo(m0, 3, T, 3, lengths=rows[0].rows)           # ReflectionPad1d(3) at each utterance's end
         cur = ops.alloc_act(B, T, plan.stem.meta["N"], prec, dev)
         plan.stem(m0, B, T, out=cur)                                      # model.1 (+ model.2's LeakyReLU)
         L = T
@@ -349,9 +387,14 @@ class Generator(layers.PlanOwner, nn.Module):
         for si, (r, C, up, blocks) in enumerate(plan.stages):
             Lr = r * L
             d0 = blocks[0][0]
+            rs = rows[si + 1] if rows is not None else None
+            if rows is not None:
+                ops.zero_tail(cur, 0, L, rows[si].rows)    # the ConvTranspose reads frame m + 1 = lengths[b] as zero
             x_raw = ops.alloc_act(B, Lr, C, prec, dev)
             xa = ops.alloc_act(B, Lr + 2 * d0, C, prec, dev)
             up(cur, B, L, out=xa, out_row0=d0, reflect=d0, out_raw=x_raw, phases=r)     # ConvTranspose1d
+            if rs is not None:
+                ops.reflect_halo(xa, d0, Lr, d0, lengths=rs.rows)          # the right halo at each utterance's end
             if taps is not None:
                 taps[f"up{si}"] = packing.act_to_float(x_raw, prec)
             fuse = self.fuse_resblocks and ops.Resblock.eligible(C, Lr, prec)
@@ -368,6 +411,8 @@ class Generator(layers.PlanOwner, nn.Module):
                     y_raw = ops.alloc_act(B, Lr, C, prec, dev)
                     ya = ops.alloc_act(B, Lr + 2 * dn, C, prec, dev)
                     run(out=ya, out_row0=dn, reflect=dn, out_raw=y_raw)
+                    if rs is not None:
+                        ops.reflect_halo(ya, dn, Lr, dn, lengths=rs.rows)
                     x_raw, xa = y_raw, ya
                 elif si + 1 < n_stage:
                     cur = ops.alloc_act(B, Lr, C, prec, dev)
@@ -382,5 +427,6 @@ class Generator(layers.PlanOwner, nn.Module):
                     if taps is not None:
                         taps[f"stage{si}"] = packing.act_to_float(raw, prec)
             L = Lr
-        wav = ops.conv_to_mono_tanh(final.view(B, L, -1), plan.w_out, plan.b_out)      # model.22-25
+        last_kw = layers._lengths_kw(rows[-1].rows if rows is not None else None)
+        wav = ops.conv_to_mono_tanh(final.view(B, L, -1), plan.w_out, plan.b_out, **last_kw)      # model.22-25
         return wav.unsqueeze(1)

@@ -244,15 +244,18 @@ class ConvGemm:
         return out if out is not None else (out2 if out2 is not None else out_raw)
 
 
-def reflect_halo(buf, row0, L, reflect):
-    """Fill the `reflect` mirrored rows each side of rows [row0, row0 + L) of a channels-last buffer [B][rows][C']."""
+def reflect_halo(buf, row0, L, reflect, lengths=None):
+    """Fill the `reflect` mirrored rows each side of rows [row0, row0 + L) of a channels-last buffer [B][rows][C'].
+    lengths (device int32 [B], reflect < lengths[b] <= L): utterance b of a padded batch ends at row row0 + lengths[b]
+    - 1, and its right halo mirrors about that row."""
     lib = _lib.load()
     _require_cuda(buf)
     assert buf.dim() == 3 and buf.is_contiguous()
     B, rows, _ = buf.shape
+    lens = _check_lengths(lengths, B) if lengths is not None else None
     with PROFILER.span("halo", bytes=float(2 * B * 2 * reflect * buf.shape[2] * buf.element_size())):
         _lib.check(lib.avc_reflect_halo(buf.data_ptr(), B, rows, buf.shape[2] * buf.element_size(), row0, L, reflect,
-                                        _stream()), "avc_reflect_halo")
+                                        _stream(), lens), "avc_reflect_halo")
     return buf
 
 
@@ -276,6 +279,38 @@ def zero_tail(buf, row0, T, lengths):
         _lib.check(lib.avc_zero_tail(buf.data_ptr(), B, rows, row_bytes, row0, T, _check_lengths(lengths, B), _stream()),
                    "avc_zero_tail")
     return buf
+
+
+class RaggedRows:
+    """Valid rows per utterance of one buffer geometry (one generator stage) of a padded batch.  ``host``: list of B
+    ints; ``rows``: the same as a device int32 [B] tensor (the ``lengths`` of reflect_halo / zero_tail /
+    conv_to_mono_tanh); ``tiles[S]``: (device int32 [B + 1] prefix table of ceil(host[b] / S), its total) -- the
+    compacted tile space avc_resblock2 runs over with tiles of stride S."""
+
+    def __init__(self, host, rows, tiles):
+        self.host, self.rows, self.tiles = host, rows, tiles
+
+
+def ragged_rows(lengths, scales, strides, device):
+    """RaggedRows of rows = s * lengths[b] for every scale s, with tile tables for every stride.  `lengths` is a host
+    list already validated by the caller; all rows and tables go to the device in ONE int32 copy."""
+    B = len(lengths)
+    flat, layout = [], []
+    for s in scales:
+        host = [s * n for n in lengths]
+        off = len(flat)
+        flat += host
+        tables = {}
+        for S in strides:
+            start = [0]
+            for r in host:
+                start.append(start[-1] + (r + S - 1) // S)
+            tables[S] = (len(flat), start[-1])
+            flat += start
+        layout.append((host, off, tables))
+    dev = torch.tensor(flat, dtype=torch.int32).to(device)
+    return [RaggedRows(host, dev[off:off + B], {S: (dev[o:o + B + 1], n) for S, (o, n) in tables.items()})
+            for host, off, tables in layout]
 
 
 # Cap on the CTAs one persistent LSTM launch may take (None: the whole device).  pipeline.convert_pairs sets it to half
@@ -607,17 +642,19 @@ def transpose_pad(x, pad, precision, round_tf32=True):
     return out
 
 
-def conv_to_mono_tanh(x, w, bias):
-    """x [B][L][C] fp32, w [K][C] fp32 -> tanh(conv) [B][L] with reflect padding K//2."""
+def conv_to_mono_tanh(x, w, bias, lengths=None):
+    """x [B][L][C] fp32, w [K][C] fp32 -> tanh(conv) [B][L] with reflect padding K//2.  lengths (device int32 [B],
+    K // 2 < lengths[b] <= L): utterance b reflects at its own last sample, its samples past it are 0."""
     lib = _lib.load()
     _require_cuda(x, w)
     assert x.dtype == torch.float32 and x.is_contiguous() and w.dtype == torch.float32 and w.is_contiguous()
     B, L, C = x.shape
     K = w.shape[0]
+    lens = _check_lengths(lengths, B) if lengths is not None else None
     out = torch.empty(B, L, dtype=torch.float32, device=x.device)
     with PROFILER.span("mono_conv", bytes=float(x.numel() * 4 + out.numel() * 4), flops=2.0 * K * C * B * L):
         _lib.check(lib.avc_conv_to_mono_tanh(x.data_ptr(), w.data_ptr(), float(bias), out.data_ptr(), B, L, C, K,
-                                             _stream()), "avc_conv_to_mono_tanh")
+                                             _stream(), lens), "avc_conv_to_mono_tanh")
     return out
 
 
@@ -691,12 +728,16 @@ class Resblock2:
         self.w, self.bias3, self.bias1 = self.w.to(device), self.bias3.to(device), self.bias1.to(device)
         return self
 
-    def __call__(self, x, B, L, y=None, y_row0=0, y_reflect=0, y_act=False, out2=None, wav=None, mono=None):
+    def __call__(self, x, B, L, y=None, y_row0=0, y_reflect=0, y_act=False, out2=None, wav=None, mono=None,
+                 lengths=None):
         """x [B][L + 2d][2C] fp16 two-term residual stream with reflected halo rows (time t at row t + d).
         y: raw output (y_act False) or LeakyReLU(output) (True) as two fp16 terms [B][rows][2C] at rows y_row0 + t
         (+ `y_reflect` mirrored halo rows); out2: LeakyReLU(output) as exact fp32 [B*L][C]; wav [B][L] fp32 with
         mono = (w [K][C] fp32, bias): the generator's output layer applied in the block's epilogue (C = 32).
-        Exactly one of y / out2 / wav."""
+        Exactly one of y / out2 / wav.
+        lengths (RaggedRows of this stage): a padded batch -- only the tiles holding a valid row run, wav reflects at
+        each utterance's end and is 0 past it in its last tile; the right halo of y at each utterance's end is the
+        caller's (reflect_halo with lengths), and so is zero-filling wav."""
         lib = _lib.load()
         C, d = self.C, self.dilation
         _require_cuda(self.w, x)
@@ -721,12 +762,19 @@ class Resblock2:
             assert wav.dtype == torch.float32 and wav.shape == (B, L) and wav.is_contiguous()
             assert w_out.dtype == torch.float32 and w_out.is_contiguous() and w_out.shape[1] == C and w_out.shape[0] in (3, 5, 7)
             desc.wav, desc.mono_w, desc.mono_bias, desc.mono_taps = wav.data_ptr(), w_out.data_ptr(), float(b_out), w_out.shape[0]
+        rows = B * L
+        if lengths is not None:
+            assert isinstance(lengths, RaggedRows) and len(lengths.host) == B and max(lengths.host) <= L
+            stride = 128 - (mono[0].shape[0] - 1) if wav is not None else 128
+            tile_start, n_tiles = lengths.tiles[stride]
+            desc.lengths, desc.tile_start, desc.n_tiles = _check_lengths(lengths.rows, B), tile_start.data_ptr(), n_tiles
+            rows = sum(lengths.host)
         dbg = getattr(self, "debug_clk", None)
         if dbg is not None:
             desc.debug_clk = dbg.data_ptr()
-        extra = 2.0 * mono[0].numel() * B * L if wav is not None else 0.0
-        with PROFILER.span(self.tag, flops=2.0 * 5 * C * C * B * L + extra,
-                           bytes=float(x.numel() * 2 + (B * L * 4 if wav is not None else B * L * C * 4))):
+        extra = 2.0 * mono[0].numel() * rows if wav is not None else 0.0
+        with PROFILER.span(self.tag, flops=2.0 * 5 * C * C * rows + extra,
+                           bytes=float(x.numel() * 2 * rows / (B * L) + (rows * 4 if wav is not None else rows * C * 4))):
             _lib.check(lib.avc_resblock2(ctypes.byref(desc), _stream()), "avc_resblock2")
         return y if y is not None else (out2 if out2 is not None else wav)
 

@@ -4,8 +4,9 @@ Follows the reference's own recipe for utterances whose length is not a multiple
 the end, convert, trim the padding off again (util/evaluate.py:36-43 ``crop_mel`` pads with constant 0;
 :85-92 trims ``mel_trans`` back), then vocode ``mel_trans.transpose(2, 1)`` (conversion.ipynb cell 14,
 util/evaluate.py:96-98).  ``convert`` and ``convert_batches`` take batches whose utterances share one T (plain zero
-padding changes the result, SURVEY.md 5); ``convert_utterances`` and ``embed_utterances`` take utterances of any length
-and batch them with per-utterance lengths, which gives each one exactly its result converted alone."""
+padding changes the result, SURVEY.md 5); ``convert_utterances``, ``embed_utterances``, ``vocode_utterances`` and
+``convert_and_vocode_utterances`` take utterances of any length and batch them with per-utterance lengths, which gives
+each one exactly its result computed alone."""
 import os
 
 import numpy as np
@@ -196,6 +197,40 @@ def embed_utterances(embedder, mels, max_batch=64):
         for k, i in enumerate(ids):
             out[i] = e[k]
     return torch.stack(out)
+
+
+@torch.no_grad()
+def vocode_utterances(generator, mels, max_batch=32):
+    """MelGAN waveforms of utterances of any lengths: mels is a list of (T_i, 80) device tensors, T_i >= 4.  The
+    utterances are batched by ``sharding.make_ragged_batches`` on their exact lengths and each batch is vocoded once
+    with per-utterance lengths.  A batch is padded to an even number of frames, so that every stage of 32 / 64 / 128
+    channels takes the fused ResnetBlock kernels (their stage length 64 T must be a multiple of 128).  Returns the list
+    of waveforms (hop_length * T_i,) in input order, each what the generator gives for the utterance alone."""
+    from . import sharding
+    out = [None] * len(mels)
+    hop = generator.hop_length
+    for T_batch, ids in sharding.make_ragged_batches([m.shape[0] for m in mels], max_batch, 1):
+        T_pad = T_batch + T_batch % 2
+        x = mels[ids[0]].new_zeros(len(ids), mels[ids[0]].shape[1], T_pad)
+        lens = [mels[i].shape[0] for i in ids]
+        for k, i in enumerate(ids):
+            x[k, :, :lens[k]] = mels[i].t()
+        wav = generator(x, lengths=lens).squeeze(1)
+        for k, i in enumerate(ids):
+            out[i] = wav[k, :hop * lens[k]]
+    return out
+
+
+@torch.no_grad()
+def convert_and_vocode_utterances(embedder, model, generator, mels_src, mels_trg_ref):
+    """``convert_and_vocode`` on utterances of any lengths (lists of (T_i, 80) and (T2_i, 80) device tensors):
+    ``embed_utterances`` -> ``convert_utterances`` -> ``vocode_utterances``, each with variable-length batches.
+    Returns (converted mels [(T_i, 80)], waveforms [(256 T_i,)], emb_org, emb_trg), in input order."""
+    n = len(mels_src)
+    emb = embed_utterances(embedder, list(mels_src) + list(mels_trg_ref))
+    emb_org, emb_trg = emb[:n], emb[n:]
+    mels = convert_utterances(model, mels_src, emb_org, emb_trg)
+    return mels, vocode_utterances(generator, mels), emb_org, emb_trg
 
 
 # ------------------------------------------------------------------------------------------------ side-by-side batches

@@ -207,6 +207,19 @@ typedef struct avc_resblock2_desc {
   const float* mono_w;       /* [K][C] fp32 */
   float mono_bias;
   int mono_taps;             /* K: 3, 5 or 7 */
+  /* A padded batch (optional): utterance b has lengths[b] valid rows at this stage, 1 <= lengths[b] <= L.  Only the tiles
+   * that hold a valid row run: ceil(lengths[b] / S) of utterance b, S = 128, or 128 - (K - 1) with wav.  tile_start
+   * [B + 1] is their prefix table (tile_start[0] = 0, tile_start[b + 1] = tile_start[b] + ceil(lengths[b] / S)) and
+   * n_tiles = tile_start[B]; every role of the kernel maps a tile index to its utterance by binary search.  Output rows
+   * of skipped tiles are not written.  The last tile of an utterance computes and stores all its rows, rows at and past
+   * lengths[b] included (their values are not those of the utterance alone), so the right halo of y for the next
+   * block is the caller's: avc_reflect_halo with the same lengths, after this launch.  With wav the output layer
+   * reflects at lengths[b] - 1 and writes 0 for the samples of the last tile at and past lengths[b]; wav samples of
+   * skipped tiles are not written (zero-fill wav first).  lengths = NULL: every utterance has L rows, as without these
+   * fields. */
+  const int* lengths;
+  const int* tile_start;
+  int n_tiles;
 } avc_resblock2_desc;
 
 int avc_resblock2(const avc_resblock2_desc* d, void* stream);
@@ -356,8 +369,12 @@ int avc_linear_rows(const float* h, const float* w, const float* bias, float* ou
  * (melgan/modules.py:77,96,121).  avc_conv_gemm can write these rows itself (out_reflect), but only on its general
  * epilogue path; the MelGAN "fp16s" layers keep the GEMM on its branch-free path and add the 2 x reflect rows per
  * utterance with this launch (a few KB).  row_bytes multiple of 16.
+ * lengths: optional [B] int32 device (NULL = every utterance has L rows), reflect < lengths[b] <= L: the right halo of
+ * utterance b mirrors about row row0 + lengths[b] - 1 instead (a padded batch; its rows row0 + lengths[b] .. are
+ * overwritten).  The left halo is the same either way.
  */
-int avc_reflect_halo(void* buf, int B, int rows_per_utt, long long row_bytes, int row0, int L, int reflect, void* stream);
+int avc_reflect_halo(void* buf, int B, int rows_per_utt, long long row_bytes, int row0, int L, int reflect, void* stream,
+                     const int* lengths);
 
 /*
  * Zero the padded tail of every utterance of a channels-last buffer [B][rows_per_utt][row_bytes]: rows
@@ -382,9 +399,11 @@ int avc_transpose_pad(const float* in, void* out, int B, int C, int L, int pad, 
  * MelGAN output layer: out[b, t] = tanh( bias + sum_k sum_c w[k][c] * x[b, reflect(t + k - K/2), c] )
  * (ReflectionPad1d(3) + WNConv1d(32 -> 1, k7) + Tanh, melgan/modules.py:120-124; the preceding LeakyReLU is applied
  * by the producer).  x [B][L][C] fp32, w [K][C] fp32 (weight norm folded), out [B][L] fp32.  K odd <= 15, C <= 64.
+ * lengths: optional [B] int32 device (NULL = all L), K / 2 < lengths[b] <= L: utterance b reflects at its own last
+ * sample lengths[b] - 1, and out[b, t] = 0 for t >= lengths[b]; rows of x past lengths[b] are never read.
  */
 int avc_conv_to_mono_tanh(const float* x, const float* w, float bias, float* out, int B, int L, int C, int K,
-                          void* stream);
+                          void* stream, const int* lengths);
 
 /* ------------------------------------------------------------------------------------------------------------
  * MetaPool / MetaConv glue (factory/MetaPool.py, factory/MetaConv.py, factory/MLPMixer.py).  All inputs are fp32
