@@ -6,7 +6,6 @@
 // k-block, shifted in time by the tap offset; frames outside the utterance are zero-filled by TMA, which IS
 // the convolution's zero padding -- tiles never bleed across utterances.
 #include <cuda_bf16.h>
-#include <cstdlib>
 
 #include "../../include/avc_b200.h"
 #include "avc_host.h"
@@ -535,16 +534,6 @@ static int launch(const GemmParams& p, long long m_tiles, int ctas, cudaStream_t
   return ctas == 2 ? launch_impl<BN, BF16, 2>(p, m_tiles, stream) : launch_impl<BN, BF16, 1>(p, m_tiles, stream);
 }
 
-// CTA pairs by default; AVC_CTA_GROUP=1 forces the single-CTA kernel (A/B testing).
-static int default_cta_group() {
-  static int v = 0;
-  if (v == 0) {
-    const char* e = getenv("AVC_CTA_GROUP");
-    v = (e && e[0] == '1') ? 1 : 2;
-  }
-  return v;
-}
-
 }  // namespace avc
 
 extern "C" int avc_conv_gemm(const avc_gemm_desc* d, void* stream_v) {
@@ -614,7 +603,7 @@ extern "C" int avc_conv_gemm(const avc_gemm_desc* d, void* stream_v) {
   p.num_kb = kb_total;
   AVC_REQUIRE(kb_total * kc == d->k_pad, "avc_conv_gemm: k_pad %d != %d k-blocks x %d", d->k_pad, kb_total, kc);
   const long long m_tiles = (long long)p.tiles_t * tiles_b;
-  int ctas = d->cta_group == 1 || d->cta_group == 2 ? d->cta_group : default_cta_group();
+  int ctas = d->cta_group == 1 ? 1 : 2;     // CTA pairs unless the descriptor asks for single CTAs
   if (m_tiles < 2) ctas = 1;
   // each CTA of a pair stages bn / 2 rows of the weight tile
   if (!encode_tmap_2d(&p.tmap_b, es, d->w_ptr, (uint64_t)d->k_pad, (uint64_t)d->n_pad, (uint64_t)d->k_pad * es, kc,

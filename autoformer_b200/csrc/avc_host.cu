@@ -2,6 +2,7 @@
 #include "avc_host.h"
 
 #include <atomic>
+#include <cstdlib>
 #include <cstring>
 #include <mutex>
 
@@ -98,6 +99,42 @@ int num_sms() {
   if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= PerDeviceOnce::kMaxDevices) return 148;
   if (n[dev] == 0 && cudaDeviceGetAttribute(&n[dev], cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) n[dev] = 148;
   return n[dev];
+}
+
+int persistent_launch_config(cudaLaunchConfig_t& cfg, cudaLaunchAttribute (&attr)[2], const void* kern, int cluster,
+                             const char* name) {
+  static const bool no_coop = getenv("AVC_LSTM_NO_COOP") != nullptr;
+  int na = 0;
+  if (cluster > 1) {
+    attr[na].id = cudaLaunchAttributeClusterDimension;
+    attr[na].val.clusterDim.x = cluster;
+    attr[na].val.clusterDim.y = 1;
+    attr[na].val.clusterDim.z = 1;
+    ++na;
+  }
+  if (!no_coop) {
+    attr[na].id = cudaLaunchAttributeCooperative;
+    attr[na].val.cooperative = 1;
+    ++na;
+  }
+  cfg.attrs = attr;
+  cfg.numAttrs = na;
+  int resident = 0;
+  if (cluster > 1) {
+    int clusters = 0;
+    AVC_CHECK_CUDA(cudaOccupancyMaxActiveClusters(&clusters, kern, &cfg));
+    resident = clusters * cluster;
+  } else {
+    int per_sm = 0;
+    AVC_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, (int)cfg.blockDim.x, cfg.dynamicSmemBytes));
+    resident = per_sm * num_sms();
+  }
+  const int grid = (int)cfg.gridDim.x;
+  if (resident < grid) {
+    set_error("%s: persistent grid %d does not fit (%d CTAs resident)", name, grid, resident);
+    return AVC_ERR_NOT_RESIDENT;
+  }
+  return 0;
 }
 
 }  // namespace avc

@@ -26,6 +26,15 @@ bool encode_tmap_2d(CUtensorMap* map, int elem_bytes, const void* base, uint64_t
 
 int num_sms();   // of the CURRENT device (cached per device)
 
+// Launch set-up of a persistent kernel whose CTAs wait on each other through a grid barrier: the cluster attribute
+// (cluster > 1) and the cooperative attribute go into `attr` / `cfg`, then the occupancy query.  A grid that cannot be
+// resident at once returns AVC_ERR_NOT_RESIDENT with the error text set, before anything is launched, so the caller may
+// fall back.  AVC_LSTM_NO_COOP set (profiling aid: a profiler cannot replay a cooperative launch) drops the cooperative
+// attribute: co-residency then rests on this occupancy check on an otherwise idle GPU, and the kernels' bounded waits
+// turn a violation into a trap.  Returns 0, AVC_ERR_NOT_RESIDENT, or -2 on a CUDA error.
+int persistent_launch_config(cudaLaunchConfig_t& cfg, cudaLaunchAttribute (&attr)[2], const void* kern, int cluster,
+                             const char* name);
+
 // Per-device "already configured" flag for a kernel's cudaFuncSetAttribute: function attributes are per device, so a
 // process that drives several GPUs must set them once on each.  One instance per kernel instantiation (a function-local
 // static at the launch site); `first_use()` returns true exactly once per (instance, current device).

@@ -25,7 +25,6 @@
 //   per-step    t_end = t_begin + 1, one launch per frame (stream order is the time dependency)
 //   persistent  one cooperative launch for all frames; a barrier among the CTAs of a batch group separates frames
 #include <cuda_bf16.h>
-#include <cstdlib>
 #include <type_traits>
 
 #include "../../include/avc_b200.h"
@@ -125,40 +124,6 @@ __device__ __forceinline__ void load_gates(uint32_t lane_addr, int j, float (&z)
   }
 }
 
-// The same for a group of U (4 or 8) hidden units starting at unit j * U of the tile: tiles whose width is not a
-// multiple of 8 units (G = 28: 37 tiles of H = 1024 fill all 148 SMs) are walked in groups of 4.
-template <class SA, int G, int U>
-__device__ __forceinline__ void load_gates_u(uint32_t lane_addr, int j, float (&z)[4][U]) {
-  uint32_t a[4][U], b[4][U];
-#pragma unroll
-  for (int g = 0; g < 4; ++g) {
-    if constexpr (U == 8) tmem_ld_32x8(lane_addr + SA::first(g * G + j * U), a[g]);
-    else tmem_ld_32x4(lane_addr + SA::first(g * G + j * U), a[g]);
-  }
-  if (SA::kCols != 4 * G) {
-#pragma unroll
-    for (int g = 0; g < 4; ++g) {
-      if constexpr (U == 8) tmem_ld_32x8(lane_addr + SA::second(g * G + j * U), b[g]);
-      else tmem_ld_32x4(lane_addr + SA::second(g * G + j * U), b[g]);
-    }
-    tmem_ld_wait();
-#pragma unroll
-    for (int g = 0; g < 4; ++g)
-#pragma unroll
-      for (int e = 0; e < U; ++e) z[g][e] = __uint_as_float(a[g][e]) + __uint_as_float(b[g][e]);
-  } else {
-    tmem_ld_wait();
-#pragma unroll
-    for (int g = 0; g < 4; ++g)
-#pragma unroll
-      for (int e = 0; e < U; ++e) z[g][e] = __uint_as_float(a[g][e]);
-  }
-}
-
-// Stores of U (4 or 8) new hidden values of one cell thread: see store_h8.
-template <int MODE, int U>
-__device__ __forceinline__ void store_h_u(const LstmParams& p, long long row, int b, int t, int u, const float (&hn)[U]);
-
 // Stores of one cell thread's 8 new hidden values (utterance row `row` = b*T + t, hidden units u..u+7): the recurrent
 // operand in the layer's operand format, plus the optional exact fp32 copies.
 template <int MODE>
@@ -197,36 +162,6 @@ __device__ __forceinline__ void store_h8(const LstmParams& p, long long row, int
     float* hp = p.h_last + (long long)b * p.H + u;
     *reinterpret_cast<float4*>(hp) = make_float4(hn[0], hn[1], hn[2], hn[3]);
     *reinterpret_cast<float4*>(hp + 4) = make_float4(hn[4], hn[5], hn[6], hn[7]);
-  }
-}
-
-template <int MODE, int U>
-__device__ __forceinline__ void store_h_u(const LstmParams& p, long long row, int b, int t, int u, const float (&hn)[U]) {
-  if constexpr (U == 8) {
-    store_h8<MODE>(p, row, b, t, u, hn);
-  } else {
-    static_assert(U == 4, "unit groups of 4 or 8");
-    const long long hoff = row * p.H + u;
-    if (MODE == 2) {
-      float lo[4];
-#pragma unroll
-      for (int e = 0; e < 4; ++e) lo[e] = hn[e] - __bfloat162float(__float2bfloat16_rn(hn[e]));
-      __nv_bfloat16* hp = static_cast<__nv_bfloat16*>(p.hseq) + row * (2LL * p.H) + u;
-      *reinterpret_cast<uint2*>(hp) = make_uint2(pack_bf16(hn[0], hn[1]), pack_bf16(hn[2], hn[3]));
-      *reinterpret_cast<uint2*>(hp + p.H) = make_uint2(pack_bf16(lo[0], lo[1]), pack_bf16(lo[2], lo[3]));
-    } else if (MODE == 1) {
-      *reinterpret_cast<uint2*>(static_cast<__nv_bfloat16*>(p.hseq) + hoff) =
-          make_uint2(pack_bf16(hn[0], hn[1]), pack_bf16(hn[2], hn[3]));
-    } else if (MODE == 3) {
-      *reinterpret_cast<uint2*>(static_cast<__half*>(p.hseq) + hoff) =
-          make_uint2(pack_f16(hn[0], hn[1]), pack_f16(hn[2], hn[3]));
-    } else {
-      *reinterpret_cast<float4*>(static_cast<float*>(p.hseq) + hoff) =
-          make_float4(round_tf32(hn[0]), round_tf32(hn[1]), round_tf32(hn[2]), round_tf32(hn[3]));
-    }
-    if (p.hseq_f32) *reinterpret_cast<float4*>(p.hseq_f32 + hoff) = make_float4(hn[0], hn[1], hn[2], hn[3]);
-    if (p.h_last && t == p.T - 1)
-      *reinterpret_cast<float4*>(p.h_last + (long long)b * p.H + u) = make_float4(hn[0], hn[1], hn[2], hn[3]);
   }
 }
 
@@ -582,14 +517,10 @@ __global__ void __launch_bounds__(kFusedThreads, 1) lstm_fused_kernel(const __gr
     __syncwarp();
   } else {
     // ---------------- cell warps: thread owns utterance b; the two warps of a TMEM lane quarter take alternate groups
-    // of U hidden units (8, or 4 when the tile width is not a multiple of 8 units); the running cell state stays in
-    // registers across frames.  Units past H (the ragged last tile when G does not divide H) are never stored: their
-    // weight rows and biases are zero padding.
-    constexpr int U = G % 8 == 0 ? 8 : 4;
-    constexpr int NG = G / U;
-    static_assert(G % U == 0, "tile width must be a multiple of 4 hidden units");
+    // of 8 hidden units; the running cell state stays in registers across frames.
+    constexpr int NG = G / 8;
     constexpr int NJ = (NG + kEpiWarps / 4 - 1) / (kEpiWarps / 4);
-    float cq[NJ][U];
+    float cq[NJ][8];
     uint32_t acc_phase = 0;      // bit i = parity of tmem_full[i]
     const int q = warp & 3;
     const int half = (warp - 2) >> 2;
@@ -605,11 +536,11 @@ __global__ void __launch_bounds__(kFusedThreads, 1) lstm_fused_kernel(const __gr
         for (int jj = 0; jj < NJ; ++jj) {
           const int j = half + jj * (kEpiWarps / 4);
 #pragma unroll
-          for (int e = 0; e < U; ++e) cq[jj][e] = 0.f;
-          if (valid && t > 0 && j < NG && u0 + j * U < p.H) {      // per-step launches carry c through global memory
+          for (int e = 0; e < 8; ++e) cq[jj][e] = 0.f;
+          if (valid && t > 0 && j < NG) {      // per-step launches carry c through global memory
 #pragma unroll
-            for (int e = 0; e < U; e += 4) {
-              const float4 c4 = *reinterpret_cast<const float4*>(cp + j * U + e);
+            for (int e = 0; e < 8; e += 4) {
+              const float4 c4 = *reinterpret_cast<const float4*>(cp + j * 8 + e);
               cq[jj][e] = c4.x; cq[jj][e + 1] = c4.y; cq[jj][e + 2] = c4.z; cq[jj][e + 3] = c4.w;
             }
           }
@@ -626,32 +557,32 @@ __global__ void __launch_bounds__(kFusedThreads, 1) lstm_fused_kernel(const __gr
       for (int jj = 0; jj < NJ; ++jj) {
         const int j = half + jj * (kEpiWarps / 4);
         if (j >= NG) break;
-        float acc[4][U];
-        load_gates_u<SA, G, U>(lane_addr, j, acc);
-        if (valid && u0 + j * U < p.H) {
-          float z[4][U];
+        float acc[4][8];
+        load_gates<SA, G>(lane_addr, j, acc);
+        if (valid) {
+          float z[4][8];
 #pragma unroll
           for (int g = 0; g < 4; ++g) {
 #pragma unroll
-            for (int e = 0; e < U; e += 4) {
-              const float4 x0 = *reinterpret_cast<const float4*>(sbias + g * G + j * U + e);       // broadcast reads
+            for (int e = 0; e < 8; e += 4) {
+              const float4 x0 = *reinterpret_cast<const float4*>(sbias + g * G + j * 8 + e);       // broadcast reads
               z[g][e] = acc[g][e] + x0.x;
               z[g][e + 1] = acc[g][e + 1] + x0.y;
               z[g][e + 2] = acc[g][e + 2] + x0.z;
               z[g][e + 3] = acc[g][e + 3] + x0.w;
             }
           }
-          float cn[U], hn[U];
+          float cn[8], hn[8];
 #pragma unroll
-          for (int e = 0; e < U; ++e) lstm_cell(z[0][e], z[1][e], z[2][e], z[3][e], cq[jj][e], cn[e], hn[e]);
+          for (int e = 0; e < 8; ++e) lstm_cell(z[0][e], z[1][e], z[2][e], z[3][e], cq[jj][e], cn[e], hn[e]);
 #pragma unroll
-          for (int e = 0; e < U; ++e) cq[jj][e] = cn[e];
+          for (int e = 0; e < 8; ++e) cq[jj][e] = cn[e];
           if (t + 1 == p.t_end) {       // a later launch (per-step mode) resumes from global memory
 #pragma unroll
-            for (int e = 0; e < U; e += 4)
-              *reinterpret_cast<float4*>(cp + j * U + e) = make_float4(cn[e], cn[e + 1], cn[e + 2], cn[e + 3]);
+            for (int e = 0; e < 8; e += 4)
+              *reinterpret_cast<float4*>(cp + j * 8 + e) = make_float4(cn[e], cn[e + 1], cn[e + 2], cn[e + 3]);
           }
-          store_h_u<MODE, U>(p, row, b, t, u0 + j * U, hn);
+          store_h8<MODE>(p, row, b, t, u0 + j * 8, hn);
         }
       }
       fence_proxy_async_global();   // order the h stores before later async-proxy (TMA) reads
@@ -689,42 +620,10 @@ static int run(LstmParams p, const avc_lstm_desc* d, int m_tiles, cudaStream_t s
   cfg.dynamicSmemBytes = C::kSmemBytes;
   cfg.stream = stream;
   cudaLaunchAttribute attr[2];
-  int na = 0;
-  if (CTAS > 1) {
-    attr[na].id = cudaLaunchAttributeClusterDimension;
-    attr[na].val.clusterDim.x = CTAS;
-    attr[na].val.clusterDim.y = 1;
-    attr[na].val.clusterDim.z = 1;
-    ++na;
-  }
   if (d->persistent) {
     AVC_REQUIRE(d->grid_barrier != nullptr, "avc_lstm_seq: persistent mode needs grid_barrier scratch");
-    // AVC_LSTM_NO_COOP=1 (profiling aid): launch without the cooperative attribute.  Co-residency is then only
-    // implied by the occupancy check below on an otherwise idle GPU; the bounded waits turn a violation into a trap.
-    static const bool no_coop = getenv("AVC_LSTM_NO_COOP") != nullptr;
-    if (!no_coop) {
-      attr[na].id = cudaLaunchAttributeCooperative;
-      attr[na].val.cooperative = 1;
-      ++na;
-    }
-  }
-  cfg.attrs = attr;
-  cfg.numAttrs = na;
-  if (d->persistent) {
-    int resident = 0;
-    if (CTAS > 1) {
-      int clusters = 0;
-      AVC_CHECK_CUDA(cudaOccupancyMaxActiveClusters(&clusters, kern, &cfg));
-      resident = clusters * CTAS;
-    } else {
-      int per_sm = 0;
-      AVC_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, C::kSmemBytes));
-      resident = per_sm * num_sms();
-    }
-    if (resident < grid) {   // distinct code: the caller may fall back to one launch per frame
-      set_error("avc_lstm_seq: persistent grid %d does not fit (%d CTAs resident)", grid, resident);
-      return AVC_ERR_NOT_RESIDENT;
-    }
+    const int rc = persistent_launch_config(cfg, attr, reinterpret_cast<const void*>(kern), CTAS, "avc_lstm_seq");
+    if (rc != 0) return rc;   // AVC_ERR_NOT_RESIDENT: the caller may fall back to one launch per frame
     AVC_REQUIRE((m_tiles + CTAS - 1) / CTAS <= 64, "avc_lstm_seq: at most 64 batch groups in persistent mode");
     AVC_CHECK_CUDA(cudaMemsetAsync(d->grid_barrier, 0, 64 * 32 * sizeof(unsigned int), stream));
     p.t_begin = 0;
@@ -732,6 +631,12 @@ static int run(LstmParams p, const avc_lstm_desc* d, int m_tiles, cudaStream_t s
     AVC_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
     count_launch();
   } else {
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = CTAS;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = CTAS > 1 ? 1 : 0;
     for (int t = 0; t < d->T; ++t) {
       p.t_begin = t;
       p.t_end = t + 1;
@@ -740,15 +645,6 @@ static int run(LstmParams p, const avc_lstm_desc* d, int m_tiles, cudaStream_t s
     count_launch(d->T);
   }
   return 0;
-}
-
-static int lstm_cta_group() {
-  static int v = 0;
-  if (v == 0) {
-    const char* e = getenv("AVC_LSTM_CTA_GROUP");
-    v = (e && e[0] == '1') ? 1 : 2;
-  }
-  return v;
 }
 
 // h_last[b] = hseq_f32[b][lengths[b] - 1] (a padded batch).  The recurrence kernels keep their T - 1 store: a
@@ -781,14 +677,10 @@ extern "C" int avc_lstm_seq(const avc_lstm_desc* d, void* stream_v) {
     return 0;
   }
   AVC_REQUIRE(d->dtype >= AVC_DTYPE_TF32 && d->dtype <= AVC_DTYPE_F16, "avc_lstm_seq: bad dtype %d", d->dtype);
-  AVC_REQUIRE(d->gate_group == 16 || d->gate_group == 28 || d->gate_group == 32, "avc_lstm_seq: gate_group %d (16, 28 or 32)",
-              d->gate_group);
+  AVC_REQUIRE(d->gate_group == 16 || d->gate_group == 32, "avc_lstm_seq: gate_group %d (16 or 32)", d->gate_group);
   const bool fused = d->xin != nullptr;
-  // G = 28 (37 tiles of H = 1024: two batch groups x CTA pairs fill all 148 SMs) is built for the fused kernel only; its
-  // last tile is ragged (H need not be a multiple of G: the packed weights carry zero rows for the missing units)
-  AVC_REQUIRE(d->B > 0 && d->T > 0 && d->H > 0 && d->H % 4 == 0 && (d->H % d->gate_group == 0 || d->gate_group == 28),
+  AVC_REQUIRE(d->B > 0 && d->T > 0 && d->H > 0 && d->H % 4 == 0 && d->H % d->gate_group == 0,
               "avc_lstm_seq: bad shape B=%d T=%d H=%d", d->B, d->T, d->H);
-  AVC_REQUIRE(d->gate_group != 28 || fused, "avc_lstm_seq: gate_group 28 needs the fused input projection (xin)");
   AVC_REQUIRE(d->w_hh && d->hseq && d->c_state, "avc_lstm_seq: missing buffer");
   AVC_REQUIRE(fused ? (d->w_ih && d->bias && !d->xproj) : d->xproj != nullptr,
               "avc_lstm_seq: give either xproj, or xin + w_ih + bias (fused input projection)");
@@ -799,12 +691,11 @@ extern "C" int avc_lstm_seq(const avc_lstm_desc* d, void* stream_v) {
   const bool split = d->dtype == AVC_DTYPE_BF16X3;                      // activations as [hi | lo]
   const bool w2 = split || d->dtype == AVC_DTYPE_F16;                   // weights as [w_hi | w_lo]
   const uint64_t H = (uint64_t)d->H;
-  const int n_tiles = (d->H + d->gate_group - 1) / d->gate_group;
-  const uint64_t w_rows = (uint64_t)n_tiles * bn;      // packed gate rows (4H, or more when the last tile is ragged)
+  const int n_tiles = d->H / d->gate_group;
   const uint64_t ld = split ? 2 * H : H;     // elements per row of hseq ([hi | lo] when split)
   const uint64_t ldw_hh = w2 ? 2 * H : H;    // elements per row of the packed W_hh
   const int m_tiles = (d->B + kBlockM - 1) / kBlockM;
-  const int ctas = (m_tiles >= 2 && lstm_cta_group() == 2) ? 2 : 1;
+  const int ctas = m_tiles >= 2 ? 2 : 1;
   // A small batch owned by one CTA loads only its real rows (rounded up to 8): the MMA still spans 128 rows, but the
   // rows past the batch are never stored and every accumulator row depends on its own operand row only, so whatever
   // those shared-memory rows hold is harmless -- and the stage shrinks from 32 KB to a few KB of activations.
@@ -818,7 +709,7 @@ extern "C" int avc_lstm_seq(const avc_lstm_desc* d, void* stream_v) {
     const uint64_t sh[3] = {(uint64_t)d->T * ld * es, H * es, ld * es};
     const uint32_t bh[4] = {(uint32_t)kc, (uint32_t)a_rows, parts, 1};
     if (!encode_tmap_4d(&p.tmap_h, es, d->hseq, dh, sh, bh)) return -3;
-    if (!encode_tmap_3d(&p.tmap_w, es, d->w_hh, H, w_rows, wparts, ldw_hh * es, H * es, kc, bn / ctas, wparts)) return -3;
+    if (!encode_tmap_3d(&p.tmap_w, es, d->w_hh, H, 4 * H, wparts, ldw_hh * es, H * es, kc, bn / ctas, wparts)) return -3;
   }
   if (fused) {
     // input sequence [B][T][xin_ld] holding xin_channels logical channels ([hi | lo] halves when split); channels past
@@ -833,7 +724,7 @@ extern "C" int avc_lstm_seq(const avc_lstm_desc* d, void* stream_v) {
     const uint64_t sx[3] = {(uint64_t)d->T * d->xin_ld * es, cin * es, (uint64_t)d->xin_ld * es};
     const uint32_t bx[4] = {(uint32_t)kc, (uint32_t)a_rows, parts, 1};
     if (!encode_tmap_4d(&p.tmap_xi, es, d->xin, dx, sx, bx)) return -3;
-    if (!encode_tmap_3d(&p.tmap_wi, es, d->w_ih, kpad, w_rows, wparts, ldw * es, kpad * es, kc, bn / ctas, wparts)) return -3;
+    if (!encode_tmap_3d(&p.tmap_wi, es, d->w_ih, kpad, 4 * H, wparts, ldw * es, kpad * es, kc, bn / ctas, wparts)) return -3;
     p.bias = d->bias;
   } else {
     if (!encode_tmap_3d(&p.tmap_x, 4, d->xproj, 4 * H, (uint64_t)d->T, (uint64_t)d->B, 4 * H * 4,
@@ -867,12 +758,6 @@ extern "C" int avc_lstm_seq(const avc_lstm_desc* d, void* stream_v) {
     case AVC_DTYPE_BF16: AVC_LSTM_DISPATCH2(BN_, 1)      \
     case AVC_DTYPE_F16: AVC_LSTM_DISPATCH2(BN_, 3)       \
     default: AVC_LSTM_DISPATCH2(BN_, 2)                  \
-  }
-  if (bn == 112) {      // fused kernel only, 16-bit two-term precisions, CTA pairs (the full-batch configuration it exists for)
-    AVC_REQUIRE(ctas == 2 && (d->dtype == AVC_DTYPE_F16 || d->dtype == AVC_DTYPE_BF16X3),
-                "avc_lstm_seq: gate_group 28 needs B > 128 and the fp16x2 / split precision");
-    if (d->dtype == AVC_DTYPE_F16) return run<112, 3, 2, true>(p, d, m_tiles, stream);
-    return run<112, 2, 2, true>(p, d, m_tiles, stream);
   }
   switch (bn) {
     case 64: AVC_LSTM_DISPATCH(64)

@@ -31,7 +31,6 @@
 // Warp roles: 0 = grid barrier + operand producer, 1 = MMA issuer, 2..5 (2..9 at 64 utterances) = reduction + cell
 // (warps 2, 3 store h_t).
 #include <cuda_fp16.h>
-#include <cstdlib>
 #include <cstring>
 
 #include "../../include/avc_b200.h"
@@ -418,26 +417,8 @@ static int launch_stack(const StackParams& p, const avc_lstm_stack_desc* d, cuda
   cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;
   cudaLaunchAttribute attr[2];
-  int na = 0;
-  attr[na].id = cudaLaunchAttributeClusterDimension;
-  attr[na].val.clusterDim.x = 2;
-  attr[na].val.clusterDim.y = 1;
-  attr[na].val.clusterDim.z = 1;
-  ++na;
-  static const bool no_coop = getenv("AVC_LSTM_NO_COOP") != nullptr;   // profiling aid, see avc_lstm.cu
-  if (!no_coop) {
-    attr[na].id = cudaLaunchAttributeCooperative;
-    attr[na].val.cooperative = 1;
-    ++na;
-  }
-  cfg.attrs = attr;
-  cfg.numAttrs = na;
-  int clusters = 0;
-  AVC_CHECK_CUDA(cudaOccupancyMaxActiveClusters(&clusters, kern, &cfg));
-  if (clusters * 2 < grid) {
-    set_error("avc_lstm_stack_ws: grid %d does not fit (%d CTAs resident)", grid, clusters * 2);
-    return AVC_ERR_NOT_RESIDENT;
-  }
+  const int rc = persistent_launch_config(cfg, attr, reinterpret_cast<const void*>(kern), 2, "avc_lstm_stack_ws");
+  if (rc != 0) return rc;
   AVC_CHECK_CUDA(cudaMemsetAsync(d->grid_barrier, 0, sizeof(unsigned int), stream));
   // frame 0 of every layer's sequence: the zero initial state
   const size_t frame_bytes = (size_t)d->B * d->H * 2, layer_bytes = frame_bytes * (size_t)(d->T + 1);

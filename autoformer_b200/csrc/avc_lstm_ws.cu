@@ -7,7 +7,7 @@
 //   z^T [4H x B] = W_hh [4H x H] . h_{t-1}^T [H x B]
 // W is the M-side operand and never moves: the grid is R = 4H / 128 row blocks x S K-slices, and CTA (r, s) keeps
 // W[128 r .. 128 r + 128, slice s] (hi and lo halves, <= 128 KB) on chip for the whole sequence -- in tensor memory, as
-// the A operand of tcgen05.mma (AVC_WS_W_SMEM=1: in shared memory, the first version, kept for A/B timing).  Per frame a
+// the A operand of tcgen05.mma.  Per frame a
 // CTA loads only its K-slice of h_{t-1} (B rows: a few KB), issues
 //   W_hi x [h_hi ; h_lo]   (one MMA of width N = 2 B')      and      W_lo x h_hi   (N = B')
 // into a 128 x 2B' accumulator, and the S CTAs of a row block -- one thread-block CLUSTER -- reduce their partial sums
@@ -26,7 +26,6 @@
 //
 // Warp roles: 0 = grid barrier + h_{t-1} producer, 1 = MMA issuer, 2..5 = reduction + cell (warp 2 stores h_t).
 #include <cuda_bf16.h>
-#include <cstdlib>
 
 #include "../../include/avc_b200.h"
 #include "avc_host.h"
@@ -36,11 +35,9 @@ namespace avc {
 
 constexpr int kWsThreads = 192;
 constexpr int kWsCellWarps = 4;
-constexpr int kWChunkBytes = 2 * kATileBytes;        // W_hi tile + W_lo tile of one 64-channel chunk
 
 struct alignas(64) WsParams {
-  CUtensorMap tmap_w;     // w_hh as (H, 4H, part), box {64, 128, 2}  (weights in shared memory)
-  const __nv_bfloat16* w; // w_hh [4H][2H]                            (weights in tensor memory)
+  const __nv_bfloat16* w; // w_hh [4H][2H]
   CUtensorMap tmap_h;     // hseq as (H, B, part, T), box {64, AR, 2, 1}
   const float* xproj;
   __nv_bfloat16* hseq;
@@ -64,15 +61,14 @@ struct WsCfg {
   static constexpr int kRedBytes = (kRedFrameBytes + 1023) / 1024 * 1024;
   static constexpr int kStageBytes = (AR * kUnitsOwn * 4 + 1023) / 1024 * 1024;
   static constexpr uint32_t kAccCols = 2 * AR < 32 ? 32 : 2 * AR;
-  // tensor memory: the accumulator, then (WT) this CTA's W slice as the A operand: [hi: 32 chunks columns | lo]
-  __host__ __device__ static uint32_t tmem_cols(int chunks, bool wt) {
-    uint32_t need = kAccCols + (wt ? 64u * chunks : 0u), c = 32;
+  // tensor memory: the accumulator, then this CTA's W slice as the A operand: [hi: 32 chunks columns | lo]
+  __host__ __device__ static uint32_t tmem_cols(int chunks) {
+    uint32_t need = kAccCols + 64u * chunks, c = 32;
     while (c < need) c *= 2;
     return c;
   }
-  static int smem_bytes(int chunks, bool wt, bool f16) {
-    return chunks * ((wt ? 0 : kWChunkBytes) + (f16 ? 1 : 2) * kHTile) + kRedBytes + kStageBytes + 128 +
-           1024 /* alignment slack */;
+  static int smem_bytes(int chunks, bool f16) {
+    return chunks * (f16 ? 1 : 2) * kHTile + kRedBytes + kStageBytes + 128 + 1024 /* alignment slack */;
   }
 };
 
@@ -89,18 +85,16 @@ __device__ __forceinline__ void st_async_f4(uint32_t addr, uint32_t mbar, float4
 }
 // (mbar_wait_cluster: the cluster-scope acquire wait lives in avc_ptx.cuh)
 
-// F16 ("fp16x2" precision, W in tensor memory only): h is one fp16 value per unit, the weights two fp16 terms; both
-// products W_hi x h and W_lo x h are N = AR MMAs onto the SAME accumulator columns.
-template <int AR, int S, bool WT, bool F16>
+// F16 ("fp16x2" precision): h is one fp16 value per unit, the weights two fp16 terms; both products W_hi x h and
+// W_lo x h are N = AR MMAs onto the SAME accumulator columns.
+template <int AR, int S, bool F16>
 __global__ void __launch_bounds__(kWsThreads, 1) lstm_ws_kernel(const __grid_constant__ WsParams p) {
-  static_assert(!F16 || WT, "the fp16x2 form keeps W in tensor memory");
   using Cfg = WsCfg<AR, S>;
   constexpr int HP = F16 ? 1 : 2;                    // tiles of h per 64-channel chunk (hi / lo halves)
   constexpr int NQ = AR / 4;                         // groups of 4 utterances
   extern __shared__ uint8_t smem_raw[];
   uint8_t* base = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  uint8_t* s_w = base;
-  uint8_t* s_h = s_w + (WT ? 0 : p.chunks * kWChunkBytes);
+  uint8_t* s_h = base;
   float* s_red = reinterpret_cast<float*>(s_h + p.chunks * HP * Cfg::kHTile);
   float* s_stage = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(s_red) + Cfg::kRedBytes);
   uint64_t* bars = reinterpret_cast<uint64_t*>(reinterpret_cast<uint8_t*>(s_stage) + Cfg::kStageBytes);
@@ -121,16 +115,15 @@ __global__ void __launch_bounds__(kWsThreads, 1) lstm_ws_kernel(const __grid_con
   if (clk) clk[((long long)(t_) * n_ctas + blockIdx.x) * 8 + (i_)] = clock64()
 
   if (threadIdx.x == 0) {
-    mbar_init(w_full, WT ? kWsCellWarps : 1);
+    mbar_init(w_full, kWsCellWarps);
     mbar_init(h_full, 1);
     mbar_init(d_full, 1);
     mbar_init(red_full, 1);
     mbar_init(epi_done, AR > 32 ? 2 : 1);     // one arrival per warp that stores h_t
     fence_mbar_init();
-    if (!WT) prefetch_tmap(&p.tmap_w);
     prefetch_tmap(&p.tmap_h);
   }
-  const uint32_t tmem_cols = Cfg::tmem_cols(p.chunks, WT);
+  const uint32_t tmem_cols = Cfg::tmem_cols(p.chunks);
   if (warp == 1) {
     tmem_alloc(tmem_ptr, tmem_cols);
     tmem_relinquish();
@@ -139,14 +132,9 @@ __global__ void __launch_bounds__(kWsThreads, 1) lstm_ws_kernel(const __grid_con
   cluster_sync_all();                 // peers credit bytes to this CTA's red_full: its init must be visible cluster-wide
   tc_fence_after();
   const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_ptr);
-  const uint32_t tmem_w = tmem_base + Cfg::kAccCols;        // WT: W_hi at columns [0, 32 chunks), W_lo behind it
+  const uint32_t tmem_w = tmem_base + Cfg::kAccCols;        // W_hi at columns [0, 32 chunks), W_lo behind it
 
   if (warp == 0) {
-    if (!WT && lane == 0) {
-      mbar_arrive_expect_tx(w_full, p.chunks * kWChunkBytes);
-      for (int c = 0; c < p.chunks; ++c)
-        tma_load_3d(s_w + c * kWChunkBytes, &p.tmap_w, w_full, k0 + c * 64, r * kBlockM, 0);
-    }
     if (lane == 0) {
       for (int t = 1; t < p.T; ++t) {
         // h_{t-1}: this CTA's part is stored, then every CTA's
@@ -183,7 +171,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) lstm_ws_kernel(const __grid_con
 #pragma unroll
             for (int k = 0; k < 4; ++k)
               umma_bf16_ts(tmem_base, w_lo + k * 8, umma_desc_sw128(h + k * 32), idesc16, 1u);
-          } else if (WT) {
+          } else {
             const uint32_t w_hi = tmem_w + c * 32, w_lo = w_hi + p.chunks * 32;   // 8 columns per K = 16
 #pragma unroll
             for (int k = 0; k < 4; ++k)
@@ -191,15 +179,6 @@ __global__ void __launch_bounds__(kWsThreads, 1) lstm_ws_kernel(const __grid_con
 #pragma unroll
             for (int k = 0; k < 4; ++k)
               umma_bf16_ts(tmem_base, w_lo + k * 8, umma_desc_sw128(h + k * 32), narrow, 1u);
-          } else {
-            const uint32_t w_hi = smem_u32(s_w + c * kWChunkBytes), w_lo = w_hi + kATileBytes;
-#pragma unroll
-            for (int k = 0; k < 4; ++k)
-              umma_bf16(tmem_base, umma_desc_sw128(w_hi + k * 32), umma_desc_sw128(h + k * 32), wide,
-                        (c == 0 && k == 0) ? 0u : 1u);
-#pragma unroll
-            for (int k = 0; k < 4; ++k)
-              umma_bf16(tmem_base, umma_desc_sw128(w_lo + k * 32), umma_desc_sw128(h + k * 32), narrow, 1u);
           }
         }
         umma_commit(d_full);
@@ -219,25 +198,23 @@ __global__ void __launch_bounds__(kWsThreads, 1) lstm_ws_kernel(const __grid_con
     const int slot = (row & 3) * Cfg::kUnitsOwn + (row % Cfg::kRowsOwn) / 4;
     const uint32_t push_addr = map_to_cta(smem_u32(s_red + ((int)rank * NQ * Cfg::kRowsOwn + slot) * 4), owner);
     const uint32_t owner_bar = map_to_cta(smem_u32(red_full), owner);
-    if (WT) {
-      // this thread's W row -> its TMEM lane, once: 32 bf16 (16 columns) per store, hi half then lo half
-      const uint4* src = reinterpret_cast<const uint4*>(p.w + ((long long)r * kBlockM + row) * (2LL * p.H) + k0);
-      const uint32_t lane_base = tmem_w + (static_cast<uint32_t>(q * 32) << 16);
-      for (int part = 0; part < 2; ++part)
-        for (int g = 0; g < 2 * p.chunks; ++g) {
-          uint32_t v[16];
+    // this thread's W row -> its TMEM lane, once: 32 bf16 (16 columns) per store, hi half then lo half
+    const uint4* src = reinterpret_cast<const uint4*>(p.w + ((long long)r * kBlockM + row) * (2LL * p.H) + k0);
+    const uint32_t lane_base = tmem_w + (static_cast<uint32_t>(q * 32) << 16);
+    for (int part = 0; part < 2; ++part)
+      for (int g = 0; g < 2 * p.chunks; ++g) {
+        uint32_t v[16];
 #pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            const uint4 u = __ldg(src + part * (p.H / 8) + g * 4 + i);
-            v[4 * i] = u.x; v[4 * i + 1] = u.y; v[4 * i + 2] = u.z; v[4 * i + 3] = u.w;
-          }
-          tmem_st_32x16(lane_base + part * p.chunks * 32 + g * 16, v);
+        for (int i = 0; i < 4; ++i) {
+          const uint4 u = __ldg(src + part * (p.H / 8) + g * 4 + i);
+          v[4 * i] = u.x; v[4 * i + 1] = u.y; v[4 * i + 2] = u.z; v[4 * i + 3] = u.w;
         }
-      tmem_st_wait();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(w_full);
-    }
+        tmem_st_32x16(lane_base + part * p.chunks * 32 + g * 16, v);
+      }
+    tmem_st_wait();
+    tc_fence_before();
+    __syncwarp();
+    if (lane == 0) mbar_arrive(w_full);
     float c_state[4] = {0.f, 0.f, 0.f, 0.f};
     const long long H4 = 4LL * p.H;
     for (int t = 0; t < p.T; ++t) {
@@ -350,11 +327,11 @@ __global__ void __launch_bounds__(kWsThreads, 1) lstm_ws_kernel(const __grid_con
   }
 }
 
-template <int AR, int S, bool WT, bool F16 = false>
+template <int AR, int S, bool F16>
 static int launch_ws(WsParams p, const avc_lstm_ws_desc* d, cudaStream_t stream) {
   using Cfg = WsCfg<AR, S>;
-  auto kern = lstm_ws_kernel<AR, S, WT, F16>;
-  const int smem = Cfg::smem_bytes(p.chunks, WT, F16);
+  auto kern = lstm_ws_kernel<AR, S, F16>;
+  const int smem = Cfg::smem_bytes(p.chunks, F16);
   AVC_REQUIRE(smem <= 227 * 1024, "avc_lstm_seq_ws: H=%d B=%d needs %d bytes of shared memory", d->H, d->B, smem);
   static int configured[PerDeviceOnce::kMaxDevices] = {};   // largest size set so far, per device
   int dev = 0;
@@ -372,26 +349,8 @@ static int launch_ws(WsParams p, const avc_lstm_ws_desc* d, cudaStream_t stream)
   cfg.dynamicSmemBytes = smem;
   cfg.stream = stream;
   cudaLaunchAttribute attr[2];
-  int na = 0;
-  attr[na].id = cudaLaunchAttributeClusterDimension;
-  attr[na].val.clusterDim.x = S;
-  attr[na].val.clusterDim.y = 1;
-  attr[na].val.clusterDim.z = 1;
-  ++na;
-  static const bool no_coop = getenv("AVC_LSTM_NO_COOP") != nullptr;   // profiling aid, see avc_lstm.cu
-  if (!no_coop) {
-    attr[na].id = cudaLaunchAttributeCooperative;
-    attr[na].val.cooperative = 1;
-    ++na;
-  }
-  cfg.attrs = attr;
-  cfg.numAttrs = na;
-  int clusters = 0;
-  AVC_CHECK_CUDA(cudaOccupancyMaxActiveClusters(&clusters, kern, &cfg));
-  if (clusters * S < grid) {
-    set_error("avc_lstm_seq_ws: grid %d does not fit (%d CTAs resident)", grid, clusters * S);
-    return AVC_ERR_NOT_RESIDENT;
-  }
+  const int rc = persistent_launch_config(cfg, attr, reinterpret_cast<const void*>(kern), S, "avc_lstm_seq_ws");
+  if (rc != 0) return rc;
   AVC_CHECK_CUDA(cudaMemsetAsync(d->grid_barrier, 0, sizeof(unsigned int), stream));
   AVC_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
   count_launch();
@@ -411,7 +370,7 @@ extern "C" int avc_lstm_seq_ws(const avc_lstm_ws_desc* d, void* stream_v) {
   const int ar = d->B <= 16 ? 16 : (d->B <= 32 ? 32 : 64);
   WsParams p;
   memset(&p, 0, sizeof(p));
-  if (!encode_tmap_3d(&p.tmap_w, 2, d->w_hh, H, 4 * H, 2, 2 * H * 2, H * 2, 64, kBlockM, 2)) return -3;
+  AVC_REQUIRE((reinterpret_cast<uintptr_t>(d->w_hh) & 15u) == 0, "avc_lstm_seq_ws: w_hh is not 16-byte aligned");
   AVC_REQUIRE(d->dtype == 0 || d->dtype == AVC_DTYPE_BF16X3 || d->dtype == AVC_DTYPE_F16, "avc_lstm_seq_ws: dtype %d",
               d->dtype);
   const bool f16 = d->dtype == AVC_DTYPE_F16;          // h: one fp16 per unit; else [hi | lo] bf16
@@ -420,8 +379,6 @@ extern "C" int avc_lstm_seq_ws(const avc_lstm_ws_desc* d, void* stream_v) {
   const uint64_t sh[3] = {(uint64_t)d->T * hp * H * 2, H * 2, hp * H * 2};
   const uint32_t bh[4] = {64, (uint32_t)ar, (uint32_t)hp, 1};
   if (!encode_tmap_4d(&p.tmap_h, 2, d->hseq, dh, sh, bh)) return -3;
-  // the W slice lives in tensor memory as the MMA's A operand (AVC_WS_W_SMEM=1: in shared memory, for A/B timing)
-  static const bool wt = getenv("AVC_WS_W_SMEM") == nullptr;
   p.w = static_cast<const __nv_bfloat16*>(d->w_hh);
   p.xproj = d->xproj;
   p.hseq = static_cast<__nv_bfloat16*>(d->hseq);
@@ -439,15 +396,12 @@ extern "C" int avc_lstm_seq_ws(const avc_lstm_ws_desc* d, void* stream_v) {
 #define AVC_WS_DISPATCH(S_)                                                                     \
   if (d->H % (64 * S_) == 0 && R * S_ <= num_sms()) {                                           \
     p.chunks = d->H / S_ / 64;                                                                  \
-    const int rc = f16 ? (ar == 16   ? launch_ws<16, S_, true, true>(p, d, stream)              \
-                          : ar == 32 ? launch_ws<32, S_, true, true>(p, d, stream)              \
-                                     : launch_ws<64, S_, true, true>(p, d, stream))             \
-                   : wt ? (ar == 16   ? launch_ws<16, S_, true>(p, d, stream)                   \
-                         : ar == 32 ? launch_ws<32, S_, true>(p, d, stream)                     \
-                                    : launch_ws<64, S_, true>(p, d, stream))                    \
-                      : (ar == 16   ? launch_ws<16, S_, false>(p, d, stream)                    \
-                         : ar == 32 ? launch_ws<32, S_, false>(p, d, stream)                    \
-                                    : launch_ws<64, S_, false>(p, d, stream));                  \
+    const int rc = f16 ? (ar == 16   ? launch_ws<16, S_, true>(p, d, stream)                    \
+                          : ar == 32 ? launch_ws<32, S_, true>(p, d, stream)                    \
+                                     : launch_ws<64, S_, true>(p, d, stream))                   \
+                       : (ar == 16   ? launch_ws<16, S_, false>(p, d, stream)                   \
+                          : ar == 32 ? launch_ws<32, S_, false>(p, d, stream)                   \
+                                     : launch_ws<64, S_, false>(p, d, stream));                 \
     if (rc != AVC_ERR_NOT_RESIDENT) return rc;                                                  \
   }
   AVC_WS_DISPATCH(8)

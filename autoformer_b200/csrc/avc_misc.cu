@@ -1,8 +1,6 @@
 // HBM-bound glue and the small-H bidirectional LSTM (see include/avc_b200.h).
 #include <cuda_bf16.h>
 
-#include <cstdlib>
-
 #include "../../include/avc_b200.h"
 #include "avc_host.h"
 #include "avc_pipe.cuh"
@@ -497,8 +495,7 @@ extern "C" int avc_bilstm_small(const float* xproj, const float* w_hh, void* out
   const int grid = (B + kSmallWarps / 2 - 1) / (kSmallWarps / 2);
   // four lanes per unit: a 2.9x shorter dependent chain per step, four times the warps.  Measured (T = 1024 / 128, two
   // layers): B = 1 1.15 -> 0.78 ms, B = 32 1.47 -> 0.79 ms, but B = 512 0.21 -> 0.24 ms (issue-bound there): small batches only
-  static const bool lanes4 = getenv("AVC_BILSTM_WARP") == nullptr;   // AVC_BILSTM_WARP=1: the warp-per-direction kernel (A/B timing)
-  if (H == 32 && lanes4 && B <= 128) {
+  if (H == 32 && B <= 128) {
     bilstm32_kernel<<<2 * B, 128, 0, stream>>>(xproj, w_hh, out, out_dtype, out_round_tf32, codes, T, freq, lengths);
   } else if (H == 32) {   // AutoVC "A" (dim_neck = 32): recurrent weights in registers
     auto kern = bilstm_small_kernel<1, true>;

@@ -179,13 +179,6 @@ __device__ __forceinline__ void tmem_ld_32x8(uint32_t taddr, uint32_t (&v)[8]) {
       : "r"(taddr)
       : "memory");
 }
-// 32 lanes x 4 consecutive fp32 columns.
-__device__ __forceinline__ void tmem_ld_32x4(uint32_t taddr, uint32_t (&v)[4]) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];"
-               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3])
-               : "r"(taddr)
-               : "memory");
-}
 // 32 lanes x 16 consecutive 32-bit columns from registers: thread i of the warp writes row (lane base + i).
 __device__ __forceinline__ void tmem_st_32x16(uint32_t taddr, const uint32_t (&v)[16]) {
   asm volatile(

@@ -25,7 +25,7 @@ class LstmDV(layers.PlanOwner, nn.Module):
         self.num_layers, self.dim_cell = num_layers, dim_cell
         self.precision = "fp32"
         self.persistent_lstm = True
-        self.wavefront = None           # None: the library default (on; AVC_LSTM_STACK=0 turns it off)
+        self.wavefront = None           # None: the library default (on, layers.LstmStack)
         self._cache = layers.PlanCache()
 
     def _build_plan(self):

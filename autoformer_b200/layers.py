@@ -1,6 +1,4 @@
 """Packed layer objects shared by the drop-in models: they own folded/re-packed weights and call ``ops``."""
-import os
-
 import torch
 import torch.nn as nn
 
@@ -222,23 +220,9 @@ def _lengths_kw(lengths):
     return {} if lengths is None else {"lengths": lengths}
 
 
-def lstm_ws_default():
-    """AVC_LSTM_WS=0 keeps small batches on the batched recurrence kernel (A/B timing)."""
-    return os.environ.get("AVC_LSTM_WS", "1") != "0"
-
-
-def gate28_default():
-    """AVC_LSTM_G28=1 selects 28-unit gate tiles where they fill more SMs (H = 1024, B = 512: 37 x 4 = 148 CTAs instead
-    of 128).  Built, parity-tested (bit-identical outputs) and MEASURED SLOWER on the bench configuration -- LSTM layers
-    4.30 ms against 4.14 ms per step (gpurun r02i): the frame is bound by its serial shadow (barrier among more CTAs, cell
-    update in groups of 4 units, 15 % more h-tile loads out of L2), not by the MMAs the extra SMs would shorten -- so
-    the default stays 32."""
-    return os.environ.get("AVC_LSTM_G28", "0") == "1"
-
-
 def lstm_fused_default():
-    """AVC_LSTM_FUSED=0 selects the two-kernel form (dense input projection, then the recurrence) for A/B timing."""
-    return os.environ.get("AVC_LSTM_FUSED", "1") != "0"
+    """LstmLayer's default for `fused`.  Kept as a function because bench.py imports it to name the roofline kernel."""
+    return True
 
 
 class LstmLayer:
@@ -246,13 +230,13 @@ class LstmLayer:
     fused into that kernel (its MMAs fill the tensor pipe while the cell update and the grid barrier of the previous
     frame are in flight); `fused=False` runs it as one dense GEMM per layer in front of the recurrence."""
 
-    def __init__(self, w_ih, w_hh, b_ih, b_hh, precision, fused=None):
+    def __init__(self, w_ih, w_hh, b_ih, b_hh, precision, fused=True):
         self.w_ih, self.w_hh, self.b_ih, self.b_hh = w_ih.detach(), w_hh.detach(), b_ih.detach(), b_hh.detach()
         self.precision = precision
         self.H = w_hh.shape[1]
         self.C_in = w_ih.shape[1]
-        self.fused = lstm_fused_default() if fused is None else fused
-        self.ws = lstm_ws_default()
+        self.fused = fused
+        self.ws = True
         self._packs = {}
         self._fused_packs = {}
 
@@ -300,7 +284,7 @@ class LstmLayer:
                      **_lengths_kw(lengths[b0:b1] if lengths is not None else None))
             return out
         if persistent and self.ws and ops.ws_supported(B, self.H, self.precision):
-            # small batch: dense input projection, then the recurrence with W_hh resident in shared memory
+            # small batch: dense input projection, then the recurrence with W_hh resident in tensor memory
             ih, hh = self.packs(packing.WS_GROUP)
             xp = torch.empty(B * T, 4 * self.H, dtype=torch.float32, device=x.device)
             ih(x, B, T, out2=xp)
@@ -310,7 +294,7 @@ class LstmLayer:
                 return out
             self.ws = False             # the device cannot hold the grid: batched kernel from now on
         fused = self.use_fused(B)
-        group = ops.choose_gate_group(B, self.H, persistent, fused=fused and gate28_default(), precision=self.precision)
+        group = ops.choose_gate_group(B, self.H, persistent)
         if fused:
             wih, bias, hh = self.fused_packs(group)
             return ops.lstm_seq(None, hh, B, T, self.H, self.precision, group, hseq=hseq, hseq_f32=hseq_f32,
@@ -328,11 +312,6 @@ def lstm_layers(sd, prefix, num_layers, precision):
                       sd[f"{prefix}.bias_hh_l{l}"], precision) for l in range(num_layers)]
 
 
-def lstm_stack_default():
-    """AVC_LSTM_STACK=0 keeps small-batch stacks on the layer-by-layer kernels (A/B timing)."""
-    return os.environ.get("AVC_LSTM_STACK", "1") != "0"
-
-
 class LstmStack:
     """nn.LSTM(num_layers = L) of which only the top layer's last frame is used (LstmDV.py:20-21, Adjust.py:40-41).
 
@@ -346,7 +325,7 @@ class LstmStack:
         self.layers = layers_
         self.precision = precision
         self.H = layers_[0].H
-        self.wavefront = lstm_stack_default() if wavefront is None else wavefront
+        self.wavefront = True if wavefront is None else wavefront
         self._packs = None
 
     def packs(self):

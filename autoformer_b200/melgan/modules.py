@@ -14,7 +14,6 @@ The module tree only HOLDS parameters under the reference's state_dict names (``
                                        intermediate in shared memory and the weights resident
   LeakyReLU + ReflectionPad1d(3) + WNConv1d(32 -> 1, k7) + Tanh -> avc_conv_to_mono_tanh
 """
-import os
 
 import numpy as np
 import torch
@@ -235,10 +234,8 @@ class Generator(layers.PlanOwner, nn.Module):
         self.precision = "fp32"
         self.collect_taps = False
         self.taps = {}
-        # AVC_MELGAN_FUSED=0 (profiling aid): run every ResnetBlock as two avc_conv_gemm launches
-        self.fuse_resblocks = os.environ.get("AVC_MELGAN_FUSED", "1") != "0"
-        # AVC_MELGAN_FUSED_OUT=0 (A/B timing): the output convolution as its own pass (avc_conv_to_mono_tanh)
-        self.fuse_output_conv = os.environ.get("AVC_MELGAN_FUSED_OUT", "1") != "0"
+        # False: every ResnetBlock as two avc_conv_gemm launches (the unfused reference path)
+        self.fuse_resblocks = True
         self._cache = layers.PlanCache()
 
     def _plan(self):
@@ -304,7 +301,7 @@ class Generator(layers.PlanOwner, nn.Module):
                         fused(xs, B, Lr, y=cur, y_act=True, **block_kw)                  # + the next model.{i} LeakyReLU
                         if taps is not None:
                             taps[f"stage{si}"] = _inv_lrelu(packing.act_to_float(cur, P))
-                    elif taps is None and self.fuse_output_conv and C == 32:
+                    elif taps is None and C == 32:
                         # model.22-25 (LeakyReLU, ReflectionPad1d(3), Conv1d(32 -> 1, k7), tanh) in the block's epilogue:
                         # the block's output (1 GB at B = 32) is neither written nor re-read.  A padded batch skips the
                         # tiles past each utterance's end, so their samples come from the zero fill.

@@ -331,11 +331,8 @@ def persistent_batch_cap(H, n_sm=148):
     return best
 
 
-def choose_gate_group(B, H, persistent=False, n_sm=148, fused=False, precision=None):
-    """Hidden units per accumulator tile (tile width 4G): fill the SMs without exceeding one wave when persistent.
-
-    G = 28 (the fused kernel, two-term 16-bit precisions, CTA pairs): ceil(H / 28) tiles with a ragged last one -- for
-    H = 1024 and two batch groups that is 37 x 4 = 148 CTAs, every SM of a B200, where G = 32 leaves 20 idle."""
+def choose_gate_group(B, H, persistent=False, n_sm=148):
+    """Hidden units per accumulator tile (tile width 4G): fill the SMs without exceeding one wave when persistent."""
     if LSTM_CTA_BUDGET is not None:                # two batches side by side on two streams: each takes half the SMs
         n_sm = min(n_sm, LSTM_CTA_BUDGET)
     m_tiles = (B + 127) // 128
@@ -354,10 +351,6 @@ def choose_gate_group(B, H, persistent=False, n_sm=148, fused=False, precision=N
             if H % g == 0 and (not persistent or m_tiles * (H // g) <= n_sm):
                 choice = g
                 break
-    if fused and m_tiles >= 2 and precision in packing.TWO_TERM_WEIGHTS and H % 64 == 0:
-        ctas28 = m_tiles * ((H + 27) // 28)
-        if ctas28 <= n_sm and (choice is None or ctas28 > m_tiles * (H // choice)):
-            choice = 28
     if choice is not None:
         return choice
     raise RuntimeError(f"no gate group fits B={B} H={H} persistent={persistent}")
@@ -381,15 +374,14 @@ def lstm_seq(xproj, w_hh, B, T, H, precision, group, hseq=None, hseq_f32=None, h
         assert xin.shape[2] >= packing.act_channels(c_in, precision) and xin.stride(2) == 1
         assert xin.stride(0) == T * xin.stride(1) and c_in % 8 == 0
         assert w_ih.dtype == TORCH_DTYPE[precision] and w_ih.is_contiguous()
-        rows = (H + group - 1) // group * 4 * group      # 4H, or more when the last gate tile is ragged (G = 28)
-        assert w_ih.shape == (rows, 2 * kp if precision in packing.TWO_TERM_WEIGHTS else kp), (w_ih.shape, kp)
-        assert bias.dtype == torch.float32 and bias.is_contiguous() and bias.numel() == rows
+        assert w_ih.shape == (4 * H, 2 * kp if precision in packing.TWO_TERM_WEIGHTS else kp), (w_ih.shape, kp)
+        assert bias.dtype == torch.float32 and bias.is_contiguous() and bias.numel() == 4 * H
         _require_cuda(w_ih, bias)
     else:
         assert xproj.dtype == torch.float32 and xproj.is_contiguous() and xproj.numel() == B * T * 4 * H
     wk = 2 * H if precision in packing.TWO_TERM_WEIGHTS else H
     assert w_hh.dtype == TORCH_DTYPE[precision] and w_hh.is_contiguous()
-    assert w_hh.shape == ((H + group - 1) // group * 4 * group, wk), (w_hh.shape, H, group)
+    assert w_hh.shape == (4 * H, wk), (w_hh.shape, H, group)
     if hseq is None:
         hseq = alloc_act(B, T, H, precision, dev)
     assert hseq.is_contiguous() and hseq.shape == (B, T, packing.act_channels(H, precision))
@@ -460,7 +452,7 @@ def ws_supported(B, H, precision, n_sm=148):
 
 def lstm_seq_ws(xproj, w_hh, B, T, H, hseq=None, hseq_f32=None, h_last=None, debug_clk=None, precision="fp32",
                 lengths=None):
-    """Small-batch recurrence with W_hh resident in shared memory (split precision).  xproj [B*T][4H] fp32 and w_hh
+    """Small-batch recurrence with W_hh resident in tensor memory (split precision).  xproj [B*T][4H] fp32 and w_hh
     [4H][2H] bf16 in the packing.WS_GROUP gate order.  Returns hseq, or None when the device cannot hold the grid
     (nothing was launched; the caller uses lstm_seq).  lengths: optional device int32 [B], h_last[b] = h at frame
     lengths[b] - 1."""

@@ -256,36 +256,22 @@ WS_GROUP = "ws"     # gate packing of the weight-stationary small-batch recurren
 
 def gate_permutation(hidden: int, group, device=None) -> torch.Tensor:
     """index[p] = PyTorch gate row (g*H + u) stored at packed position p = (u//G)*4G + g*G + u%G; for
-    group == WS_GROUP the four gates of a unit are adjacent: p = 128 (u//32) + 4 (u%32) + g.
-
-    When G does not divide H (G = 28: 37 tiles of H = 1024 fill the 148 SMs) the last tile is ragged: there are
-    ceil(H/G) * 4G packed positions and those of the missing units hold -1 (``take_rows`` turns them into zero rows)."""
+    group == WS_GROUP the four gates of a unit are adjacent: p = 128 (u//32) + 4 (u%32) + g."""
+    p = torch.arange(4 * hidden, device=device)
     if group == WS_GROUP:
-        p = torch.arange(4 * hidden, device=device)
         assert hidden % 32 == 0
         return (p % 4) * hidden + (p // 128) * 32 + (p % 128) // 4
-    tiles = (hidden + group - 1) // group
-    p = torch.arange(tiles * 4 * group, device=device)
+    assert hidden % group == 0
     blk = p // (4 * group)
     g = (p % (4 * group)) // group
-    u = blk * group + p % group
-    return torch.where(u < hidden, g * hidden + u, torch.full_like(u, -1))
-
-
-def take_rows(t: torch.Tensor, perm: torch.Tensor) -> torch.Tensor:
-    """t[perm] with zero rows where perm is -1 (the padding units of a ragged last gate tile)."""
-    out = t[perm.clamp(min=0)]
-    if bool((perm < 0).any()):
-        out = out.clone()
-        out[perm < 0] = 0
-    return out
+    return g * hidden + blk * group + p % group
 
 
 def pack_lstm_ih(w_ih, b_ih, b_hh, precision, group):
     """Input projection of one uni-directional layer with gate-interleaved output columns."""
     h = w_ih.shape[0] // 4
     perm = gate_permutation(h, group, w_ih.device)
-    return pack_linear(take_rows(w_ih, perm), take_rows(b_ih + b_hh, perm), precision)
+    return pack_linear(w_ih[perm], (b_ih + b_hh)[perm], precision)
 
 
 def pack_lstm_ih_fused(w_ih, b_ih, b_hh, precision, group):
@@ -295,8 +281,8 @@ def pack_lstm_ih_fused(w_ih, b_ih, b_hh, precision, group):
     perm = gate_permutation(h, group, w_ih.device)
     kpad = _ceil_to(c_in, KC[precision])
     w = torch.zeros(perm.numel(), kpad, dtype=torch.float32, device=w_ih.device)
-    w[:, :c_in] = take_rows(w_ih.float(), perm)
-    bias = take_rows(b_ih.float() + b_hh.float(), perm).contiguous()
+    w[:, :c_in] = w_ih.float()[perm]
+    bias = (b_ih.float() + b_hh.float())[perm].contiguous()
     if precision in TWO_TERM_WEIGHTS:
         hi, lo = split_terms(w, precision)
         return torch.cat([hi, lo], dim=1).contiguous(), bias
@@ -306,7 +292,7 @@ def pack_lstm_ih_fused(w_ih, b_ih, b_hh, precision, group):
 def pack_lstm_hh(w_hh, precision, group):
     h = w_hh.shape[1]
     perm = gate_permutation(h, group, w_hh.device)
-    w = take_rows(w_hh.float(), perm)
+    w = w_hh.float()[perm]
     if precision in TWO_TERM_WEIGHTS:
         hi, lo = split_terms(w, precision)
         # [w_hi | w_lo]; "fp32": the kernel forms a_hi*w_hi + a_lo*w_hi + a_hi*w_lo, "fp16x2": a*w_hi + a*w_lo
@@ -320,11 +306,11 @@ def pack_lstm_stack(w_ih, w_hh, b_ih, b_hh, first):
     bias go through the dense projection in front (pack_lstm_ih) and are None here."""
     h = w_hh.shape[1]
     perm = gate_permutation(h, WS_GROUP, w_hh.device)
-    one = lambda w: sat_f16(take_rows(w.float(), perm)).to(torch.float16).contiguous()
+    one = lambda w: sat_f16(w.float()[perm]).to(torch.float16).contiguous()
     if first:
         return None, one(w_hh), None
     assert w_ih.shape == (4 * h, h), "the layers above the first take the hidden sequence of the layer below"
-    return one(w_ih), one(w_hh), take_rows(b_ih.float() + b_hh.float(), perm).contiguous()
+    return one(w_ih), one(w_hh), (b_ih.float() + b_hh.float())[perm].contiguous()
 
 
 def pack_bilstm_ih(w_ih_f, b_ih_f, b_hh_f, w_ih_r, b_ih_r, b_hh_r, precision):

@@ -266,7 +266,7 @@ int avc_lstm_seq(const avc_lstm_desc* d, void* stream);
 
 /*
  * Small-batch form of the same recurrence (B <= 64, split-bf16 or fp16x2 precision): the recurrent weights stay in
- * shared memory for the whole sequence (4H/128 row blocks x S K-slices, one thread-block cluster per row block
+ * tensor memory for the whole sequence (4H/128 row blocks x S K-slices, one thread-block cluster per row block
  * reducing its partial sums through distributed shared memory), so a frame moves only h_{t-1}.
  * Same semantics and references as avc_lstm_seq (factory/AutoVC.py:77,96,103,110; factory/LstmDV.py:12,20).
  * Gate rows of w_hh and columns of xproj are packed  p = 128 (u / 32) + 4 (u % 32) + gate.

@@ -64,7 +64,7 @@ def build(what):
     if what == "misc":
         # the small kernels no other workload launches: gn_apply (MetaConv), global_stats / adain (AdaIN "2" variants),
         # audio_frames / complex_mag (Audio2Mel), resblock_kernel (MelGAN in the split format), lstm_step_kernel
-        # (un-fused input projection, one launch per frame)
+        # (un-fused input projection, one launch per frame: LstmLayer.use_fused picks it for the decoder's lstm2 at B = 8)
         from autoformer_b200.factory.AutoVC import AutoVC
         from autoformer_b200.factory.AutoVC2 import AutoVC2
         from autoformer_b200.factory.MetaConv import MetaConv
@@ -82,7 +82,6 @@ def build(what):
         av.load_state_dict(seeded_state_dict(templates.autovc_template(*args), 0))
         av = av.cuda().eval()
         av.persistent_lstm = False
-        os.environ["AVC_LSTM_FUSED"] = "0"
         xa, coa, cta = synthetic_mel(64, 64, 1).cuda(), synthetic_speaker(64, 1, "org").cuda(), synthetic_speaker(64, 1, "trg").cuda()
         fft = Audio2Mel().cuda()
         audio = torch.randn(8, 22050, device="cuda") * 0.1

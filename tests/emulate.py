@@ -128,8 +128,7 @@ def _emu_lstm_seq(xproj, w_hh, B, T, H, precision, group, hseq=None, hseq_f32=No
         assert xproj is None
         kc = KC[precision]
         kp = (c_in + kc - 1) // kc * kc
-        rows = (H + group - 1) // group * 4 * group          # ragged last gate tile when G does not divide H
-        assert w_ih.shape == (rows, 2 * kp if two else kp) and bias.shape == (rows,) and w_hh.shape[0] == rows
+        assert w_ih.shape == (4 * H, 2 * kp if two else kp) and bias.shape == (4 * H,) and w_hh.shape[0] == 4 * H
         wi = (w_ih[:, :kp].double() + w_ih[:, kp:].double()) if two else w_ih.double()
         assert float(wi[:, c_in:].abs().max()) == 0.0 if kp > c_in else True
         assert xin.shape[:2] == (B, T) and xin.dtype == packing.TORCH_DTYPE[precision]

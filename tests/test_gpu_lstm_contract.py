@@ -4,8 +4,7 @@ Every kernel reads h_{t-1} back from a buffer the test can see (avc_lstm_seq and
 hseq; avc_lstm_stack_ws: hs[l][t] and hs[l-1][t+1]; avc_bilstm_small: the exact fp32 h, visible when `out` is fp32 and
 unrounded).  So the reference does not free-run: for every frame it recomputes the pre-activations in fp64 from the
 kernel's own stored h_{t-1}, with exactly the products the kernel forms, from the RAW PyTorch-layout weights split with
-packing.split_terms / sat_f16 (never from the packed tensors, so a gate-permutation or ragged-tile packing error fails
-too):
+packing.split_terms / sat_f16 (never from the packed tensors, so a gate-permutation packing error fails too):
     split bf16 ("fp32")  a_hi w_hi + a_lo w_hi + a_hi w_lo      (the kernel drops lo * lo)
     "fp16x2"             a w_hi + a w_lo
     "bf16", "tf32"       a w on the stored operands
@@ -22,12 +21,12 @@ The cell state is not exported: c is chained in fp64 from the teacher-forced gat
   * bit-exact stores (operand hseq = packing.to_act(hseq_f32), h_last = the last frame, stack frame 0 = 0, BiLSTM
     output formats and codes against the unrounded fp32 run);
   * NaN sentinels around every output (spare utterances, a spare layer, NaN channels past the input's logical ones);
-  * bit identity of per-step and persistent launches, of a repeated launch, and of G = 28 and G = 32 tiles.
+  * bit identity of per-step and persistent launches and of a repeated launch.
 The CPU tests check the declared cases against mirrors of the host dispatch, and check the checker itself on the
 tests/emulate.py stand-ins, with and without injected faults.
 
-Not covered, on purpose: the A/B-timing environment switches AVC_LSTM_CTA_GROUP=1, AVC_WS_W_SMEM=1, AVC_BILSTM_WARP=1
-and AVC_LSTM_NO_COOP.  They are read once per process and are not production paths.
+Not covered, on purpose: AVC_LSTM_NO_COOP (a profiling aid that launches the same persistent kernels without the
+cooperative attribute).  It is read once per process.
 """
 import itertools
 import zlib
@@ -57,16 +56,13 @@ def _nan(shape, dtype, dev):
 
 # ------------------------------------------------------------------------------------------------ dispatch mirrors
 def seq_cell(B, H, prec, group, fused):
-    """Mirror of avc_lstm_seq's host dispatch (avc_lstm.cu:756-857): (kernel, MODE, BN, geometry, a_rows < 128)."""
+    """Mirror of avc_lstm_seq's host dispatch (avc_lstm.cu:663-769): (kernel, MODE, BN, geometry, a_rows < 128)."""
     from autoformer_b200 import packing
-    assert group in (16, 28, 32)
+    assert group in (16, 32)
     kc = packing.KC[prec]
-    assert H % kc == 0 and H % 4 == 0 and (H % group == 0 or group == 28)
+    assert H % kc == 0 and H % 4 == 0 and H % group == 0
     m_tiles = -(-B // 128)
-    ctas = 2 if m_tiles >= 2 else 1
     a_rows = -(-B // 8) * 8 if m_tiles == 1 else 128
-    if group == 28:                                             # fused only, two-term precisions, CTA pairs
-        assert fused and ctas == 2 and prec in packing.TWO_TERM_WEIGHTS
     geo = "single" if m_tiles == 1 else ("phantom" if m_tiles % 2 else "pair")
     return ("fused" if fused else "step", MODE[prec], 4 * group, geo, a_rows < 128)
 
@@ -104,9 +100,6 @@ def _declare_seq():
                                                                    ("single", "pair", "phantom"))):
         cases.append(dict(kern=kern, prec=prec, group=group, B=SEQ_B[geo], H=128, T=(5, 1, 2, 7)[i % 4],
                           c_in=(72, 40, 104)[i % 3]))
-    # G = 28: ragged last tiles (H = 768: 12 live units of 28, H = 1024: 16)
-    for i, (prec, H) in enumerate(itertools.product(("fp32", "fp16x2"), (768, 1024))):
-        cases.append(dict(kern="fused", prec=prec, group=28, B=(300, 256)[i % 2], H=H, T=(3, 2)[i % 2], c_in=72))
     return cases
 
 
@@ -153,9 +146,6 @@ def test_lstm_case_matrix_covers_every_cell():
             for g in ("single", "pair", "phantom")}
     assert need <= {c[:4] for c in cells}, sorted(need - {c[:4] for c in cells})
     assert all(c[4] == (c[3] == "single") for c in cells)                  # one m-tile loads only its rows
-    g28 = {(c[1], c[3]) for c in cells if c[2] == 112}
-    assert {MODE["fp32"], MODE["fp16x2"]} == {m for m, _ in g28} and {"pair", "phantom"} == {g for _, g in g28}
-    assert {c["H"] - (c["H"] // 28) * 28 for c in SEQ_CASES if c["group"] == 28} == {12, 16}   # live units, last tile
     assert {1, 2} <= {c["T"] for c in SEQ_CASES}
     for p in PRECS:                   # an input width that is not a whole number of k-blocks, in every precision
         assert any(c["c_in"] % packing.KC[p] for c in SEQ_CASES if c["prec"] == p and c["kern"] == "fused")
@@ -185,7 +175,7 @@ def test_lstm_case_matrix_covers_every_cell():
     # production shapes reach the kernels the tests below launch them on
     for B in (512, 300):
         for H in (512, 1024):
-            assert ops.choose_gate_group(B, H, True, fused=False, precision="fp16x2") == {512: 16, 1024: 32}[H]
+            assert ops.choose_gate_group(B, H, True) == {512: 16, 1024: 32}[H]
     assert seq_cell(512, 1024, "fp16x2", 32, True)[3] == "pair" and seq_cell(300, 1024, "fp16x2", 32, True)[3] == "phantom"
     assert ops.persistent_batch_cap(512) >= 512 and ops.persistent_batch_cap(1024) >= 512
     assert ops.stack_supported(32, 768, 3, "fp16x2") and ops.stack_supported(8, 768, 3, "fp16x2")
@@ -386,8 +376,8 @@ def seq_nadd(prec, H, kx, extra=3):
 
 
 def run_seq_case(c, dev, lstm_seq=None, seed=None):
-    """Launch one declared avc_lstm_seq case per-step and persistent (plus a repeat and, for G = 28, G = 32) and check
-    every launch.  Returns the persistent SeqRun."""
+    """Launch one declared avc_lstm_seq case per-step and persistent (plus a repeat) and check every launch.  Returns
+    the persistent SeqRun."""
     from autoformer_b200 import _lib, ops, packing
     lstm_seq = lstm_seq or ops.lstm_seq
     seed = zlib.crc32(_seq_id(c).encode()) % 10007 if seed is None else seed
@@ -401,23 +391,21 @@ def run_seq_case(c, dev, lstm_seq=None, seed=None):
     else:
         xproj = make_xproj(B, T, 4 * H, seed + 1, "cpu")
     runs = {}
-    groups = (G, 32) if G == 28 else (G,)
-    for group in groups:
-        perm = packing.gate_permutation(H, group)
-        hh = packing.pack_lstm_hh(w_hh, prec, group).to(dev)
-        for persistent in (False, True, True):
-            r = SeqRun(B, T, H, prec, dev)
-            kw = dict(hseq=r.hseq, hseq_f32=r.hseq_f32, h_last=r.h_last, persistent=persistent)
-            n0 = _lib.launch_count() if dev == "cuda" else 0
-            if fused:
-                wih, bias = packing.pack_lstm_ih_fused(w_ih, b_ih, b_hh, prec, group)
-                lstm_seq(None, hh, B, T, H, prec, group, xin=xin, w_ih=wih.to(dev), bias=bias.to(dev), c_in=c_in, **kw)
-            else:
-                lstm_seq(xproj[..., perm].contiguous().view(B * T, 4 * H).to(dev), hh, B, T, H, prec, group, **kw)
-            if dev == "cuda":
-                torch.cuda.synchronize()
-                assert _lib.launch_count() - n0 == (1 if persistent else T), "persistent grid fell back to per-step"
-            runs.setdefault((group, persistent), []).append(r)
+    perm = packing.gate_permutation(H, G)
+    hh = packing.pack_lstm_hh(w_hh, prec, G).to(dev)
+    for persistent in (False, True, True):
+        r = SeqRun(B, T, H, prec, dev)
+        kw = dict(hseq=r.hseq, hseq_f32=r.hseq_f32, h_last=r.h_last, persistent=persistent)
+        n0 = _lib.launch_count() if dev == "cuda" else 0
+        if fused:
+            wih, bias = packing.pack_lstm_ih_fused(w_ih, b_ih, b_hh, prec, G)
+            lstm_seq(None, hh, B, T, H, prec, G, xin=xin, w_ih=wih.to(dev), bias=bias.to(dev), c_in=c_in, **kw)
+        else:
+            lstm_seq(xproj[..., perm].contiguous().view(B * T, 4 * H).to(dev), hh, B, T, H, prec, G, **kw)
+        if dev == "cuda":
+            torch.cuda.synchronize()
+            assert _lib.launch_count() - n0 == (1 if persistent else T), "persistent grid fell back to per-step"
+        runs.setdefault(persistent, []).append(r)
     what = _seq_id(c)
     if fused:
         base, x_pairs = fused_base_and_pairs(xin, w_ih.to(dev), b_ih.to(dev), b_hh.to(dev), prec, c_in)
@@ -425,13 +413,13 @@ def run_seq_case(c, dev, lstm_seq=None, seed=None):
     else:
         base, x_pairs, nadd = xproj.double().to(dev), [], seq_nadd(prec, H, 0)
     key = f"lstm_seq/{prec}"
-    main = runs[(G, True)][0]
+    main = runs[True][0]
     main.check(base, x_pairs, w_hh.to(dev), nadd, what + " persistent", key)
-    runs[(G, False)][0].check(base, x_pairs, w_hh.to(dev), nadd, what + " per-step", key)
+    runs[False][0].check(base, x_pairs, w_hh.to(dev), nadd, what + " per-step", key)
     ref_bits = _bits(main.hseq_f32)
-    for (group, persistent), rs in runs.items():
+    for persistent, rs in runs.items():
         for r in rs:
-            assert torch.equal(_bits(r.hseq_f32), ref_bits), f"{what}: G={group} persistent={persistent} differs in bits"
+            assert torch.equal(_bits(r.hseq_f32), ref_bits), f"{what}: persistent={persistent} differs in bits"
             assert torch.equal(_bits(r.hseq), _bits(main.hseq))
     return main
 
@@ -682,7 +670,7 @@ def _expect_fail(fn, *needles):
 
 
 SELF_SEQ = [dict(kern="step", prec="fp32", group=16, B=5, H=64, T=4, c_in=40),
-            dict(kern="fused", prec="fp16x2", group=28, B=130, H=128, T=3, c_in=40),
+            dict(kern="fused", prec="fp16x2", group=32, B=130, H=128, T=3, c_in=40),
             dict(kern="fused", prec="bf16", group=32, B=3, H=64, T=3, c_in=24),
             dict(kern="step", prec="tf32", group=16, B=4, H=32, T=2, c_in=40)]
 
