@@ -213,47 +213,77 @@ __global__ void __launch_bounds__(256) patchify_kernel(const float* __restrict__
 }
 
 // ---------------------------------------------------------------- LayerNorm statistics along rows / columns
-// rows: one warp per row of C entries;  cols: one thread per column, looping over R rows (coalesced across threads)
+// Moments as (count n, mean m, M2 = sum of squared deviations): Welford's update per element, Chan's formula to merge
+// two partial sets.  The variance is never formed as E[x^2] - mean^2, which cancels in fp32 once |mean| is large next
+// to the standard deviation (at |mean| / std = 1000 the normalised values were off by ~0.4); with centred sums the error
+// grows only linearly in |mean| / std, with the length of the longest Welford chain plus the merge depth.
+struct Moments {
+  float n, m, M2;
+};
+
+// 1/n does not depend on the data, so it stays off the dependency chain through m; the approximate reciprocal (2 ulp)
+// is well inside the error bound tests/test_gpu_meta_contract.py holds the statistics to
+__device__ __forceinline__ void welford_add(Moments& a, float v) {
+  a.n += 1.0f;
+  const float inv_n = __fdividef(1.0f, a.n);
+  const float d = v - a.m;
+  a.m = fmaf(d, inv_n, a.m);
+  a.M2 = fmaf(d, v - a.m, a.M2);
+}
+
+__device__ __forceinline__ Moments chan_merge(Moments a, Moments b) {
+  const float n = a.n + b.n;
+  if (n == 0.0f) return a;
+  const float d = b.m - a.m, wb = __fdividef(b.n, n);
+  return {n, fmaf(d, wb, a.m), a.M2 + b.M2 + d * d * (a.n * wb)};
+}
+
+// rows: one warp per row of C entries, lane l takes entries l, l + 32, ... (chains of ceil(C / 32)), then five merge
+// levels across the warp.  Writes (mean, rstd) at stats[2 * row].
 __global__ void __launch_bounds__(256) ln_row_stats_kernel(const float* __restrict__ x, float* __restrict__ stats,
                                                            long long rows, int C, float eps) {
   const long long row = blockIdx.x * (long long)(blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= rows) return;
   const int lane = threadIdx.x & 31;
   const float* xr = x + row * C;
-  float s = 0.f, ss = 0.f;
-  for (int c = lane; c < C; c += 32) {
-    const float v = __ldg(xr + c);
-    s += v;
-    ss += v * v;
-  }
+  Moments a = {0.f, 0.f, 0.f};
+  for (int c = lane; c < C; c += 32) welford_add(a, __ldg(xr + c));
   for (int o = 16; o > 0; o >>= 1) {
-    s += __shfl_xor_sync(0xffffffffu, s, o);
-    ss += __shfl_xor_sync(0xffffffffu, ss, o);
+    const Moments b = {__shfl_xor_sync(0xffffffffu, a.n, o), __shfl_xor_sync(0xffffffffu, a.m, o),
+                       __shfl_xor_sync(0xffffffffu, a.M2, o)};
+    a = chan_merge(a, b);
   }
   if (lane == 0) {
-    const float mean = s / C;
-    const float var = fmaxf(ss / C - mean * mean, 0.0f);
-    stats[2 * row] = mean;
-    stats[2 * row + 1] = rsqrtf(var + eps);
+    stats[2 * row] = a.m;
+    stats[2 * row + 1] = rsqrtf(a.M2 / C + eps);
   }
 }
 
-__global__ void __launch_bounds__(256) ln_col_stats_kernel(const float* __restrict__ x, float* __restrict__ stats,
-                                                           int R, int C, float eps) {
-  const int b = blockIdx.y;
-  const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  if (c >= C) return;
-  const float* xb = x + (long long)b * R * C + c;
-  float s = 0.f, ss = 0.f;
-  for (int r = 0; r < R; ++r) {
-    const float v = __ldg(xb + (long long)r * C);
-    s += v;
-    ss += v * v;
+// cols: a block covers 32 columns x kColGroups row groups; thread (tx, ty) takes rows ty, ty + kColGroups, ... of
+// column tx (a warp reads 32 consecutive floats of one row), then the groups merge in shared memory in a fixed tree
+// (chains of ceil(R / kColGroups), three merge levels).  Writes (mean, rstd) at stats[2 * (b * C + c)].
+constexpr int kColGroups = 8;
+__global__ void __launch_bounds__(32 * kColGroups) ln_col_stats_kernel(const float* __restrict__ x,
+                                                                       float* __restrict__ stats, int R, int C,
+                                                                       float eps) {
+  __shared__ Moments part[kColGroups][32];
+  const int b = blockIdx.y, tx = threadIdx.x, ty = threadIdx.y;
+  const int c = blockIdx.x * 32 + tx;
+  Moments a = {0.f, 0.f, 0.f};
+  if (c < C) {
+    const float* xb = x + (long long)b * R * C + c;
+    for (int r = ty; r < R; r += kColGroups) welford_add(a, __ldg(xb + (long long)r * C));
   }
-  const float mean = s / R;
-  const float var = fmaxf(ss / R - mean * mean, 0.0f);
-  stats[2 * ((long long)b * C + c)] = mean;
-  stats[2 * ((long long)b * C + c) + 1] = rsqrtf(var + eps);
+  part[ty][tx] = a;
+  for (int s = kColGroups / 2; s > 0; s >>= 1) {
+    __syncthreads();
+    if (ty < s) part[ty][tx] = chan_merge(part[ty][tx], part[ty + s][tx]);
+  }
+  if (ty == 0 && c < C) {
+    const Moments t = part[0][tx];
+    stats[2 * ((long long)b * C + c)] = t.m;
+    stats[2 * ((long long)b * C + c) + 1] = rsqrtf(t.M2 / R + eps);
+  }
 }
 
 // x [B][R][C] -> out [B][C][R_pad] (transposed), optional normalisation.  64 x 64 tiles through shared memory: the
@@ -491,7 +521,7 @@ extern "C" int avc_ln_transpose(const float* x, const float* gamma, const float*
     ln_row_stats_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, stream>>>(x, scratch, rows, C, 1e-5f);
     count_launch();
   } else if (ln_axis == 2) {
-    ln_col_stats_kernel<<<dim3((C + 255) / 256, B), 256, 0, stream>>>(x, scratch, R, C, 1e-5f);
+    ln_col_stats_kernel<<<dim3((C + 31) / 32, B), dim3(32, kColGroups), 0, stream>>>(x, scratch, R, C, 1e-5f);
     count_launch();
   }
   dim3 grid((C + kLnTile - 1) / kLnTile, (R_pad + kLnTile - 1) / kLnTile, B);

@@ -407,7 +407,8 @@ int avc_conv_to_mono_tanh(const float* x, const float* w, float bias, float* out
 
 /* ------------------------------------------------------------------------------------------------------------
  * MetaPool / MetaConv glue (factory/MetaPool.py, factory/MetaConv.py, factory/MLPMixer.py).  All inputs are fp32
- * channels-last; `out_dtype` selects the operand format of the output (0 fp32, 1 bf16, 2 split bf16).
+ * channels-last; `out_dtype` selects the operand format of the output (0 fp32, TF32-rounded when out_round_tf32,
+ * 1 bf16, 2 split bf16, 3 fp16 saturating at +-65504).
  * ------------------------------------------------------------------------------------------------------------ */
 
 /* GroupNorm(1, C) statistics (factory/Norm.py:53-60): stats[b] = {mean, 1/sqrt(biased var + eps)} over the n
@@ -427,20 +428,25 @@ int avc_gn_apply(const float* x, const float* stats, const float* gamma, const f
 
 /* einops "b c (h p1) (w p2) -> b (h w) (p1 p2 c)" (factory/MLPMixer.py:76-78) of the S x S image whose rows are the
  * CHANNELS and whose columns are the LENGTH axis of a [B][L=S][C=S] channels-last tensor, optionally after
- * GroupNorm(1, S) (stats/gamma/beta may be NULL): tokens [B][(S/p)^2][p*p] in operand format. */
+ * GroupNorm(1, S) (stats/gamma/beta may be NULL): tokens [B][(S/p)^2][p*p] in operand format.  S % p == 0, S % 4 == 0
+ * and (p*p) % 8 == 0. */
 int avc_patchify(const float* a, const float* stats, const float* gamma, const float* beta, void* out_op, int out_dtype,
                  int out_round_tf32, int B, int S, int p, void* stream);
 
 /* Transpose with optional LayerNorm (factory/MLPMixer.py:27-33): x [B][R][C] fp32 -> out_op [B][C][R] (operand
  * format) and/or out_f32 [B][C][R] (the un-normalised values).  ln_axis: 0 none, 1 normalise every ROW over its C
  * entries (gamma/beta indexed by column), 2 normalise every COLUMN over its R entries (gamma/beta indexed by row);
- * biased variance, eps 1e-5.  `scratch` holds 2*B*max(R,C) floats. */
+ * biased variance, eps 1e-5.  out_op and out_f32 have R_pad = R rounded up to 8 columns; columns [R, R_pad) are zero.
+ * `scratch` holds 2*B*max(R,C) floats; it receives the LayerNorm statistics as (mean, rstd) float pairs, at
+ * scratch[2*(b*R + r)] for row r on axis 1 and at scratch[2*(b*C + c)] for column c on axis 2 (unused on axis 0).  They
+ * are accumulated as centred sums (Welford, Chan's merge), so their error grows linearly, not quadratically, with
+ * |mean| / std. */
 int avc_ln_transpose(const float* x, const float* gamma, const float* beta, int ln_axis, void* out_op, int out_dtype,
                      int out_round_tf32, float* out_f32, float* scratch, int B, int R, int C, void* stream);
 
 /* Meta decoder input (factory/MetaPool.py:262-271 feeding Decoder.forward:160-162, which reads the (B, T, 2H+E)
  * tensor as channels = T, length = 2H+E): out[b][f][t] = f < 2H ? codes[b][t / freq][f] : c_trg[b][f - 2H],
- * channels-last [B][2H+E][T] in operand format.  T multiple of 4. */
+ * channels-last [B][2H+E][T] in operand format.  T % 8 == 0 and T % freq == 0. */
 int avc_meta_decoder_input(const float* codes, const float* c_trg, void* out_op, int out_dtype, int out_round_tf32,
                            int B, int T, int freq, int H2, int E, void* stream);
 
