@@ -13,7 +13,7 @@ ACT_NONE, ACT_RELU, ACT_TANH, ACT_LRELU, ACT_GELU, ACT_LOG10_CLAMP = 0, 1, 2, 3,
 ACTS = {"none": ACT_NONE, "relu": ACT_RELU, "tanh": ACT_TANH, "lrelu": ACT_LRELU, "gelu": ACT_GELU,
         "log10_clamp": ACT_LOG10_CLAMP}
 
-EXPORTS = ["avc_version", "avc_last_error", "avc_launch_count", "avc_conv_gemm", "avc_lstm_seq", "avc_lstm_seq_ws", "avc_lstm_stack_ws",
+EXPORTS = ["avc_version", "avc_last_error", "avc_launch_count", "avc_conv_gemm", "avc_lstm_seq", "avc_lstm_seq2", "avc_lstm_seq_ws", "avc_lstm_stack_ws",
            "avc_bilstm_small", "avc_concat_bcast", "avc_linear_l2norm", "avc_linear_rows", "avc_transpose_pad",
            "avc_conv_to_mono_tanh", "avc_gn_stats", "avc_gn_pool_residual", "avc_gn_apply", "avc_patchify",
            "avc_ln_transpose", "avc_meta_decoder_input", "avc_gather_codes", "avc_global_stats", "avc_adain", "avc_audio_frames",
@@ -237,6 +237,8 @@ def load():
     lib.avc_conv_gemm.restype = ctypes.c_int
     lib.avc_lstm_seq.argtypes = [ctypes.POINTER(LstmDesc), ctypes.c_void_p]
     lib.avc_lstm_seq.restype = ctypes.c_int
+    lib.avc_lstm_seq2.argtypes = [ctypes.POINTER(LstmDesc), ctypes.POINTER(LstmDesc), ctypes.c_void_p]
+    lib.avc_lstm_seq2.restype = ctypes.c_int
     lib.avc_lstm_seq_ws.argtypes = [ctypes.POINTER(LstmWsDesc), ctypes.c_void_p]
     lib.avc_lstm_seq_ws.restype = ctypes.c_int
     lib.avc_lstm_stack_ws.argtypes = [ctypes.POINTER(LstmStackDesc), ctypes.c_void_p]

@@ -19,7 +19,8 @@
 //
 // Two kernels:
 //   lstm_fused_kernel  (default) input projection and recurrence in one kernel, two TMEM accumulators: the x_t products
-//                      of frame t+1 run while the cell update and the grid barrier of frame t are in flight
+//                      of frame t+1 run while the cell update and the grid barrier of frame t are in flight; with
+//                      LAYERS = 2 it runs two stacked layers in one launch, two frames apart (avc_lstm_seq2)
 //   lstm_step_kernel   recurrence only, on a precomputed fp32 projection (xproj) -- small batches with wide inputs
 // and two launch modes for each:
 //   per-step    t_end = t_begin + 1, one launch per frame (stream order is the time dependency)
@@ -60,6 +61,15 @@ struct alignas(64) LstmParams {
   uint32_t stages;        // ring depth: as many stages as the shared-memory ring holds, at most kMaxStages
   uint32_t stage_tx;      // bytes one CTA's loads of a stage credit to the full barrier
 };
+
+// Two stacked layers in one launch (avc_lstm_seq2): l[1]'s input maps (tmap_xi) read l[0]'s hseq.
+struct LstmPair {
+  LstmParams l[2];
+};
+template <int LAYERS>
+using FusedArgs = std::conditional_t<LAYERS == 1, LstmParams, LstmPair>;
+__device__ __forceinline__ const LstmParams& layer_params(const LstmParams& p, int) { return p; }
+__device__ __forceinline__ const LstmParams& layer_params(const LstmPair& p, int l) { return p.l[l]; }
 
 // Accumulator layout of the split-bf16 mode.  Wide MMA (N = 2 * BN): B rows = this CTA's [W_hi tile ; W_lo tile], so with
 // h = BN / CTAS gate columns per CTA the accumulator columns are, per CTA r of the pair, [hi*hi (h) | hi*lo (h)] at
@@ -383,17 +393,120 @@ __global__ void __launch_bounds__(kNumThreads, 1) lstm_step_kernel(const __grid_
 // Warp roles: 0 = producer of everything that is independent of the recurrence (x_t tiles, W_ih tiles, W_hh tiles);
 // 1 = MMA issuer; 2..9 = cell warps; 10 = producer of the h_{t-1} tiles, which also owns the grid barrier.  Both
 // producers walk the same ring in the same order: frame t = num_kx input stages, then (t > 0) num_kb recurrent stages.
+//
+// LAYERS = 2 (avc_lstm_seq2): two stacked layers of equal H and G in one launch, layer 1 two frames behind layer 0, one
+// TMEM accumulator per layer.  Tick t (0 <= t <= T + 1) finishes frame t of layer 0 and frame t - 2 of layer 1; its
+// stage groups, in ring order (WaveTick), are
+//   rec0 = h0_{t-1} W_hh0   rec1 = h1_{t-3} W_hh1          after the tick's barrier: the serial chain
+//   in0  = x_{t+1} W_ih0    in1  = h0_{t-1} W_ih1          the shadow of the cell updates and of the next barrier
+// with one in0 group (frame 0) in front of tick 0.  Two frames apart, the inter-layer product h0 . W_ih1 reads h0 of
+// the PREVIOUS tick and leaves the chain.  Every accumulator still receives its input part, then its recurrent part,
+// with the MMAs of the one-layer kernel in the same order, so the outputs are bit-identical to two one-layer launches.
+// The in-groups reuse an accumulator within the tick, which no barrier covers: the issuer waits on tmem_empty[l], on
+// which every cell warp of the pair arrives after its last TMEM read of layer l.
 constexpr int kFusedThreads = kNumThreads + 32;
-constexpr int kBiasBytes = 1024;
+// Shared memory after the ring: the bias tile of each layer (4 * BN <= 512 bytes), then the stage counters in the last 16
+// bytes.  Two layers take 1.5 KB, not 2: the 7-stage rings of the 32 KB-stage modes then still fit beside it.
+template <int LAYERS>
+constexpr int kBiasBytes = LAYERS == 1 ? 1024 : 1536;
 
-template <int BN, int MODE, int CTAS>
-__global__ void __launch_bounds__(kFusedThreads, 1) lstm_fused_kernel(const __grid_constant__ LstmParams p) {
+struct WaveTick {
+  bool rec0, rec1, in0, in1;
+  bool cells;     // the cell warps update a layer (only tick 1 of T = 1 updates none)
+  __device__ WaveTick(int t, int T)
+      : rec0(t >= 1 && t < T), rec1(t >= 3), in0(t + 1 < T), in1(t >= 1 && t <= T), cells(t < T || t >= 2) {}
+};
+
+__device__ __forceinline__ uint32_t ld_acquire_cta(const uint32_t* ctr) {
+  uint32_t v;
+  asm volatile("ld.acquire.cta.shared::cta.u32 %0, [%1];" : "=r"(v) : "r"(smem_u32(ctr)) : "memory");
+  return v;
+}
+// Wait until a shared-memory counter that other threads advance with release semantics reaches `want` (acquire),
+// calling idle() between polls.
+template <class Idle>
+__device__ __forceinline__ void wait_count(const uint32_t* ctr, uint32_t want, Idle idle) {
+  const long long t0 = clock64();
+  for (uint32_t seen = ld_acquire_cta(ctr); seen < want; seen = ld_acquire_cta(ctr)) {
+    idle();
+    if (clock64() - t0 > 4000000000LL) {
+      printf("avc: shared counter timeout block %d seen %u want %u\n", (int)blockIdx.x, seen, want);
+      __trap();
+    }
+  }
+}
+__device__ __forceinline__ void wait_count(const uint32_t* ctr, uint32_t want) { wait_count(ctr, want, [] {}); }
+// Second half of grid_arrive_wait: wait until the batch group's counter reaches `target` (acquire).
+__device__ __forceinline__ void grid_wait(const unsigned int* bar, unsigned int target) {
+  const long long t0 = clock64();
+  unsigned int seen;
+  do {
+    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(bar) : "memory");
+    if (seen < target && clock64() - t0 > 4000000000LL) {
+      printf("avc: grid barrier timeout block %d seen %u target %u\n", (int)blockIdx.x, seen, target);
+      __trap();
+    }
+  } while (seen < target);
+}
+
+// One cell warp's share of frame t of one layer: its groups j of 8 hidden units (the two warps of a TMEM lane quarter
+// alternate), z = accumulator + bias, the LSTM cell on the register-resident c, the h stores, and c_state after the
+// launch's last frame.  `drained` (two-layer launch): right after its last TMEM read the warp hands the accumulator back
+// to the MMA issuer, an arrival on the leader CTA's barrier, ahead of its last group's cell math and stores.
+template <class SA, int MODE, int G, int NJ>
+__device__ __forceinline__ void cell_frame(const LstmParams& p, uint32_t lane_addr, const float* sbias, float (&cq)[NJ][8],
+                                           int half, bool valid, int b, int t, long long row, float* cp, int u0,
+                                           uint64_t* drained) {
+  constexpr int NG = G / 8;
+#pragma unroll
+  for (int jj = 0; jj < NJ; ++jj) {
+    const int j = half + jj * (kEpiWarps / 4);
+    if (j >= NG) break;
+    float acc[4][8];
+    load_gates<SA, G>(lane_addr, j, acc);
+    if (drained && j + kEpiWarps / 4 >= NG) {
+      tc_fence_before();
+      __syncwarp();
+      if ((threadIdx.x & 31) == 0) mbar_arrive_leader(drained);
+    }
+    if (valid) {
+      float z[4][8];
+#pragma unroll
+      for (int g = 0; g < 4; ++g) {
+#pragma unroll
+        for (int e = 0; e < 8; e += 4) {
+          const float4 x0 = *reinterpret_cast<const float4*>(sbias + g * G + j * 8 + e);       // broadcast reads
+          z[g][e] = acc[g][e] + x0.x;
+          z[g][e + 1] = acc[g][e + 1] + x0.y;
+          z[g][e + 2] = acc[g][e + 2] + x0.z;
+          z[g][e + 3] = acc[g][e + 3] + x0.w;
+        }
+      }
+      float cn[8], hn[8];
+#pragma unroll
+      for (int e = 0; e < 8; ++e) lstm_cell(z[0][e], z[1][e], z[2][e], z[3][e], cq[jj][e], cn[e], hn[e]);
+#pragma unroll
+      for (int e = 0; e < 8; ++e) cq[jj][e] = cn[e];
+      if (t + 1 == p.t_end) {       // a later launch (per-step mode) resumes from global memory
+#pragma unroll
+        for (int e = 0; e < 8; e += 4)
+          *reinterpret_cast<float4*>(cp + j * 8 + e) = make_float4(cn[e], cn[e + 1], cn[e + 2], cn[e + 3]);
+      }
+      store_h8<MODE>(p, row, b, t, u0 + j * 8, hn);
+    }
+  }
+}
+
+template <int BN, int MODE, int CTAS, int LAYERS>
+__global__ void __launch_bounds__(kFusedThreads, 1) lstm_fused_kernel(const __grid_constant__ FusedArgs<LAYERS> fp) {
   constexpr int PARTS = MODE >= 2 ? 2 : 1;       // weight tiles per stage (ring sizing)
   constexpr int APARTS = MODE == 2 ? 2 : 1;      // activation tiles per stage
   using SA = SplitAcc<BN, CTAS, MODE >= 2>;
-  using C = PipeCfg<BN, CTAS, PARTS, false, kBiasBytes, 2, SA::kCols>;
+  using C = PipeCfg<BN, CTAS, PARTS, false, kBiasBytes<LAYERS>, 2, SA::kCols>;
   constexpr int G = BN / 4;
-  static_assert(BN * 4 <= kBiasBytes - 16, "bias tile + the h_ready counter");
+  static_assert(LAYERS * BN * 4 <= kBiasBytes<LAYERS> - 16, "bias tiles + the stage counters");
+  const LstmParams& p = layer_params(fp, 0);
+  const LstmParams& p1 = layer_params(fp, LAYERS - 1);     // layer 1 of a two-layer launch
   extern __shared__ uint8_t smem_raw[];
   const PipeSmem s = carve_smem<C>(smem_raw);
   const int warp = threadIdx.x >> 5;
@@ -412,15 +525,212 @@ __global__ void __launch_bounds__(kFusedThreads, 1) lstm_fused_kernel(const __gr
     prefetch_tmap(&p.tmap_w);
     prefetch_tmap(&p.tmap_xi);
     prefetch_tmap(&p.tmap_wi);
+    if (LAYERS == 2) {
+      prefetch_tmap(&p1.tmap_h);
+      prefetch_tmap(&p1.tmap_w);
+      prefetch_tmap(&p1.tmap_xi);
+      prefetch_tmap(&p1.tmap_wi);
+    }
   }
-  float* sbias = reinterpret_cast<float*>(s.extra);
-  // Recurrent stages whose slot the static producer has claimed (empty barrier observed, W tiles in flight).  The h
-  // producer may not test the empty barriers itself: it skips the input stages, so it can be several ring rounds
-  // ahead of the consumer, and an mbarrier parity wait only tells adjacent phases apart.
-  uint32_t* h_ready = reinterpret_cast<uint32_t*>(s.extra + kBiasBytes - 16);
+  float* sbias = reinterpret_cast<float*>(s.extra);          // layer l's tile at sbias + l * BN
+  // Stages whose A tile the h producer loads and whose slot the static producer has claimed (empty barrier observed, W
+  // tiles in flight).  The h producer may not test the empty barriers itself: it skips the other stages, so it can be
+  // several ring rounds ahead of the consumer, and an mbarrier parity wait only tells adjacent phases apart.
+  uint32_t* h_ready = reinterpret_cast<uint32_t*>(s.extra + kBiasBytes<LAYERS> - 16);
+  // two-layer launch: cell updates done, one count per cell warp and tick that updates a layer.  Ticks without one are
+  // not counted: a warp would pass them at once, and its count would then stand in for a slower warp's unfinished one.
+  uint32_t* cells_done = h_ready + 1;
   if (threadIdx.x == 0) *h_ready = 0u;
+  if (LAYERS == 2 && threadIdx.x == 0) *cells_done = 0u;
   if (threadIdx.x >= 64 && threadIdx.x < 64 + BN) sbias[threadIdx.x - 64] = p.bias[n0 + threadIdx.x - 64];
+  if (LAYERS == 2 && threadIdx.x >= 64 + BN && threadIdx.x < 64 + 2 * BN)
+    sbias[threadIdx.x - 64] = p1.bias[n0 + threadIdx.x - 64 - BN];
   const uint32_t tmem_base = pipe_setup<C>(s);     // (its CTA / cluster barrier also publishes the bias tile)
+
+  if constexpr (LAYERS == 2) {
+    const int T = p.T;
+    // 12 clock64 stamps per (tick, CTA): 0 barrier passed, 1 first rec0 stage landed, 2 / 3 rec0 / rec1 issued,
+    // 4 / 5 layer 0 accumulator ready / cell done, 6 / 7 the same for layer 1, 8 the previous tick's cell warps done
+    // (seen by the h producer), 9 this tick's barrier arrival issued, 10 / 11 in0 / in1 issued
+    auto stamps = [&](int t) -> long long* {
+      return p.debug_clk ? p.debug_clk + ((long long)t * gridDim.x + blockIdx.x) * 12 : nullptr;
+    };
+    if (warp == 0) {
+      if (lane == 0) {
+        RingState rs;
+        uint32_t h_claimed = 0;
+        // nk stages {A tile, W tile(s)}: this thread credits each stage's full byte count and loads the W tiles, and
+        // the A tiles unless they come from the h producer (ta == nullptr)
+        auto group = [&](const CUtensorMap* tw, int nk, const CUtensorMap* ta, int frame) {
+          for (int kb = 0; kb < nk; ++kb) {
+            mbar_wait(&s.empty[rs.stage], rs.phase ^ 1u);
+            uint8_t* st = s.base + rs.stage * p.stage_bytes;
+            const int kc0 = kb * p.kc_elems;
+            if (CTAS == 1 || leader) mbar_arrive_expect_tx(&s.full[rs.stage], CTAS * p.stage_tx);
+            load_w<CTAS>(st + APARTS * p.a_tile, tw, &s.full[rs.stage], kc0, nb0);
+            if (ta) {
+              load_act<CTAS>(st, ta, &s.full[rs.stage], kc0, b0, frame);
+            } else {
+              ++h_claimed;
+              asm volatile("st.release.cta.shared::cta.u32 [%0], %1;" ::"r"(smem_u32(h_ready)), "r"(h_claimed) : "memory");
+            }
+            rs.advance(p.stages);
+          }
+        };
+        group(&p.tmap_wi, p.num_kx, &p.tmap_xi, 0);
+        for (int t = 0; t < T + 2; ++t) {
+          const WaveTick k(t, T);
+          if (k.rec0) group(&p.tmap_w, p.num_kb, nullptr, 0);
+          if (k.rec1) group(&p1.tmap_w, p1.num_kb, nullptr, 0);
+          if (k.in0) group(&p.tmap_wi, p.num_kx, &p.tmap_xi, t + 1);
+          if (k.in1) group(&p1.tmap_wi, p1.num_kx, nullptr, 0);
+        }
+      }
+      __syncwarp();
+    } else if (warp == 1) {
+      if (lane == 0 && leader) {
+        RingState rs;
+        uint32_t drain_phase = 0;    // bit l = parity of tmem_empty[l]
+        auto group = [&](int nk, uint32_t acc, bool first, long long* landed) {
+          for (int i = 0; i < nk; ++i) {
+            mbar_wait(&s.full[rs.stage], rs.phase);
+            if (landed && i == 0) *landed = clock64();
+            tc_fence_after();
+            const uint32_t a_hi = smem_u32(s.base + rs.stage * p.stage_bytes);
+            issue_stage<BN, MODE, CTAS>(a_hi, a_hi + p.a_tile, a_hi + APARTS * p.a_tile, acc, first && i == 0);
+            if (CTAS == 2) umma_commit_2sm(&s.empty[rs.stage], 0x3); else umma_commit(&s.empty[rs.stage]);
+            rs.advance(p.stages);
+          }
+        };
+        auto full = [&](int l) {
+          if (CTAS == 2) umma_commit_2sm(&s.tmem_full[l], 0x3); else umma_commit(&s.tmem_full[l]);
+        };
+        auto drained = [&](int l) {  // every cell warp of the pair has read layer l's accumulator of this tick
+          mbar_wait(&s.tmem_empty[l], (drain_phase >> l) & 1u);
+          drain_phase ^= 1u << l;
+          tc_fence_after();
+        };
+        const uint32_t acc0 = tmem_base, acc1 = tmem_base + static_cast<uint32_t>(SA::kCols);
+        group(p.num_kx, acc0, true, nullptr);
+        for (int t = 0; t < T + 2; ++t) {
+          long long* dbg = stamps(t);
+          const WaveTick k(t, T);
+          if (k.rec0) group(p.num_kb, acc0, false, dbg ? dbg + 1 : nullptr);
+          if (t < T) full(0);
+          if (dbg) dbg[2] = clock64();
+          if (k.rec1) group(p1.num_kb, acc1, false, nullptr);
+          if (t >= 2) full(1);
+          if (dbg) dbg[3] = clock64();
+          if (k.in0) {
+            drained(0);
+            group(p.num_kx, acc0, true, nullptr);
+          }
+          if (dbg) dbg[10] = clock64();
+          if (k.in1) {
+            if (t >= 2) drained(1);
+            group(p1.num_kx, acc1, true, nullptr);
+          }
+          if (dbg) dbg[11] = clock64();
+        }
+      }
+      __syncwarp();
+    } else if (warp == 2 + kEpiWarps) {
+      if (lane == 0) {
+        RingState rs;
+        uint32_t h_issued = 0;
+        unsigned int sync_count = 0;   // barriers arrived at
+        uint32_t cells_need = 0;       // cell-warp counts of the ticks so far
+        bool due = false;              // this CTA's arrival at the next tick's barrier is outstanding
+        long long* due_dbg = nullptr;
+        unsigned int* bar = p.grid_barrier + 32 * (unit / p.n_tiles);
+        // The next tick's barrier waits for this CTA's cell warps only, so the arrival goes out as soon as they are
+        // done -- also from inside the waits for ring slots of the in-groups, which are as long as those groups' MMAs:
+        // the barrier then runs under them instead of after them.
+        auto arrive = [&](bool block) {
+          if (!due || (!block && ld_acquire_cta(cells_done) < cells_need)) return;
+          wait_count(cells_done, cells_need);
+          if (due_dbg) due_dbg[8] = clock64();
+          // release: the cell warps' h stores (observed through cells_done) become visible with the counter
+          asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(bar) : "memory");
+          if (due_dbg) due_dbg[9] = clock64();
+          due = false;
+        };
+        auto skip = [&](int nk) {
+          for (int kb = 0; kb < nk; ++kb) rs.advance(p.stages);
+        };
+        auto group = [&](const CUtensorMap* ta, int nk, int frame) {
+          for (int kb = 0; kb < nk; ++kb) {
+            wait_count(h_ready, ++h_issued, [&] { arrive(false); });
+            load_act<CTAS>(s.base + rs.stage * p.stage_bytes, ta, &s.full[rs.stage], kb * p.kc_elems, b0, frame);
+            rs.advance(p.stages);
+          }
+        };
+        skip(p.num_kx);
+        for (int t = 0; t < T + 2; ++t) {
+          long long* dbg = stamps(t);
+          const WaveTick k(t, T);
+          if (t > 0) {
+            // h0_{t-1} and h1_{t-3} come from tick t - 1: this CTA's cell warps, then every CTA of the batch group
+            arrive(true);
+            grid_wait(bar, sync_count * (unsigned)(p.n_tiles * CTAS));
+          }
+          if (dbg) dbg[0] = clock64();
+          fence_proxy_async_global();   // h was written with generic stores (other CTAs)
+          if (k.cells) cells_need += kEpiWarps;
+          if (t + 1 < T + 2) {         // the next tick's barrier
+            ++sync_count;
+            due = true;
+            due_dbg = stamps(t + 1);
+          }
+          if (k.rec0) group(&p.tmap_h, p.num_kb, t - 1);
+          if (k.rec1) group(&p1.tmap_h, p1.num_kb, t - 3);
+          if (k.in0) skip(p.num_kx);
+          if (k.in1) group(&p1.tmap_xi, p1.num_kx, t - 1);
+        }
+      }
+      __syncwarp();
+    } else {
+      // cell warps: layer 0's update (h0_t) runs while rec1 is on the tensor pipe, then layer 1's (h1_{t-2})
+      constexpr int NJ = (G / 8 + kEpiWarps / 4 - 1) / (kEpiWarps / 4);
+      float cq[2][NJ][8];
+      uint32_t acc_phase = 0;      // bit l = parity of tmem_full[l]
+      const int q = warp & 3;
+      const int half = (warp - 2) >> 2;
+      const int b = b0 + q * 32 + lane;
+      const bool valid = b < p.B;
+      const int u0 = n_tile * G;
+      for (int t = 0; t < T + 2; ++t) {
+        long long* dbg = stamps(t);
+#pragma unroll
+        for (int l = 0; l < 2; ++l) {
+          const int f = t - 2 * l;         // frame of layer l this tick finishes
+          if (f < 0 || f >= T) continue;
+          if (f == 0) {
+#pragma unroll
+            for (int jj = 0; jj < NJ; ++jj)
+#pragma unroll
+              for (int e = 0; e < 8; ++e) cq[l][jj][e] = 0.f;
+          }
+          mbar_wait(&s.tmem_full[l], (acc_phase >> l) & 1u);
+          acc_phase ^= 1u << l;
+          tc_fence_after();
+          if (dbg && threadIdx.x == 64) dbg[4 + 2 * l] = clock64();
+          const uint32_t lane_addr =
+              tmem_base + static_cast<uint32_t>(l * SA::kCols) + (static_cast<uint32_t>(q * 32) << 16);
+          const LstmParams& pl = layer_params(fp, l);
+          cell_frame<SA, MODE, G, NJ>(pl, lane_addr, sbias + l * BN, cq[l], half, valid, b, f, (long long)b * T + f,
+                                      pl.c_state + (long long)b * pl.H + u0, u0, &s.tmem_empty[l]);
+          if (dbg && threadIdx.x == 64) dbg[5 + 2 * l] = clock64();
+        }
+        if (!WaveTick(t, T).cells) continue;
+        fence_proxy_async_global();   // order the h stores before later async-proxy (TMA) reads
+        __syncwarp();
+        if (lane == 0) asm volatile("red.release.cta.shared::cta.add.u32 [%0], 1;" ::"r"(smem_u32(cells_done)) : "memory");
+      }
+    }
+    pipe_teardown<C>(tmem_base);
+    return;
+  }
 
   if (warp == 0) {
     if (lane == 0) {
@@ -553,38 +863,7 @@ __global__ void __launch_bounds__(kFusedThreads, 1) lstm_fused_kernel(const __gr
       if (dbg && threadIdx.x == 64) dbg[4] = clock64();                    // accumulator ready
       const uint32_t lane_addr =
           tmem_base + static_cast<uint32_t>(buf * SA::kCols) + (static_cast<uint32_t>(q * 32) << 16);
-#pragma unroll
-      for (int jj = 0; jj < NJ; ++jj) {
-        const int j = half + jj * (kEpiWarps / 4);
-        if (j >= NG) break;
-        float acc[4][8];
-        load_gates<SA, G>(lane_addr, j, acc);
-        if (valid) {
-          float z[4][8];
-#pragma unroll
-          for (int g = 0; g < 4; ++g) {
-#pragma unroll
-            for (int e = 0; e < 8; e += 4) {
-              const float4 x0 = *reinterpret_cast<const float4*>(sbias + g * G + j * 8 + e);       // broadcast reads
-              z[g][e] = acc[g][e] + x0.x;
-              z[g][e + 1] = acc[g][e + 1] + x0.y;
-              z[g][e + 2] = acc[g][e + 2] + x0.z;
-              z[g][e + 3] = acc[g][e + 3] + x0.w;
-            }
-          }
-          float cn[8], hn[8];
-#pragma unroll
-          for (int e = 0; e < 8; ++e) lstm_cell(z[0][e], z[1][e], z[2][e], z[3][e], cq[jj][e], cn[e], hn[e]);
-#pragma unroll
-          for (int e = 0; e < 8; ++e) cq[jj][e] = cn[e];
-          if (t + 1 == p.t_end) {       // a later launch (per-step mode) resumes from global memory
-#pragma unroll
-            for (int e = 0; e < 8; e += 4)
-              *reinterpret_cast<float4*>(cp + j * 8 + e) = make_float4(cn[e], cn[e + 1], cn[e + 2], cn[e + 3]);
-          }
-          store_h8<MODE>(p, row, b, t, u0 + j * 8, hn);
-        }
-      }
+      cell_frame<SA, MODE, G, NJ>(p, lane_addr, sbias, cq, half, valid, b, t, row, cp, u0, nullptr);
       fence_proxy_async_global();   // order the h stores before later async-proxy (TMA) reads
       tc_fence_before();            // ... and this warp's TMEM reads before the MMAs that reuse the accumulator
       __syncwarp();
@@ -595,20 +874,24 @@ __global__ void __launch_bounds__(kFusedThreads, 1) lstm_fused_kernel(const __gr
   pipe_teardown<C>(tmem_base);
 }
 
-template <int BN, int MODE, int CTAS, bool FUSED>
-static int run(LstmParams p, const avc_lstm_desc* d, int m_tiles, cudaStream_t stream) {
+template <int BN, int MODE, int CTAS, bool FUSED, int LAYERS = 1>
+static int run(FusedArgs<LAYERS> args, const avc_lstm_desc* d, int m_tiles, cudaStream_t stream) {
   auto kern = [] {      // (if constexpr: a tile width built for one kernel only must not instantiate the other)
-    if constexpr (FUSED) return lstm_fused_kernel<BN, MODE, CTAS>;
+    if constexpr (FUSED) return lstm_fused_kernel<BN, MODE, CTAS, LAYERS>;
     else return lstm_step_kernel<BN, MODE, CTAS>;
   }();
+  LstmParams* layer[LAYERS];
+  if constexpr (LAYERS == 1) layer[0] = &args;
+  else for (int l = 0; l < LAYERS; ++l) layer[l] = &args.l[l];
+  const LstmParams& p = *layer[0];
   constexpr int kAccCols = SplitAcc<BN, CTAS, MODE >= 2>::kCols;
-  using C = std::conditional_t<FUSED, PipeCfg<BN, CTAS, MODE >= 2 ? 2 : 1, false, kBiasBytes, 2, kAccCols>,
+  using C = std::conditional_t<FUSED, PipeCfg<BN, CTAS, MODE >= 2 ? 2 : 1, false, kBiasBytes<LAYERS>, 2, kAccCols>,
                                PipeCfg<BN, CTAS, MODE >= 2 ? 2 : 1, false, BN / 32 * kATileBytes, 1, kAccCols>>;
   constexpr int kThreads = FUSED ? kFusedThreads : kNumThreads;
   // small batches shrink the stage (a_rows < 128): the same ring memory then holds more, shallower stages, which is what
   // a latency-bound frame wants (a TMA round trip costs ~3 K cycles whatever the tile size)
   const int fit = C::kStages * C::kStageBytes / p.stage_bytes;
-  p.stages = (uint32_t)(fit < kMaxStages ? fit : kMaxStages);
+  for (LstmParams* lp : layer) lp->stages = (uint32_t)(fit < kMaxStages ? fit : kMaxStages);
   static PerDeviceOnce configured;
   if (configured.first_use()) {
     AVC_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes));
@@ -626,11 +909,14 @@ static int run(LstmParams p, const avc_lstm_desc* d, int m_tiles, cudaStream_t s
     if (rc != 0) return rc;   // AVC_ERR_NOT_RESIDENT: the caller may fall back to one launch per frame
     AVC_REQUIRE((m_tiles + CTAS - 1) / CTAS <= 64, "avc_lstm_seq: at most 64 batch groups in persistent mode");
     AVC_CHECK_CUDA(cudaMemsetAsync(d->grid_barrier, 0, 64 * 32 * sizeof(unsigned int), stream));
-    p.t_begin = 0;
-    p.t_end = d->T;
-    AVC_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
+    for (LstmParams* lp : layer) {
+      lp->t_begin = 0;
+      lp->t_end = d->T;
+    }
+    AVC_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, args));
     count_launch();
   } else {
+    AVC_REQUIRE(LAYERS == 1, "avc_lstm_seq2: persistent mode only");
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = CTAS;
     attr[0].val.clusterDim.y = 1;
@@ -638,44 +924,34 @@ static int run(LstmParams p, const avc_lstm_desc* d, int m_tiles, cudaStream_t s
     cfg.attrs = attr;
     cfg.numAttrs = CTAS > 1 ? 1 : 0;
     for (int t = 0; t < d->T; ++t) {
-      p.t_begin = t;
-      p.t_end = t + 1;
-      AVC_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
+      layer[0]->t_begin = t;
+      layer[0]->t_end = t + 1;
+      AVC_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, args));
     }
     count_launch(d->T);
   }
   return 0;
 }
 
-// h_last[b] = hseq_f32[b][lengths[b] - 1] (a padded batch).  The recurrence kernels keep their T - 1 store: a
-// per-utterance comparison in their cell epilogue costs 4-9 registers in every instantiation (-Xptxas -v), so the
-// variable-length form reads the exact fp32 copy of the sequence instead -- the same bits the in-kernel store writes.
-__global__ void __launch_bounds__(256) gather_last_kernel(const float* __restrict__ hseq_f32, const int* __restrict__ lengths,
-                                                          float* __restrict__ h_last, int T, int H) {
-  const int b = blockIdx.x;
-  const float4* src = reinterpret_cast<const float4*>(hseq_f32 + ((long long)b * T + __ldg(lengths + b) - 1) * H);
-  float4* dst = reinterpret_cast<float4*>(h_last + (long long)b * H);
-  for (int i = threadIdx.x; i < H / 4; i += blockDim.x) dst[i] = src[i];
+// Calls f(BN, MODE, CTAS), each an std::integral_constant, for the kernel instantiation of a layer's shape.
+template <int N>
+using IntC = std::integral_constant<int, N>;
+template <class F>
+static int dispatch(int bn, int dtype, int ctas, F&& f) {
+  auto with_ctas = [&](auto bn_c, auto mode_c) { return ctas == 2 ? f(bn_c, mode_c, IntC<2>{}) : f(bn_c, mode_c, IntC<1>{}); };
+  auto with_mode = [&](auto bn_c) {
+    switch (dtype) {
+      case AVC_DTYPE_TF32: return with_ctas(bn_c, IntC<0>{});
+      case AVC_DTYPE_BF16: return with_ctas(bn_c, IntC<1>{});
+      case AVC_DTYPE_F16: return with_ctas(bn_c, IntC<3>{});
+      default: return with_ctas(bn_c, IntC<2>{});
+    }
+  };
+  return bn == 64 ? with_mode(IntC<64>{}) : with_mode(IntC<128>{});
 }
 
-}  // namespace avc
-
-extern "C" int avc_lstm_seq(const avc_lstm_desc* d, void* stream_v) {
-  using namespace avc;
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
-  AVC_REQUIRE(d != nullptr, "avc_lstm_seq: null descriptor");
-  if (d->lengths && d->h_last) {
-    AVC_REQUIRE(d->hseq_f32 != nullptr, "avc_lstm_seq: lengths with h_last need hseq_f32 (h_last is read from it)");
-    avc_lstm_desc full = *d;
-    full.h_last = nullptr;
-    full.lengths = nullptr;
-    const int rc = avc_lstm_seq(&full, stream_v);
-    if (rc != 0) return rc;
-    gather_last_kernel<<<d->B, 256, 0, stream>>>(d->hseq_f32, d->lengths, d->h_last, d->T, d->H);
-    AVC_CHECK_CUDA(cudaGetLastError());
-    count_launch();
-    return 0;
-  }
+// Kernel parameters of one layer (validated); m_tiles = 128-utterance tiles, ctas = CTAs per batch group.
+static int lstm_params(const avc_lstm_desc* d, LstmParams& p, int& m_tiles, int& ctas) {
   AVC_REQUIRE(d->dtype >= AVC_DTYPE_TF32 && d->dtype <= AVC_DTYPE_F16, "avc_lstm_seq: bad dtype %d", d->dtype);
   AVC_REQUIRE(d->gate_group == 16 || d->gate_group == 32, "avc_lstm_seq: gate_group %d (16 or 32)", d->gate_group);
   const bool fused = d->xin != nullptr;
@@ -694,14 +970,13 @@ extern "C" int avc_lstm_seq(const avc_lstm_desc* d, void* stream_v) {
   const int n_tiles = d->H / d->gate_group;
   const uint64_t ld = split ? 2 * H : H;     // elements per row of hseq ([hi | lo] when split)
   const uint64_t ldw_hh = w2 ? 2 * H : H;    // elements per row of the packed W_hh
-  const int m_tiles = (d->B + kBlockM - 1) / kBlockM;
-  const int ctas = m_tiles >= 2 ? 2 : 1;
+  m_tiles = (d->B + kBlockM - 1) / kBlockM;
+  ctas = m_tiles >= 2 ? 2 : 1;
   // A small batch owned by one CTA loads only its real rows (rounded up to 8): the MMA still spans 128 rows, but the
   // rows past the batch are never stored and every accumulator row depends on its own operand row only, so whatever
   // those shared-memory rows hold is harmless -- and the stage shrinks from 32 KB to a few KB of activations.
   const int a_rows = m_tiles == 1 ? (d->B + 7) / 8 * 8 : kBlockM;
 
-  LstmParams p;
   memset(&p, 0, sizeof(p));
   const uint32_t parts = split ? 2 : 1, wparts = w2 ? 2 : 1;
   {
@@ -748,22 +1023,67 @@ extern "C" int avc_lstm_seq(const avc_lstm_desc* d, void* stream_v) {
   p.a_tile = a_rows * kRowBytes;
   p.stage_bytes = (int)parts * p.a_tile + (int)wparts * (bn / ctas * kRowBytes);
   p.stage_tx = (uint32_t)p.stage_bytes;
-#define AVC_LSTM_DISPATCH3(BN_, MODE_, CTAS_) \
-  return fused ? run<BN_, MODE_, CTAS_, true>(p, d, m_tiles, stream) : run<BN_, MODE_, CTAS_, false>(p, d, m_tiles, stream);
-#define AVC_LSTM_DISPATCH2(BN_, MODE_) \
-  if (ctas == 2) { AVC_LSTM_DISPATCH3(BN_, MODE_, 2) } else { AVC_LSTM_DISPATCH3(BN_, MODE_, 1) }
-#define AVC_LSTM_DISPATCH(BN_)                           \
-  switch (d->dtype) {                                    \
-    case AVC_DTYPE_TF32: AVC_LSTM_DISPATCH2(BN_, 0)      \
-    case AVC_DTYPE_BF16: AVC_LSTM_DISPATCH2(BN_, 1)      \
-    case AVC_DTYPE_F16: AVC_LSTM_DISPATCH2(BN_, 3)       \
-    default: AVC_LSTM_DISPATCH2(BN_, 2)                  \
+  return 0;
+}
+
+// h_last[b] = hseq_f32[b][lengths[b] - 1] (a padded batch).  The recurrence kernels keep their T - 1 store: a
+// per-utterance comparison in their cell epilogue costs 4-9 registers in every instantiation (-Xptxas -v), so the
+// variable-length form reads the exact fp32 copy of the sequence instead -- the same bits the in-kernel store writes.
+__global__ void __launch_bounds__(256) gather_last_kernel(const float* __restrict__ hseq_f32, const int* __restrict__ lengths,
+                                                          float* __restrict__ h_last, int T, int H) {
+  const int b = blockIdx.x;
+  const float4* src = reinterpret_cast<const float4*>(hseq_f32 + ((long long)b * T + __ldg(lengths + b) - 1) * H);
+  float4* dst = reinterpret_cast<float4*>(h_last + (long long)b * H);
+  for (int i = threadIdx.x; i < H / 4; i += blockDim.x) dst[i] = src[i];
+}
+
+}  // namespace avc
+
+extern "C" int avc_lstm_seq(const avc_lstm_desc* d, void* stream_v) {
+  using namespace avc;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
+  AVC_REQUIRE(d != nullptr, "avc_lstm_seq: null descriptor");
+  if (d->lengths && d->h_last) {
+    AVC_REQUIRE(d->hseq_f32 != nullptr, "avc_lstm_seq: lengths with h_last need hseq_f32 (h_last is read from it)");
+    avc_lstm_desc full = *d;
+    full.h_last = nullptr;
+    full.lengths = nullptr;
+    const int rc = avc_lstm_seq(&full, stream_v);
+    if (rc != 0) return rc;
+    gather_last_kernel<<<d->B, 256, 0, stream>>>(d->hseq_f32, d->lengths, d->h_last, d->T, d->H);
+    AVC_CHECK_CUDA(cudaGetLastError());
+    count_launch();
+    return 0;
   }
-  switch (bn) {
-    case 64: AVC_LSTM_DISPATCH(64)
-    default: AVC_LSTM_DISPATCH(128)
+  LstmParams p;
+  int m_tiles, ctas;
+  const int rc = lstm_params(d, p, m_tiles, ctas);
+  if (rc != 0) return rc;
+  const bool fused = d->xin != nullptr;
+  return dispatch(4 * d->gate_group, d->dtype, ctas, [&](auto bn_c, auto mode_c, auto ctas_c) {
+    constexpr int BN = decltype(bn_c)::value, MODE = decltype(mode_c)::value, CTAS = decltype(ctas_c)::value;
+    return fused ? run<BN, MODE, CTAS, true>(p, d, m_tiles, stream) : run<BN, MODE, CTAS, false>(p, d, m_tiles, stream);
+  });
+}
+
+extern "C" int avc_lstm_seq2(const avc_lstm_desc* l0, const avc_lstm_desc* l1, void* stream_v) {
+  using namespace avc;
+  AVC_REQUIRE(l0 != nullptr && l1 != nullptr, "avc_lstm_seq2: null descriptor");
+  AVC_REQUIRE(l0->B == l1->B && l0->T == l1->T && l0->H == l1->H && l0->dtype == l1->dtype &&
+                  l0->gate_group == l1->gate_group,
+              "avc_lstm_seq2: the layers differ in B, T, H, dtype or gate_group");
+  AVC_REQUIRE(l0->xin && l1->xin, "avc_lstm_seq2: both layers need the fused input projection (xin, w_ih, bias)");
+  AVC_REQUIRE(l1->xin == l0->hseq, "avc_lstm_seq2: layer 1 must read layer 0's hseq");
+  AVC_REQUIRE(l0->persistent && l1->persistent, "avc_lstm_seq2: persistent mode only");
+  AVC_REQUIRE(!l0->lengths && !l1->lengths && !l0->h_last && !l1->h_last, "avc_lstm_seq2: no lengths or h_last");
+  LstmPair pair;
+  int m_tiles, ctas;
+  for (int l = 0; l < 2; ++l) {
+    const int rc = lstm_params(l ? l1 : l0, pair.l[l], m_tiles, ctas);
+    if (rc != 0) return rc;
   }
-#undef AVC_LSTM_DISPATCH
-#undef AVC_LSTM_DISPATCH3
-#undef AVC_LSTM_DISPATCH2
+  return dispatch(4 * l0->gate_group, l0->dtype, ctas, [&](auto bn_c, auto mode_c, auto ctas_c) {
+    constexpr int BN = decltype(bn_c)::value, MODE = decltype(mode_c)::value, CTAS = decltype(ctas_c)::value;
+    return run<BN, MODE, CTAS, true, 2>(pair, l0, m_tiles, static_cast<cudaStream_t>(stream_v));
+  });
 }

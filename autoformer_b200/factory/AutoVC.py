@@ -205,9 +205,8 @@ class AutoVC(layers.PlanOwner, nn.Module):
                 ops.zero_tail(h, 0, T, lengths)
             if taps is not None:
                 taps[f"dec_conv{i}"] = packing.act_to_float(h, prec)
-        h = plan.lstm2[0](h, B, T, persistent=self.persistent_lstm)
         f32 = torch.empty(B, T, 1024, dtype=torch.float32, device=dev) if taps is not None else None
-        h = plan.lstm2[1](h, B, T, hseq_f32=f32, persistent=self.persistent_lstm)
+        h = layers.lstm_pair(plan.lstm2, h, B, T, hseq_f32=f32, persistent=self.persistent_lstm)
         if taps is not None:
             taps["dec_lstm2"] = f32
         mel = torch.empty(B, T, 80, dtype=torch.float32, device=dev)

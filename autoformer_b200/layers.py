@@ -307,6 +307,42 @@ class LstmLayer:
                             persistent=persistent, **_lengths_kw(lengths))
 
 
+def wavefront_eligible(pair, B, persistent):
+    """Whether lstm_pair runs the two layers as one launch (ops.lstm_seq2) for a batch of B: persistent, not the
+    small-batch weight-stationary path, the fused input projection for both layers, equal hidden sizes.  The benchmark
+    has workloads on both sides: the 512-utterance batches take it, the smaller ones and the sub-batch tails do not."""
+    l0, l1 = pair
+    return (persistent and l0.H == l1.H and B <= ops.persistent_batch_cap(l0.H) and
+            not any(l.ws and ops.ws_supported(B, l.H, l.precision) for l in pair) and
+            l0.use_fused(B) and l1.use_fused(B))
+
+
+def lstm_pair(pair, x, B, T, hseq_f32=None, persistent=False, hseq=None):
+    """Two stacked LstmLayers (nn.LSTM(num_layers = 2)): layer 1's output sequence, with its exact fp32 copy in
+    hseq_f32 when given.  Eligible batches (wavefront_eligible) run both layers as one persistent launch, layer 1 two
+    frames behind layer 0, which hides each layer's cell update and barrier behind the other's MMAs; the results are
+    bit-identical to calling the layers one after the other, which is what every other batch does."""
+    l0, l1 = pair
+    cap = ops.persistent_batch_cap(l0.H) if persistent else 0
+    if persistent and B > cap > 0:
+        # independent utterances: one wave of the persistent grid at a time, as LstmLayer splits its batch
+        out = ops.alloc_act(B, T, l1.H, l1.precision, x.device) if hseq is None else hseq
+        for b0 in range(0, B, cap):
+            b1 = min(B, b0 + cap)
+            lstm_pair(pair, x[b0:b1], b1 - b0, T, hseq_f32=hseq_f32[b0:b1] if hseq_f32 is not None else None,
+                      persistent=True, hseq=out[b0:b1])
+        return out
+    if wavefront_eligible(pair, B, persistent):
+        group = ops.choose_gate_group(B, l0.H, True)
+        (wih0, bias0, hh0), (wih1, bias1, hh1) = l0.fused_packs(group), l1.fused_packs(group)
+        out = ops.lstm_seq2((hh0, hh1), B, T, l0.H, l0.precision, group, x, (wih0, wih1), (bias0, bias1), l0.C_in,
+                            hseq=(None, hseq), hseq_f32=(None, hseq_f32))
+        if out is not None:
+            return out[1]
+    h = l0(x, B, T, persistent=persistent)      # the device cannot hold the grid, or an ineligible batch
+    return l1(h, B, T, hseq_f32=hseq_f32, persistent=persistent, hseq=hseq)
+
+
 def lstm_layers(sd, prefix, num_layers, precision):
     return [LstmLayer(sd[f"{prefix}.weight_ih_l{l}"], sd[f"{prefix}.weight_hh_l{l}"], sd[f"{prefix}.bias_ih_l{l}"],
                       sd[f"{prefix}.bias_hh_l{l}"], precision) for l in range(num_layers)]

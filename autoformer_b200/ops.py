@@ -356,14 +356,9 @@ def choose_gate_group(B, H, persistent=False, n_sm=148):
     raise RuntimeError(f"no gate group fits B={B} H={H} persistent={persistent}")
 
 
-def lstm_seq(xproj, w_hh, B, T, H, precision, group, hseq=None, hseq_f32=None, h_last=None, persistent=False,
-             debug_clk=None, xin=None, w_ih=None, bias=None, c_in=None, lengths=None):
-    """Run the recurrence of one uni-directional layer.  Either xproj [B*T][4H] fp32 (packed gate order, bias
-    included), or -- fused input projection -- the layer input xin [B][T][C'] in the operand format of `precision`
-    with w_ih / bias from packing.pack_lstm_ih_fused and c_in logical input channels.
-    lengths: optional device int32 [B] of a padded batch -- h_last[b] is then h at frame lengths[b] - 1 (taken from the
-    exact fp32 sequence, allocated here when hseq_f32 is not given)."""
-    lib = _lib.load()
+def _lstm_desc(xproj, w_hh, B, T, H, precision, group, hseq, hseq_f32, h_last, persistent, debug_clk, xin, w_ih, bias,
+               c_in, lengths, c_state):
+    """Checked avc_lstm_desc of one layer; returns (desc, hseq, tensors the descriptor points to)."""
     fused = xin is not None
     _require_cuda(xin if fused else xproj, w_hh)
     dev = w_hh.device
@@ -386,7 +381,9 @@ def lstm_seq(xproj, w_hh, B, T, H, precision, group, hseq=None, hseq_f32=None, h
         hseq = alloc_act(B, T, H, precision, dev)
     assert hseq.is_contiguous() and hseq.shape == (B, T, packing.act_channels(H, precision))
     assert hseq.dtype == TORCH_DTYPE[precision]
-    c_state = torch.empty(B, H, dtype=torch.float32, device=dev)
+    if c_state is None:
+        c_state = torch.empty(B, H, dtype=torch.float32, device=dev)
+    assert c_state.is_contiguous() and c_state.shape == (B, H) and c_state.dtype == torch.float32
     d = _lib.LstmDesc()
     if fused:
         d.xin, d.xin_channels, d.xin_ld = xin.data_ptr(), c_in, xin.stride(1)
@@ -416,6 +413,21 @@ def lstm_seq(xproj, w_hh, B, T, H, precision, group, hseq=None, hseq_f32=None, h
         d.grid_barrier = bar.data_ptr()
     if debug_clk is not None:
         d.debug_clk = debug_clk.data_ptr()
+    return d, hseq, (c_state, bar, hseq_f32)
+
+
+def lstm_seq(xproj, w_hh, B, T, H, precision, group, hseq=None, hseq_f32=None, h_last=None, persistent=False,
+             debug_clk=None, xin=None, w_ih=None, bias=None, c_in=None, lengths=None, c_state=None):
+    """Run the recurrence of one uni-directional layer.  Either xproj [B*T][4H] fp32 (packed gate order, bias
+    included), or -- fused input projection -- the layer input xin [B][T][C'] in the operand format of `precision`
+    with w_ih / bias from packing.pack_lstm_ih_fused and c_in logical input channels.
+    lengths: optional device int32 [B] of a padded batch -- h_last[b] is then h at frame lengths[b] - 1 (taken from the
+    exact fp32 sequence, allocated here when hseq_f32 is not given).  c_state: optional [B][H] fp32 that receives the
+    final cell state (scratch allocated here otherwise)."""
+    lib = _lib.load()
+    fused = xin is not None
+    d, hseq, keep = _lstm_desc(xproj, w_hh, B, T, H, precision, group, hseq, hseq_f32, h_last, persistent, debug_clk,
+                               xin, w_ih, bias, c_in, lengths, c_state)
     with PROFILER.span("lstm_step", flops=2.0 * 4 * H * (H + (c_in if fused else 0)) * B * T,
                        launches=1 if persistent else T):
         rc = lib.avc_lstm_seq(ctypes.byref(d), _stream())
@@ -431,6 +443,25 @@ def lstm_seq(xproj, w_hh, B, T, H, precision, group, hseq=None, hseq_f32=None, h
             rc = lib.avc_lstm_seq(ctypes.byref(d), _stream())
         _lib.check(rc, "avc_lstm_seq")
     return hseq
+
+
+def lstm_seq2(w_hh, B, T, H, precision, group, xin, w_ih, bias, c_in, hseq=(None, None), hseq_f32=(None, None),
+              c_state=(None, None), debug_clk=None):
+    """Two stacked layers with fused input projections as ONE persistent launch (avc_lstm_seq2), layer 1 two frames
+    behind layer 0: bit-identical to two persistent lstm_seq calls.  w_hh / w_ih / bias / hseq / hseq_f32 / c_state are
+    (layer 0, layer 1) pairs; xin is layer 0's input with c_in channels, layer 1 reads layer 0's hseq.  Returns the two
+    hseq tensors, or None when the device cannot hold the grid (nothing was launched; run the layers one by one)."""
+    lib = _lib.load()
+    d0, h0, keep0 = _lstm_desc(None, w_hh[0], B, T, H, precision, group, hseq[0], hseq_f32[0], None, True, debug_clk,
+                               xin, w_ih[0], bias[0], c_in, None, c_state[0])
+    d1, h1, keep1 = _lstm_desc(None, w_hh[1], B, T, H, precision, group, hseq[1], hseq_f32[1], None, True, None,
+                               h0, w_ih[1], bias[1], H, None, c_state[1])
+    with PROFILER.span("lstm_step", flops=2.0 * 4 * H * ((H + c_in) + 2 * H) * B * T, launches=1):
+        rc = lib.avc_lstm_seq2(ctypes.byref(d0), ctypes.byref(d1), _stream())
+    if rc == _lib.ERR_NOT_RESIDENT:
+        return None
+    _lib.check(rc, "avc_lstm_seq2")
+    return h0, h1
 
 
 WS_MAX_BATCH = 64

@@ -265,6 +265,17 @@ typedef struct avc_lstm_desc {
 int avc_lstm_seq(const avc_lstm_desc* d, void* stream);
 
 /*
+ * Two stacked layers (nn.LSTM(num_layers = 2), factory/AutoVC.py:110) in ONE persistent launch, layer 1 two frames
+ * behind layer 0 on the same CTAs: each tick finishes frame t of layer 0 and frame t - 2 of layer 1, and the MMAs of
+ * one layer's inputs run while the other layer's cell update and the batch-group barrier are in flight.  Outputs
+ * are bit-identical to avc_lstm_seq(l0) followed by avc_lstm_seq(l1).  Requires equal B, T, H, dtype and gate_group,
+ * the fused input projection for both layers, l1->xin == l0->hseq, persistent mode, no lengths or h_last; the
+ * grid barrier scratch is l0's, and debug_clk (l0's) holds 12 stamps per (tick, CTA) for T + 2 ticks.  Returns
+ * AVC_ERR_NOT_RESIDENT, with nothing launched, when the grid cannot be co-resident.
+ */
+int avc_lstm_seq2(const avc_lstm_desc* l0, const avc_lstm_desc* l1, void* stream);
+
+/*
  * Small-batch form of the same recurrence (B <= 64, split-bf16 or fp16x2 precision): the recurrent weights stay in
  * tensor memory for the whole sequence (4H/128 row blocks x S K-slices, one thread-block cluster per row block
  * reducing its partial sums through distributed shared memory), so a frame moves only h_{t-1}.

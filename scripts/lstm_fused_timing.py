@@ -1,6 +1,8 @@
 """Per-frame clock64 breakdown of the fused (input projection + recurrence) persistent LSTM kernel (profiling aid).
 Stamps per (frame, CTA): 0 barrier passed (h producer), 1 first recurrent stage landed, 2 all MMAs issued,
-3 input-part MMAs issued, 4 accumulator ready (cell warps), 5 cell update done."""
+3 input-part MMAs issued, 4 accumulator ready (cell warps), 5 cell update done.
+`python scripts/lstm_fused_timing.py pair`: the same for the two-layer launch (ops.lstm_seq2) at AutoVC's lstm2 shapes,
+per tick, against the two one-layer launches it replaces."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -86,3 +88,60 @@ def per_cta(precision="fp32", B=512, T=128, H=1024, I=1024):
 if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "cta":
     per_cta(I=1024)
     per_cta(I=512)
+
+
+def run_pair(precision="fp16x2", B=512, T=128, H=1024, I=512):
+    """Two-layer launch: time per tick against two one-layer launches, and the tick's stamps (avc_lstm_seq2: 0 barrier
+    passed, 1 first rec0 stage landed, 2 / 3 rec0 / rec1 issued, 4 / 5 layer 0 accumulator ready / cell done, 6 / 7
+    layer 1, 8 cell warps done seen, 9 arrival issued, 10 / 11 in0 / in1 issued)."""
+    torch.manual_seed(0)
+    G = ops.choose_gate_group(B, H, True)
+    packs = []
+    for k in (I, H):
+        hh = packing.pack_lstm_hh(torch.randn(4 * H, H) * 0.03, precision, G).cuda()
+        wih, bias = packing.pack_lstm_ih_fused(torch.randn(4 * H, k) * 0.03, torch.zeros(4 * H), torch.zeros(4 * H),
+                                               precision, G)
+        packs.append((hh, wih.cuda(), bias.cuda()))
+    x = packing.to_act(torch.randn(B, T, I), precision).cuda()
+    (hh0, wih0, b0), (hh1, wih1, b1) = packs
+    m_tiles = (B + 127) // 128
+    m_tiles = (m_tiles + 1) // 2 * 2 if m_tiles >= 2 else m_tiles
+    grid = m_tiles * (H // G)
+
+    def two():
+        h = ops.lstm_seq(None, hh0, B, T, H, precision, G, persistent=True, xin=x, w_ih=wih0, bias=b0, c_in=I)
+        ops.lstm_seq(None, hh1, B, T, H, precision, G, persistent=True, xin=h, w_ih=wih1, bias=b1, c_in=H)
+
+    def pair(dbg=None):
+        ops.lstm_seq2((hh0, hh1), B, T, H, precision, G, x, (wih0, wih1), (b0, b1), I, debug_clk=dbg)
+
+    def timed(fn, n=5):
+        fn()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for _ in range(n):
+            fn()
+        e1.record()
+        torch.cuda.synchronize()
+        return e0.elapsed_time(e1) / n
+
+    t_two, t_pair = timed(two), timed(pair)
+    dbg = torch.zeros((T + 2) * grid * 12, dtype=torch.int64, device="cuda")
+    pair(dbg)
+    torch.cuda.synchronize()
+    d = dbg.view(T + 2, grid, 12).double().cpu()
+    cur, nxt = d[10:T - 1, 0::2 if m_tiles >= 2 else 1], d[11:T, 0::2 if m_tiles >= 2 else 1]
+    f = lambda a: f"{a.mean():.0f}"
+    print(f"pair {precision} B={B} T={T} H={H} I={I} G={G} grid={grid}: two launches {t_two:.3f} ms, one launch "
+          f"{t_pair:.3f} ms ({t_pair * 1e3 / (T + 2):.2f} us/tick); cycles from barrier passed: first h stage "
+          f"{f(cur[..., 1] - cur[..., 0])}, rec0 issued {f(cur[..., 2] - cur[..., 0])}, rec1 issued "
+          f"{f(cur[..., 3] - cur[..., 0])}, acc0 ready {f(cur[..., 4] - cur[..., 0])}, cell0 done "
+          f"{f(cur[..., 5] - cur[..., 0])}, acc1 ready {f(cur[..., 6] - cur[..., 0])}, cell1 done "
+          f"{f(cur[..., 7] - cur[..., 0])}, in0 issued {f(cur[..., 10] - cur[..., 0])}, in1 issued "
+          f"{f(cur[..., 11] - cur[..., 0])}, cells done seen {f(nxt[..., 8] - cur[..., 0])}, arrival "
+          f"{f(nxt[..., 9] - cur[..., 0])}, next barrier passed (tick) {f(nxt[..., 0] - cur[..., 0])}")
+
+
+if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "pair":
+    run_pair("fp16x2")
+    run_pair("fp32")
