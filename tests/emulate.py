@@ -361,17 +361,41 @@ def _emu_complex_mag(spec, bins, bins_pad, precision):
     return packing.to_act(mag.float().unsqueeze(0), precision)
 
 
+def resblock_terms(w, C, version):
+    """(hi, lo) fp64 (C_out, C_in) terms of W3 tap 0..2, W1, Wsc decoded from the PACKED tiles of
+    packing.pack_resblock (version 1) / pack_resblock2 (version 2), layouts as the kernels read them."""
+    w = w.double()
+    if version == 1:
+        if C == 64:
+            return [(w[i, :64], w[i, 64:]) for i in range(5)]
+        assert torch.equal(w[:, :32, :32], w[:, :32, 32:]) and not w[:, 32:, 32:].any()
+        return [(w[i, :32, :32], w[i, 32:, :32]) for i in range(5)]
+    if C == 128:      # [matrix][k-chunk][CTA 0: w_hi[0:64]; w_lo[0:64] | CTA 1: w_hi[64:128]; w_lo[64:128]][64]
+        terms = []
+        for m in range(5):
+            hi = torch.zeros(128, 128, dtype=torch.float64)
+            lo = torch.zeros(128, 128, dtype=torch.float64)
+            for kc in range(2):
+                t = w[(m * 2 + kc) * 256:(m * 2 + kc + 1) * 256]
+                ks = slice(kc * 64, kc * 64 + 64)
+                hi[0:64, ks], lo[0:64, ks], hi[64:128, ks], lo[64:128, ks] = t[0:64], t[64:128], t[128:192], t[192:256]
+            terms.append((hi, lo))
+        return terms
+    if C == 64:
+        return [(w[128 * i:128 * i + 64], w[128 * i + 64:128 * (i + 1)]) for i in range(5)]
+    k3 = [w[32 * i:32 * (i + 1)] for i in range(3)]
+    k1 = [w[96 + 64 * i:96 + 64 * (i + 1)] for i in range(2)]
+    for t in k1:
+        assert torch.equal(t[:32, :32], t[:32, 32:]) and not t[32:, 32:].any()
+    return [(t[:, :32], t[:, 32:]) for t in k3] + [(t[:32, :32], t[32:, :32]) for t in k1]
+
+
 def _emu_resblock_call(self, xa, x, B, L, out=None, out_row0=0, reflect=0, out_raw=None, out2=None):
     """Mirror of avc_resblock: reads the PACKED tiles (so packing.pack_resblock is what gets validated), the halo
     window of LeakyReLU(x) with row-shifted taps, the split intermediate, and the three output forms."""
     C, d = self.C, self.dilation
     assert xa.shape == (B, L + 2 * d, 2 * C) and x.shape == (B, L, 2 * C) and L % 128 == 0
-    w = self.w.double()
-    if C == 64:
-        mats = [w[i, :64] + w[i, 64:] for i in range(5)]
-    else:
-        assert torch.equal(w[:, :32, :32], w[:, :32, 32:]) and not w[:, 32:, 32:].any()
-        mats = [w[i, :32, :32] + w[i, 32:, :32] for i in range(5)]
+    mats = [hi + lo for hi, lo in resblock_terms(self.w, C, 1)]
     a = packing.act_to_float(xa, "fp32").double()
     mid = self.bias3.double().view(1, 1, C).expand(B, L, C).clone()
     for tap in range(3):
@@ -390,31 +414,17 @@ def _emu_resblock_call(self, xa, x, B, L, out=None, out_row0=0, reflect=0, out_r
     return out if out is not None else (out2 if out2 is not None else out_raw)
 
 
-def _emu_resblock2_call(self, x, B, L, y=None, y_row0=0, y_reflect=0, y_act=False, out2=None, wav=None, mono=None):
+def _emu_resblock2_call(self, x, B, L, y=None, y_row0=0, y_reflect=0, y_act=False, out2=None, wav=None, mono=None,
+                        lengths=None):
     """Mirror of avc_resblock2: reads the PACKED tiles (packing.pack_resblock2 is what gets validated), forms the k3
     operand as ONE fp16 value from the two-term window, keeps the intermediate as two fp16 terms, reads the shortcut
-    operand from the centre rows of the same window."""
+    operand from the centre rows of the same window.  lengths (ops.RaggedRows): a padded batch -- only the tiles that
+    hold a valid row are written, wav reflects at each utterance's own end and is 0 past it in its last tile."""
+    if lengths is not None:
+        return _emu_resblock2_ragged(self, x, B, L, lengths.host, y, y_row0, y_reflect, y_act, out2, wav, mono)
     C, d = self.C, self.dilation
     assert x.shape == (B, L + 2 * d, 2 * C) and x.dtype == torch.float16 and L % 128 == 0
-    w = self.w.double()
-    if C == 128:      # [matrix][k-chunk][CTA 0: w_hi[0:64]; w_lo[0:64] | CTA 1: w_hi[64:128]; w_lo[64:128]][64]
-        mats = []
-        for m in range(5):
-            mat = torch.zeros(128, 128, dtype=torch.float64)
-            for kc in range(2):
-                t = w[(m * 2 + kc) * 256:(m * 2 + kc + 1) * 256]
-                mat[0:64, kc * 64:kc * 64 + 64] = t[0:64] + t[64:128]
-                mat[64:128, kc * 64:kc * 64 + 64] = t[128:192] + t[192:256]
-            mats.append(mat)
-    elif C == 64:
-        tiles = [w[128 * i:128 * (i + 1)] for i in range(5)]
-        mats = [t[:64] + t[64:] for t in tiles]
-    else:
-        k3 = [w[32 * i:32 * (i + 1)] for i in range(3)]
-        k1 = [w[96 + 64 * i:96 + 64 * (i + 1)] for i in range(2)]
-        for t in k1:
-            assert torch.equal(t[:32, :32], t[:32, 32:]) and not t[32:, 32:].any()
-        mats = [t[:, :32] + t[:, 32:] for t in k3] + [t[:32, :32] + t[32:, :32] for t in k1]
+    mats = [hi + lo for hi, lo in resblock_terms(self.w, C, 2)]
     xs = packing.act_to_float(x, "fp16s").double()                                   # the stored stream (hi + lo)
     xa = F.leaky_relu(xs, 0.2).float().half().double()                                # one fp16 value
     mid = self.bias3.double().view(1, 1, C).expand(B, L, C).clone()
@@ -452,6 +462,39 @@ def _emu_resblock2_call(self, x, B, L, y=None, y_row0=0, y_reflect=0, y_act=Fals
         return wav
     out2[:] = F.leaky_relu(v, 0.2).float().reshape(B * L, C)
     return out2
+
+
+def _emu_resblock2_ragged(self, x, B, L, rows, y, y_row0, y_reflect, y_act, out2, wav, mono):
+    """_emu_resblock2_call over a padded batch: the dense result, stored only where avc_resblock2's compacted tile
+    space reaches (tiles of 128 rows, or of 128 - (K - 1) rows for wav); the right halo of y at an utterance's own end is
+    the caller's, the kernel writes the one at L only when the utterance's last tile runs."""
+    if wav is not None:
+        w_out, b_out = mono
+        K, lead = w_out.shape[0], w_out.shape[0] // 2
+        stride = 128 - (K - 1)
+        full = torch.empty(B * L, self.C)
+        _emu_resblock2_call(self, x, B, L, out2=full)
+        a = full.view(B, L, self.C).double()
+        for b, n in enumerate(rows):
+            tau = torch.arange(n)[:, None] + torch.arange(K)[None, :] - lead
+            tau = torch.where(tau < 0, -tau, tau)
+            tau = torch.where(tau >= n, 2 * (n - 1) - tau, tau)
+            acc = (a[b][tau] * w_out.double()[None]).sum(dim=(1, 2)) + b_out
+            wav[b, :n] = torch.tanh(acc).float()
+            wav[b, n:min(L, -(-n // stride) * stride)] = 0
+        return wav
+    full = y.clone() if y is not None else out2.clone()
+    _emu_resblock2_call(self, x, B, L, full if y is not None else None, y_row0, y_reflect, y_act,
+                        full if out2 is not None else None)
+    for b, n in enumerate(rows):
+        end = -(-n // 128) * 128                                                # rows of the tiles that run
+        if y is not None:
+            y[b, y_row0 - y_reflect:y_row0 + end] = full[b, y_row0 - y_reflect:y_row0 + end]
+            if end >= L:
+                y[b, y_row0 + L:y_row0 + L + y_reflect] = full[b, y_row0 + L:y_row0 + L + y_reflect]
+        else:
+            out2[b * L:b * L + end] = full[b * L:b * L + end]
+    return y if y is not None else out2
 
 
 def _emu_reflect_halo(buf, row0, L, reflect):

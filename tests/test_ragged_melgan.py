@@ -6,7 +6,6 @@ import warnings
 
 import pytest
 import torch
-import torch.nn.functional as F
 
 from oracle import rel_l2, templates
 from oracle.melgan import melgan_forward
@@ -43,42 +42,6 @@ def _emu_conv_to_mono_tanh(x, w, bias, lengths=None):
     return out
 
 
-def _emu_resblock2(self, x, B, L, y=None, y_row0=0, y_reflect=0, y_act=False, out2=None, wav=None, mono=None,
-                   lengths=None):
-    """The kernel's ragged contract: only the tiles that hold a valid row are computed and stored (the fixed-length
-    arithmetic on them); wav reflects at each utterance's end and is 0 past it in the last tile."""
-    if lengths is None:
-        return emulate._emu_resblock2_call(self, x, B, L, y, y_row0, y_reflect, y_act, out2, wav, mono)
-    rows = lengths.host
-    if wav is not None:
-        w_out, b_out = mono
-        K, lead = w_out.shape[0], w_out.shape[0] // 2
-        stride = 128 - (K - 1)
-        a = torch.empty(B * L, self.C)
-        emulate._emu_resblock2_call(self, x, B, L, out2=a)                      # LeakyReLU(y), exact fp32
-        a = a.view(B, L, -1).double()
-        for b, n in enumerate(rows):
-            tau = torch.arange(n)[:, None] + torch.arange(K)[None, :] - lead
-            tau = torch.where(tau < 0, -tau, tau)
-            tau = torch.where(tau >= n, 2 * (n - 1) - tau, tau)
-            acc = (a[b][tau] * w_out.double()[None]).sum(dim=(1, 2)) + b_out
-            wav[b, :n] = torch.tanh(acc).float()
-            wav[b, n:min(L, -(-n // stride) * stride)] = 0
-        return wav
-    full = y.clone() if y is not None else out2.clone()
-    emulate._emu_resblock2_call(self, x, B, L, full if y is not None else None, y_row0, y_reflect, y_act,
-                                full if out2 is not None else None)
-    for b, n in enumerate(rows):
-        end = -(-n // 128) * 128                                                # rows of the tiles that run
-        if y is not None:
-            y[b, y_row0 - y_reflect:y_row0 + end] = full[b, y_row0 - y_reflect:y_row0 + end]
-            if end >= L:
-                y[b, y_row0 + L:y_row0 + L + y_reflect] = full[b, y_row0 + L:y_row0 + L + y_reflect]
-        else:
-            out2[b * L:b * L + end] = full[b * L:b * L + end]
-    return y if y is not None else out2
-
-
 class _Recorder:
     def __init__(self):
         self.calls = []
@@ -98,7 +61,7 @@ def rec(monkeypatch):
     for name, fn in (("zero_tail", _emu_zero_tail), ("reflect_halo", _emu_reflect_halo),
                      ("conv_to_mono_tanh", _emu_conv_to_mono_tanh)):
         monkeypatch.setattr(ops, name, r.wrap(name, fn))
-    rb2 = r.wrap("resblock2", _emu_resblock2)
+    rb2 = r.wrap("resblock2", emulate._emu_resblock2_call)           # lengths-aware: only the tiles that run
     monkeypatch.setattr(ops.Resblock2, "__call__", lambda self, *a, **kw: rb2(self, *a, **kw))
     return r
 
