@@ -18,7 +18,7 @@ EXPORTS = ["avc_version", "avc_last_error", "avc_launch_count", "avc_conv_gemm",
            "avc_conv_to_mono_tanh", "avc_gn_stats", "avc_gn_pool_residual", "avc_gn_apply", "avc_patchify",
            "avc_ln_transpose", "avc_meta_decoder_input", "avc_gather_codes", "avc_global_stats", "avc_adain", "avc_audio_frames",
            "avc_complex_mag", "avc_resblock", "avc_resblock2", "avc_reflect_halo", "avc_bn_batch_stats", "avc_bn_apply",
-           "avc_zero_tail"]
+           "avc_zero_tail", "avc_segment_stats", "avc_adain_segmented"]
 
 
 MAX_SOURCES = 4
@@ -190,6 +190,7 @@ class Resblock2Desc(ctypes.Structure):
     ]
 
 
+SEGMENT_CHUNK = 4096    # AVC_SEGMENT_CHUNK: avc_segment_stats needs 2 * B * ceil(T * C / SEGMENT_CHUNK) doubles
 BN_MAX_PARTS = 256      # AVC_BN_MAX_PARTS: avc_bn_batch_stats needs 2 + 2 * BN_MAX_PARTS * C doubles of scratch
 
 
@@ -285,6 +286,9 @@ def load():
     lib.avc_global_stats.argtypes = [vp, ctypes.c_longlong, vp, vp, vp]
     lib.avc_adain.argtypes = [vp, vp, vp, vp, vp, ci, ci, ctypes.c_longlong, ci, vp]
     lib.avc_global_stats.restype = lib.avc_adain.restype = ctypes.c_int
+    lib.avc_segment_stats.argtypes = [vp, ci, ci, ci, vp, vp, vp, vp]
+    lib.avc_adain_segmented.argtypes = [vp, vp, vp, ci, vp, vp, vp, ci, ci, ci, ci, ci, vp]
+    lib.avc_segment_stats.restype = lib.avc_adain_segmented.restype = ctypes.c_int
     lib.avc_audio_frames.argtypes = [vp, vp, ci, ctypes.c_longlong, ci, ci, ci, ci, ci, vp]
     lib.avc_complex_mag.argtypes = [vp, vp, ctypes.c_longlong, ci, ci, ci, ci, vp]
     lib.avc_audio_frames.restype = lib.avc_complex_mag.restype = ctypes.c_int

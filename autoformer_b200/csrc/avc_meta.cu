@@ -137,6 +137,16 @@ __global__ void __launch_bounds__(256) global_stats_partial_kernel(const float* 
   }
 }
 
+// (sum x, sum x^2) over n elements -> (mean, Bessel-corrected std) as torch.mean() / torch.std(); the variance is
+// clamped at 0 against the cancellation of sum x^2 - n mean^2
+__device__ __forceinline__ void finish_mean_std(double a, double b, long long n, float* stats) {
+  const double mean = a / (double)n;
+  double var = (b - (double)n * mean * mean) / (double)(n - 1);
+  if (var < 0.0) var = 0.0;
+  stats[0] = (float)mean;
+  stats[1] = (float)sqrt(var);
+}
+
 __global__ void global_stats_final_kernel(const double* __restrict__ part, int parts, long long n,
                                           float* __restrict__ stats) {
   if (threadIdx.x == 0) {
@@ -145,30 +155,102 @@ __global__ void global_stats_final_kernel(const double* __restrict__ part, int p
       a += part[2 * i];
       b += part[2 * i + 1];
     }
-    const double mean = a / (double)n;
-    double var = (b - (double)n * mean * mean) / (double)(n - 1);      // torch.std(): Bessel-corrected
-    if (var < 0.0) var = 0.0;
-    stats[0] = (float)mean;
-    stats[1] = (float)sqrt(var);
+    finish_mean_std(a, b, n, stats);
   }
 }
 
+// ---------------------------------------------------------------- per-utterance mean / unbiased std
+// Utterance b's valid elements (rows 0 .. lengths[b]-1 x C, contiguous) are cut into chunks of AVC_SEGMENT_CHUNK
+// elements counted from its first element; CTA (k, b) sums chunk k in a fixed order (thread stride, then a fixed
+// shuffle / shared-memory tree), and one thread per utterance adds its chunks in index order.  Chunk boundaries and
+// both orders depend only on lengths[b] * C, so the bits of utterance b's statistics depend only on its own valid rows
+// -- not on B, T, its neighbours or what the padding holds (rows past lengths[b] are never read).
+constexpr int kSegThreads = 256;
+constexpr int kSegVecPerThread = AVC_SEGMENT_CHUNK / 4 / kSegThreads;
+static_assert(kSegVecPerThread * 4 * kSegThreads == AVC_SEGMENT_CHUNK, "chunk = whole float4 per thread");
+
+__global__ void __launch_bounds__(kSegThreads) segment_stats_partial_kernel(const float* __restrict__ x, int T, int C,
+                                                                            const int* __restrict__ lengths,
+                                                                            double* __restrict__ part) {
+  const int b = blockIdx.y, k = blockIdx.x;
+  const long long n4 = (long long)(lengths ? __ldg(lengths + b) : T) * C / 4;
+  const long long c0 = (long long)k * (AVC_SEGMENT_CHUNK / 4);
+  if (c0 >= n4) return;                                          // past this utterance's last chunk: never read
+  const float4* xs = reinterpret_cast<const float4*>(x + (long long)b * T * C) + c0;
+  const int m = (int)min((long long)(AVC_SEGMENT_CHUNK / 4), n4 - c0);
+  float4 v[kSegVecPerThread];
+#pragma unroll
+  for (int j = 0; j < kSegVecPerThread; ++j) {                    // all loads in flight before the first add
+    const int i = threadIdx.x + j * kSegThreads;
+    v[j] = i < m ? __ldg(xs + i) : make_float4(0.f, 0.f, 0.f, 0.f);
+  }
+  double s = 0.0, ss = 0.0;
+#pragma unroll
+  for (int j = 0; j < kSegVecPerThread; ++j) {
+    s += (double)v[j].x + (double)v[j].y + (double)v[j].z + (double)v[j].w;
+    ss += (double)v[j].x * v[j].x + (double)v[j].y * v[j].y + (double)v[j].z * v[j].z + (double)v[j].w * v[j].w;
+  }
+  __shared__ double red[2][kSegThreads / 32];
+  for (int o = 16; o > 0; o >>= 1) {
+    s += __shfl_xor_sync(0xffffffffu, s, o);
+    ss += __shfl_xor_sync(0xffffffffu, ss, o);
+  }
+  if ((threadIdx.x & 31) == 0) {
+    red[0][threadIdx.x >> 5] = s;
+    red[1][threadIdx.x >> 5] = ss;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double a = 0.0, q = 0.0;
+    for (int i = 0; i < kSegThreads / 32; ++i) {
+      a += red[0][i];
+      q += red[1][i];
+    }
+    double* p = part + 2 * ((long long)b * gridDim.x + k);
+    p[0] = a;
+    p[1] = q;
+  }
+}
+
+__global__ void segment_stats_final_kernel(const double* __restrict__ part, int B, int T, int C, int chunks,
+                                           const int* __restrict__ lengths, float* __restrict__ stats) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const long long n = (long long)(lengths ? __ldg(lengths + b) : T) * C;
+  const int used = (int)((n + AVC_SEGMENT_CHUNK - 1) / AVC_SEGMENT_CHUNK);
+  const double* p = part + 2LL * b * chunks;
+  double a = 0.0, q = 0.0;
+  for (int k = 0; k < used; ++k) {
+    a += p[2 * k];
+    q += p[2 * k + 1];
+  }
+  finish_mean_std(a, q, n, stats + 2 * b);
+}
+
 // ---------------------------------------------------------------- AdaIN: (x - mean_x) / std_x * std_t + mu_t
+// x [B][T][C]: utterance b is normalised with x_stats[2b], x_stats[2b+1] and styled with t_stats[t_stride b + {0, 1}];
+// with lengths, rows t >= lengths[b] are written as 0 and not read.  avc_adain is the case B = 1, t_stride 0, no lengths.
 __global__ void __launch_bounds__(256) adain_kernel(const float* __restrict__ x, const float* __restrict__ xs,
-                                                    const float* __restrict__ ts, float* __restrict__ out_f32,
+                                                    const float* __restrict__ ts, int t_stride,
+                                                    const int* __restrict__ lengths, float* __restrict__ out_f32,
                                                     void* __restrict__ out_op, int mode, int round, long long total4,
-                                                    int C) {
+                                                    long long T, int C) {
   const int c4n = C >> 2;
-  const float mean = __ldg(xs), inv = 1.0f / __ldg(xs + 1), mu = __ldg(ts), sd = __ldg(ts + 1);
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total4; i += (long long)gridDim.x * blockDim.x) {
     const long long row = i / c4n;
     const int c = static_cast<int>(i - row * c4n) << 2;
-    const float4 v = __ldg(reinterpret_cast<const float4*>(x + row * C + c));
-    float4 y;      // same operation order as the reference: ((x - mean) / std) * std_t + mu_t
-    y.x = (v.x - mean) * inv * sd + mu;
-    y.y = (v.y - mean) * inv * sd + mu;
-    y.z = (v.z - mean) * inv * sd + mu;
-    y.w = (v.w - mean) * inv * sd + mu;
+    const long long b = row / T;
+    float4 y = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (!lengths || row - b * T < __ldg(lengths + b)) {
+      const float mean = __ldg(xs + 2 * b), inv = 1.0f / __ldg(xs + 2 * b + 1);
+      const float mu = __ldg(ts + t_stride * b), sd = __ldg(ts + t_stride * b + 1);
+      const float4 v = __ldg(reinterpret_cast<const float4*>(x + row * C + c));
+      // same operation order as the reference: ((x - mean) / std) * std_t + mu_t
+      y.x = (v.x - mean) * inv * sd + mu;
+      y.y = (v.y - mean) * inv * sd + mu;
+      y.z = (v.z - mean) * inv * sd + mu;
+      y.w = (v.w - mean) * inv * sd + mu;
+    }
     if (out_f32) *reinterpret_cast<float4*>(out_f32 + row * C + c) = y;
     if (out_op) store_op4(out_op, mode, round, row, op_ld(C, mode), c, C, y);
   }
@@ -576,8 +658,39 @@ extern "C" int avc_adain(const float* x, const float* x_stats, const float* t_st
   AVC_REQUIRE(x && x_stats && t_stats && (out_f32 || out_op), "avc_adain: null buffer");
   AVC_REQUIRE(rows > 0 && C > 0 && C % 4 == 0 && out_dtype >= 0 && out_dtype <= 3, "avc_adain: bad shape");
   const long long total4 = rows * (C / 4);
-  adain_kernel<<<grid_for(total4), 256, 0, stream>>>(x, x_stats, t_stats, out_f32, out_op, out_dtype, out_round_tf32,
-                                                     total4, C);
+  adain_kernel<<<grid_for(total4), 256, 0, stream>>>(x, x_stats, t_stats, 0, nullptr, out_f32, out_op, out_dtype,
+                                                     out_round_tf32, total4, rows, C);
+  AVC_CHECK_CUDA(cudaGetLastError());
+  count_launch();
+  return 0;
+}
+
+extern "C" int avc_segment_stats(const float* x, int B, int T, int C, const int* lengths, float* stats,
+                                 double* scratch, void* stream_v) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
+  AVC_REQUIRE(x && stats && scratch, "avc_segment_stats: null buffer");
+  AVC_REQUIRE(B > 0 && B < 65536 && T > 0 && C > 0 && C % 4 == 0, "avc_segment_stats: bad arguments B=%d T=%d C=%d",
+              B, T, C);
+  const int chunks = (int)(((long long)T * C + AVC_SEGMENT_CHUNK - 1) / AVC_SEGMENT_CHUNK);
+  segment_stats_partial_kernel<<<dim3(chunks, B), kSegThreads, 0, stream>>>(x, T, C, lengths, scratch);
+  AVC_CHECK_CUDA(cudaGetLastError());
+  segment_stats_final_kernel<<<(B + 127) / 128, 128, 0, stream>>>(scratch, B, T, C, chunks, lengths, stats);
+  AVC_CHECK_CUDA(cudaGetLastError());
+  count_launch(2);
+  return 0;
+}
+
+extern "C" int avc_adain_segmented(const float* x, const float* x_stats, const float* t_stats, int t_stride,
+                                   const int* lengths, float* out_f32, void* out_op, int out_dtype, int out_round_tf32,
+                                   int B, int T, int C, void* stream_v) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
+  AVC_REQUIRE(x && x_stats && t_stats && (out_f32 || out_op), "avc_adain_segmented: null buffer");
+  AVC_REQUIRE(B > 0 && T > 0 && C > 0 && C % 4 == 0 && (t_stride == 0 || t_stride == 2) && out_dtype >= 0 &&
+                  out_dtype <= 3,
+              "avc_adain_segmented: bad arguments B=%d T=%d C=%d t_stride=%d", B, T, C, t_stride);
+  const long long total4 = (long long)B * T * (C / 4);
+  adain_kernel<<<grid_for(total4), 256, 0, stream>>>(x, x_stats, t_stats, t_stride, lengths, out_f32, out_op,
+                                                     out_dtype, out_round_tf32, total4, T, C);
   AVC_CHECK_CUDA(cudaGetLastError());
   count_launch();
   return 0;

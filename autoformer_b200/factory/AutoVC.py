@@ -127,11 +127,11 @@ class AutoVC(layers.PlanOwner, nn.Module):
                                lambda: _Plan(self, self.precision, self if batch else None), skip_bn_stats=batch)
 
     # hooks of the AdaIN "2" variants (factory/_adain.py); the plain model uses the mel as is and the plain postnet
-    def _encoder_features(self, x, plan, B, T):
+    def _encoder_features(self, x, plan, B, T, lengths=None):
         return x
 
-    def _run_postnet(self, plan, mel_op, mel, B, T, taps):
-        return plan.postnet(mel_op, mel, B, T, taps)
+    def _run_postnet(self, plan, mel_op, mel, B, T, taps, lengths=None):
+        return plan.postnet(mel_op, mel, B, T, taps, lengths=lengths)
 
     @ops.on_device_of_input
     @torch.no_grad()
@@ -165,7 +165,7 @@ class AutoVC(layers.PlanOwner, nn.Module):
             taps.clear()
 
         # ---- encoder: concat speaker code, 3x conv+BN+ReLU, BiLSTM, code down-sampling (AutoVC.py:45-68)
-        x = self._encoder_features(x, plan, B, T)
+        x = self._encoder_features(x, plan, B, T, lengths)
         h = ops.concat_bcast(x, c_org, T, 1, prec)
         # a padded batch: every buffer a k = 5 convolution reads gets its rows past each utterance's end zeroed (the
         # zero padding of converting it alone); conv 2's output feeds a 1x1 projection and the length-aware BiLSTM
@@ -218,7 +218,7 @@ class AutoVC(layers.PlanOwner, nn.Module):
             post = self._run_postnet(plan, mel_op, mel, B, T, taps)
         else:
             ops.zero_tail(mel_op, 0, T, lengths)
-            post = plan.postnet(mel_op, mel, B, T, taps, lengths=lengths)
+            post = self._run_postnet(plan, mel_op, mel, B, T, taps, lengths)
             ops.zero_tail(mel, 0, T, lengths)
             ops.zero_tail(post, 0, T, lengths)
         if taps is not None:

@@ -927,6 +927,48 @@ def adain(x, x_stats, t_stats, precision, want_f32=False):
     return out_op, out_f32
 
 
+def segment_stats(x, lengths=None, out=None):
+    """x [B][T][C] fp32 -> out [B][2] = (mean, std) of each utterance over its rows 0 .. lengths[b]-1 (all T rows
+    without lengths), torch defaults (Bessel-corrected std); the bits of row b depend only on utterance b's valid rows."""
+    lib = _lib.load()
+    _require_cuda(x)
+    assert x.dtype == torch.float32 and x.is_contiguous() and x.dim() == 3
+    B, T, C = x.shape
+    lens = _check_lengths(lengths, B) if lengths is not None else None
+    if out is None:
+        out = torch.empty(B, 2, dtype=torch.float32, device=x.device)
+    assert out.dtype == torch.float32 and out.is_contiguous() and out.numel() == 2 * B
+    # per call from the stream-ordered caching allocator: two batches on two streams never share it
+    chunks = -(-T * C // _lib.SEGMENT_CHUNK)
+    scratch = torch.empty(2 * B * chunks, dtype=torch.float64, device=x.device)
+    with PROFILER.span("segment_stats", bytes=4.0 * x.numel(), launches=2):
+        _lib.check(lib.avc_segment_stats(x.data_ptr(), B, T, C, lens, out.data_ptr(), scratch.data_ptr(), _stream()),
+                   "avc_segment_stats")
+    return out
+
+
+def adain_segmented(x, x_stats, t_stats, precision, lengths=None, want_f32=False):
+    """x [B][T][C] fp32 -> AdaIN with utterance b's statistics x_stats[b] (x_stats [B][2]) and the style t_stats ([2]:
+    one for every utterance, or [B][2]: one per utterance), in operand format (+ fp32 copy); with lengths, the rows past
+    each utterance's end are 0 in both outputs."""
+    lib = _lib.load()
+    _require_cuda(x, x_stats, t_stats)
+    assert x.dtype == torch.float32 and x.is_contiguous() and x.dim() == 3
+    B, T, C = x.shape
+    assert x_stats.dtype == torch.float32 and x_stats.is_contiguous() and x_stats.numel() == 2 * B
+    assert t_stats.dtype == torch.float32 and t_stats.is_contiguous() and t_stats.numel() in (2, 2 * B)
+    t_stride = 0 if t_stats.dim() == 1 else 2
+    assert t_stats.shape == ((2,) if t_stride == 0 else (B, 2)), t_stats.shape
+    lens = _check_lengths(lengths, B) if lengths is not None else None
+    out_op = alloc_act(B, T, C, precision, x.device)
+    out_f32 = torch.empty_like(x) if want_f32 else None
+    with PROFILER.span("adain", bytes=4.0 * x.numel() * 2):
+        _lib.check(lib.avc_adain_segmented(x.data_ptr(), x_stats.data_ptr(), t_stats.data_ptr(), t_stride, lens,
+                                           _ptr(out_f32), out_op.data_ptr(), _dt(precision), 1, B, T, C, _stream()),
+                   "avc_adain_segmented")
+    return out_op, out_f32
+
+
 # ------------------------------------------------------------------------------------------------ batch-statistics BatchNorm
 def bn_batch_stats(v, gamma, beta, eps=1e-5, momentum=0.1, running_mean=None, running_var=None,
                    num_batches_tracked=None, scale_shift=None):

@@ -174,7 +174,9 @@ def convert_utterances(model, mels, c_org, c_trg, max_batch=512):
     """Convert utterances of any lengths: mels is a list of (T_i, 80) device tensors, c_org / c_trg (N, dim_emb).
     Each is zero-padded to a multiple of ``model.freq`` (the reference's recipe, as ``convert``), the utterances are
     batched by ``sharding.make_ragged_batches`` and every batch runs once with per-utterance lengths.  Returns the
-    list of converted mels (mel_postnet, (T_i, 80)) in input order, each trimmed to T_i."""
+    list of converted mels (mel_postnet, (T_i, 80)) in input order, each trimmed to T_i.  An AdaIN "2" model must have
+    ``adain_stats = "utterance"`` (its forward refuses lengths otherwise); each utterance is then styled with its own
+    features, the Evaluator's ``isAdain`` recipe (util/evaluate.py:69-71, 81-82)."""
     out = [None] * len(mels)
     for _, ids, x, lens in _ragged_batches(mels, max_batch, model.freq):
         idx = torch.as_tensor(ids, device=c_org.device)

@@ -478,6 +478,26 @@ int avc_adain(const float* x, const float* x_stats, const float* t_stats, float*
               int out_round_tf32, long long rows, int C, void* stream);
 
 /*
+ * Per-utterance AdaIN statistics of a padded batch (adain_stats = "utterance"): each utterance is normalised and styled
+ * as the reference would do it alone.
+ * avc_segment_stats: stats[b] = {mean, Bessel-corrected std} over rows 0 .. lengths[b]-1 (all T rows when lengths is
+ *   NULL) x C of x [B][T][C] fp32; lengths device int32 [B], 1 <= lengths[b] <= T; C % 4 == 0, B < 65536.  fp64 partial
+ *   sums over chunks of AVC_SEGMENT_CHUNK elements counted from the utterance's first element, added in a fixed order:
+ *   the bits of stats[b] depend only on utterance b's valid rows and C (not on B, T, other utterances or the padding,
+ *   which is never read).  scratch: 2 * B * ceil(T * C / AVC_SEGMENT_CHUNK) doubles.  Two launches, no host sync.
+ * avc_adain_segmented: out[b][t] = (x[b][t] - x_stats[2b]) / x_stats[2b+1] * t_stats[t_stride b + 1]
+ *   + t_stats[t_stride b], the operation order of avc_adain; t_stride 0: one style for every utterance, 2: t_stats
+ *   [B][2].  With lengths, rows t >= lengths[b] are written as 0 in out_f32 and out_op (the zero padding of the next
+ *   k = 5 convolution) and x is not read there.  B = 1, t_stride 0, lengths NULL gives the bits of avc_adain.
+ */
+#define AVC_SEGMENT_CHUNK 4096
+int avc_segment_stats(const float* x, int B, int T, int C, const int* lengths, float* stats, double* scratch,
+                      void* stream);
+int avc_adain_segmented(const float* x, const float* x_stats, const float* t_stats, int t_stride, const int* lengths,
+                        float* out_f32, void* out_op, int out_dtype, int out_round_tf32, int B, int T, int C,
+                        void* stream);
+
+/*
  * Batch-statistics BatchNorm: nn.BatchNorm1d in training mode (torch.nn.functional.batch_norm, training=True), which is
  * how the reference's notebooks run every conv + BN layer -- they never call .eval() (conversion.ipynb cells 3 and 8,
  * util/evaluate.py; layers factory/AutoVC.py:26-39,117-171, factory/MetaPool.py:37-43,92-99, factory/Adjust.py:17-20,
